@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""Benchmark of the SCANN attention hot path on B200 (contract: see the task statement).
+"""Benchmark of the SCANN attention hot path on B200.
 
     python bench.py --gpus N --steps K --warmup W            # our sm_100a path
     python bench.py --impl reference --gpus N --steps K ...   # reference restated on CPU
+    python bench.py ... --dump-outputs DIR                    # + outputs of the last timed step as DIR/*.npy
 
 Workload = BASELINE.json configs[1]: QM9 HOMO model (configs/model_qm9.yaml) train step
 (forward + backward + Adam), 128 structures per GPU, synthetic QM9-shaped padded batch
@@ -163,6 +164,20 @@ def emit(line: str) -> None:          # replaced in main(): stdout is reserved f
     print(line)
 
 
+def dump_outputs(out_dir, eng, b, batch_global):
+    """Writes what the last timed train step computed, as float32 .npy files: ``loss`` = [loss, RMSE, MAE] (what
+    ``model.train_on_batch`` returns), ``params`` = the parameter arena after its Adam update (``model.get_weights``
+    in ParamLayout order), and ``y`` [B] / ``ga_score`` [B*M] of its training-mode forward (Dropout on).  The inputs,
+    initial weights and Dropout seeds are fixed, so two builds can be compared file by file (about 3.6 MB for qm9).
+    Expect two runs of one build to differ at float32 round-off, because atomic float32 sums are not ordered: of
+    order 1e-5 of the largest magnitude in y and the loss, less in the parameters."""
+    ws = eng._workspace(b, True)
+    out = {"loss": eng.loss_value(batch_global)[:3], "params": eng.params, "y": ws["y"], "ga_score": ws["ga"]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy().astype(np.float32))
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -255,12 +270,14 @@ def run_ours(args):
         flush.fill_(1.0)                                   # L2 flush, outside the per-step events
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        step_device()
+        last_batch = step_device()
         e1.record()
         evs.append((e0, e1))
     barrier()
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
     launches = eng.launches - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, last_batch, B * world)
     # ---- timed region 2: end to end through the public API (host buffers).  The call a user of the reference makes
     # is model.fit(iterator) (scann_model.py:232-241): every step packs the numpy batch into pinned memory, copies
     # it to the device (copy stream, overlapping the previous step), runs the step and reads [loss, rmse, mae] back
@@ -538,7 +555,13 @@ def main():
     ap.add_argument("--workload", default="qm9", choices=sorted(WORKLOADS),
                     help="qm9 (default, BASELINE.json configs[1]) | mp2018 | fullerene: other shapes, for reference")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed train step computed to DIR/<name>.npy (sm_100a arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the sm_100a arm (--impl ours)")
     # stdout carries exactly ONE JSON line.  Libraries write there too (NCCL prints "NCCL version ..." to stdout
     # under NCCL_DEBUG=VERSION, whatever NCCL_DEBUG_FILE says), so file descriptor 1 points at stderr until the
     # line is printed.

@@ -7,8 +7,8 @@ SCANN attention hot path.  Only ``tests/``, ``__graft_entry__.smoke()`` and the
 PARITY: PINNED TO REFERENCE-RUN CODE AT THE GRAPH LEVEL, UNPINNED AT THE TENSORFLOW-PRIMITIVE LEVEL.
 The reference's arithmetic lives in TensorFlow 2.10 / Keras 2.10 (environment.yml:144,212,282), which is neither
 installed nor installable here (no wheel, no network), and the reference ships no tests, golden vectors or weights
-(SURVEY.md F2, F8).  What IS checked (tests/test_reference_graph.py, run in the build container where
-/root/reference exists): the reference's own ``create_model`` / ``LocalAttention.call`` / ``GlobalAttention.call`` /
+(SURVEY.md F2, F8).  What IS checked (tests/test_reference_graph.py, run where SCANN_REFERENCE_ROOT
+names a checkout of the reference): the reference's own ``create_model`` / ``LocalAttention.call`` / ``GlobalAttention.call`` /
 ``ResidualNorm.call`` / ``GaussianExpansion`` / ``gather_shape`` / ``mrelu`` / ``root_mean_squared_error`` are imported
 UNMODIFIED and executed on a functional stand-in for the TensorFlow primitives (tests/tf_shim.py, PyTorch-CPU); this
 restatement agrees with them to fp64 round-off on outputs, ga_score, loss and every per-tensor gradient for seven
@@ -18,7 +18,7 @@ What is NOT checked: TensorFlow's own kernels behind those primitives (fp32 summ
 reductions, fused vs non-fused LayerNormalization) -- restated from the Keras documentation: non-fused
 LayerNormalization for eps < 1.001e-5, max-subtracted softmax, swish = x*sigmoid(x), Dense = x @ W + b.
 
-Every function cites the reference lines it follows (paths relative to /root/reference).
+Every function cites the reference lines it follows (paths relative to the reference's repository root).
 Run in float64 for "truth" and in float32 for the reference's own rounding behaviour.
 """
 from __future__ import annotations

@@ -2,7 +2,7 @@
 
 TensorFlow is absent (SURVEY.md F2) and the reference ships no golden vectors (F8).  The fixtures are written by
 the oracle; ``tests/test_reference_graph.py::test_golden_vectors_equal_the_reference_graph`` then runs the
-reference's OWN ``create_model`` graph (imported from /root/reference on the functional TensorFlow stand-in
+reference's OWN ``create_model`` graph (imported from the SCANN_REFERENCE_ROOT checkout on the functional TensorFlow stand-in
 ``tests/tf_shim.py``) on the same seeded cases and requires equality at fp64 round-off, so the committed values are
 pinned to reference-run code at the graph level (TensorFlow's own primitive kernels stay unpinned).
 

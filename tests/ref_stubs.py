@@ -1,5 +1,7 @@
-"""Import the reference's own pure-Python modules (from /root/reference, when it exists) with the third-party
-packages that are not installed here replaced by inert stubs.
+"""Import the reference's own pure-Python modules (from the checkout of the reference SCANN project that the
+environment variable ``SCANN_REFERENCE_ROOT`` names, when it is set) with the third-party packages that are not
+installed here replaced by inert stubs.  The reference's source is not part of this repository: without it the tests
+that import it skip, while the vectors its graph code produced (``tests/golden/ref_*.npz``) are checked everywhere.
 
 The reference is Python on TensorFlow / Keras / pymatgen / openbabel / ase (SURVEY.md F1, F2); none of them is
 installable in this image.  The modules that feed and surround the hot path -- ``scann/utils/datagenerator.py``
@@ -19,12 +21,38 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("SCANN_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("SCANN_REFERENCE_ROOT", "")
 STUB_ROOTS = ("tensorflow", "keras", "openbabel", "pymatgen", "ase", "tqdm", "h5py", "wget", "requests")
+SKIP_REASON = "needs the reference SCANN source: set SCANN_REFERENCE_ROOT to a checkout of it"
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "scann", "utils", "datagenerator.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "scann", "utils", "datagenerator.py"))
+
+
+GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference")
+
+
+def check_stored(name: str, values: dict, rtol: float = 0.0, atol: float = 0.0) -> None:
+    """Compares ``values`` (str -> array) with ``tests/golden/reference/<name>.npz``: what a comparison with the
+    reference's own code found, so that it keeps being checked where the reference's source is absent.  Where the
+    reference is present the calling test also compares the same values with it live, so a stale file cannot pass.
+    Exact (dtype and bits) unless a tolerance is given.  ``SCANN_WRITE_REFERENCE_GOLDEN=1`` rewrites the file."""
+    import numpy as np
+    path = os.path.join(GOLDEN_DIR, name + ".npz")
+    values = {k: np.asarray(v) for k, v in values.items()}
+    if os.environ.get("SCANN_WRITE_REFERENCE_GOLDEN") == "1":
+        os.makedirs(GOLDEN_DIR, exist_ok=True)
+        np.savez_compressed(path, **values)
+        return
+    z = np.load(path)
+    assert sorted(z.files) == sorted(values), (name, sorted(set(z.files) ^ set(values)))
+    for k, v in values.items():
+        assert z[k].dtype == v.dtype and z[k].shape == v.shape, (name, k, z[k].dtype, v.dtype, z[k].shape, v.shape)
+        if (rtol or atol) and v.dtype.kind == "f":
+            np.testing.assert_allclose(v, z[k], rtol=rtol, atol=atol, err_msg=f"{name}: {k}")
+        else:
+            assert np.array_equal(v, z[k], equal_nan=v.dtype.kind == "f"), (name, k)
 
 
 class _StubMeta(type):

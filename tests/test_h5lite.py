@@ -1,9 +1,9 @@
 """The dependency-free HDF5 reader/writer (scann_b200/h5lite.py) behind ``load_weights("*.h5")``.
 
-Pin: a file written by libhdf5 itself.  scipy ships a MATLAB v7.3 test file (HDF5 with a 512-byte user block,
-superblock 0, symbol-table groups, contiguous float64 dataset, fixed-length string attribute) -- the same classic
-structures h5py produces for Keras weight files."""
-import glob
+Pin: a file written by libhdf5 itself.  ``tests/golden/testhdf5_7.4_GLNX86.mat`` is a MATLAB v7.3 test file from
+SciPy's test data (scipy/io/matlab/tests/data, BSD-3-Clause, see tests/golden/LICENSE.scipy): HDF5 with a 512-byte user block, superblock 0,
+symbol-table groups, contiguous float64 dataset, fixed-length string attribute -- the same classic structures h5py
+produces for Keras weight files."""
 import os
 
 import numpy as np
@@ -13,12 +13,7 @@ from scann_b200 import h5lite
 
 
 def _matlab_file():
-    import scipy.io.matlab
-    d = os.path.join(os.path.dirname(scipy.io.matlab.__file__), "tests", "data")
-    f = glob.glob(os.path.join(d, "testhdf5_7.4_GLNX86.mat"))
-    if not f:
-        pytest.skip("scipy test data not installed")
-    return f[0]
+    return os.path.join(os.path.dirname(__file__), "golden", "testhdf5_7.4_GLNX86.mat")
 
 
 def test_reads_a_file_written_by_libhdf5():

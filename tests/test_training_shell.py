@@ -42,9 +42,9 @@ def test_sgdrc_schedule_matches_the_reference_state_machine():
     assert min(lrs) >= 1e-4 - 1e-18 and max(lrs) <= 5e-4
 
 
-def test_checkpoint_and_early_stopping():
+def test_checkpoint_and_early_stopping(tmp_path):
     m = FakeModel()
-    ck = C.ModelCheckpoint("/tmp/scann_ck/models/model_{epoch}.h5", monitor="val_mae", save_best_only=True)
+    ck = C.ModelCheckpoint(str(tmp_path / "models" / "model_{epoch}.h5"), monitor="val_mae", save_best_only=True)
     es = C.EarlyStopping(monitor="val_mae", patience=2)
     for cb in (ck, es):
         cb.set_model(m)
@@ -57,7 +57,7 @@ def test_checkpoint_and_early_stopping():
         if m.stop_training:
             stopped = ep
             break
-    assert [p for _, p in m.saved] == ["/tmp/scann_ck/models/model_1.h5", "/tmp/scann_ck/models/model_2.h5"]
+    assert [p for _, p in m.saved] == [str(tmp_path / "models" / f"model_{e}.h5") for e in (1, 2)]
     assert all(kind == "full" for kind, _ in m.saved)
     assert stopped == 3                                  # two epochs without improvement after the best (0.4)
 

@@ -3,7 +3,7 @@ reference's hot path calls, built on PyTorch-CPU so that the reference's OWN gra
 ``create_model`` (scann/models/scann_model.py:329-453), ``LocalAttention.call`` / ``GlobalAttention.call`` /
 ``ResidualNorm.call`` (scann/layers/attention.py), ``GaussianExpansion.call`` / ``gather_shape`` / ``mrelu``
 (scann/layers/custom_layers.py), ``root_mean_squared_error`` (scann/layers/losses.py) -- executes UNMODIFIED from
-/root/reference, forward and (through torch autograd) backward.  TensorFlow itself is not installable here.
+a checkout of the reference (SCANN_REFERENCE_ROOT), forward and (through torch autograd) backward.  TensorFlow itself is not installable here.
 
 What this pins and what it does not.  Everything the reference *wrote* runs as written: which layers exist and in
 which order, every einsum string, reshape, mask expression, concat order, residual, which Dense kernels carry

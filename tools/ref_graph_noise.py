@@ -1,7 +1,8 @@
 """Noise floor of the reference's OWN graph code at the full configurations of the GPU parity test
-(tests/test_gpu_parity.py::FULL_CASES, same seeds): create_model of /root/reference executed on the functional
+(tests/test_gpu_parity.py::FULL_CASES, same seeds): create_model of the reference executed on the functional
 TensorFlow stand-in (tests/tf_shim.py) in fp32 and in fp64, beside the oracle restatement in the same two precisions.
-CPU only, needs /root/reference.   usage: python tools/ref_graph_noise.py > profiles/<round>_reference_graph_noise.log"""
+CPU only, needs a checkout of the reference SCANN project.
+usage: SCANN_REFERENCE_ROOT=<reference checkout> python tools/ref_graph_noise.py > profiles/<round>_reference_graph_noise.log"""
 import os, sys, time, warnings
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 warnings.simplefilter("ignore")
