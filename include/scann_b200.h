@@ -352,6 +352,38 @@ int scann_adam_step(float* params, const float* grads, float* m, float* v, const
 int scann_loss_value(const float* params, const float* l2mask, int n, const float* sse, float batch, float l2,
                      float* out3, void* stream);
 
+/* ---- Voronoi neighbour lists (the model's input) -------------------------------------------------------------
+ * compute_voronoi_neighbor (scann/utils/voronoi_neighbor.py:11-61): pymatgen VoronoiNN(weight="solid_angle", tol=0)
+ * .get_voronoi_polyhedra + _extract_nn_info for every listed centre, in fp64, one warp per centre (voronoi.cu).
+ * Structures: lattice [S,9] (rows = lattice vectors), coords [A,3] Cartesian, struct_atom_off [S+1] int32.
+ * Centres: centre_atom [C] (global atom row), centre_struct [C], cutoff [C] (Angstrom; the point set is every image
+ * within it).  allow_pathological: emit the finite facets of a cell that also has unbounded ones (otherwise such a
+ * centre emits nothing and carries flag 1: pymatgen's caller widens its cutoff and runs it again).
+ * slots: C * cap records of scratch (cap <= 64), slot_count [C] int32.  The result goes to `blob` (device):
+ *   int32 off[C+1] (CSR), int32 flags[C] (1 = unbounded facet, plus the SCANN_ERR_VORONOI_* bits of that centre),
+ *   zero padding to a multiple of 32 bytes, then ScannVoronoiFacet records (centre c: off[c] .. off[c+1]);
+ *   blob bytes >= round_up(4 * (2C + 1), 32) + 32 * C * cap.
+ * Records of a centre: its finite facets with solid angle > 0, in no particular order.  host_blob (nullable, host,
+ * pinned for an asynchronous copy) receives the whole blob with one cudaMemcpyAsync on `stream`.
+ * status [0] |= SCANN_ERR_VORONOI_*: two points of a cell closer than 1e-8 Angstrom, a capacity of the kernel
+ * exceeded (64 facets, 32 vertices per facet, 128 points of one distance shell, |image| <= 511), a centre without a
+ * finite facet, a cut whose facet boundary is not one cycle (numerically inconsistent input). */
+#define SCANN_ERR_VORONOI_COINCIDENT 32
+#define SCANN_ERR_VORONOI_CAPACITY 64
+#define SCANN_ERR_VORONOI_NO_FACET 128
+#define SCANN_ERR_VORONOI_TOPOLOGY 256
+typedef struct ScannVoronoiFacet {
+    double solid_angle;   /* pymatgen's fan formula over the facet's vertices, seen from the centre */
+    double normalized;    /* solid_angle / the largest solid angle of the centre's cell */
+    double distance;      /* |x_j + n L - x_i| */
+    int32_t site;         /* j, index within the structure */
+    int32_t image;        /* n packed as (n0 + 512) | (n1 + 512) << 10 | (n2 + 512) << 20 */
+} ScannVoronoiFacet;
+int scann_voronoi_neighbors(const double* lattice, const double* coords, const int32_t* struct_atom_off,
+                            const int32_t* centre_atom, const int32_t* centre_struct, const double* cutoff,
+                            int n_centres, int allow_pathological, int cap, void* slots, int32_t* slot_count,
+                            void* blob, void* host_blob, int32_t* status, void* stream);
+
 /* ---- NCCL gradient all-reduce (SURVEY.md 8b / 8e) ---------------------------------------------------------------
  * One process per GPU, one communicator per process.  Rank 0: scann_allreduce_unique_id(out128) -> 128 HOST bytes
  * (ncclUniqueId) that the caller sends to the other ranks; every rank, with its device current:

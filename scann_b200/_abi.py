@@ -62,6 +62,7 @@ PROTOTYPES = {
     "scann_rmse_prepare": (ci, [vp, vp, ci, vp, vp, vp]),
     "scann_adam_step": (ci, [vp, vp, vp, vp, vp, ci, vp, vp, vp, ci, vp]),
     "scann_loss_value": (ci, [vp, vp, ci, vp, C.c_float, C.c_float, vp, vp]),
+    "scann_voronoi_neighbors": (ci, [vp] * 6 + [ci, ci, ci, vp, vp, vp, vp, vp, vp]),
     "scann_allreduce_unique_id": (ci, [vp]),
     "scann_allreduce_init": (ci, [vp, ci, ci]),
     "scann_allreduce_sum": (ci, [vp, C.c_longlong, vp]),
