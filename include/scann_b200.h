@@ -417,6 +417,97 @@ int scann_p2p_begin_step(const void* block_dev, float* sums, void* stream);
 int scann_adam_p2p_step(float* params, float* m, float* v, const float* l2mask, int n, const void* block_dev,
                         float* sums, const void* scalars_dev, float* grad_out, int apply, void* stream);
 
+/* ---- deterministic training mode (DESIGN.md section 4.7) ------------------------------------------------------
+ * The train step of the reference under TF_DETERMINISTIC_OPS=1 (train.py:16-25): every gradient element, the loss sums
+ * and the Adam inputs are computed in an order fixed by the batch and the launch configuration, never by scheduling.
+ * Each floating-point element is written once by a plain store and then receives at most one add.  Where the default
+ * kernels add into an element from many CTAs, the entry points below store per-CTA partial sums into caller-allocated
+ * "slots" instead, and scann_slot_reduce / scann_wgrad_batch_reduce add the slots up in slot order.
+ *
+ * scann_plan_inverse: inverse neighbour CSR of a pair plan -- for atom row j (of R), inv_idx[inv_ptr[j] .. inv_ptr[j+1])
+ *   are the valid pair rows p (pair_c[p] >= 0) with pair_j[p] == j, ascending.  inv_ptr: R + 1 ints, inv_idx: rows
+ *   ints, cnt_ws: R ints and tmp_ws: rows ints of workspace.  Stands in for the index bookkeeping of TF's
+ *   deterministic gather_nd gradient (attention.py:130,135 under TF_DETERMINISTIC_OPS).
+ * scann_row_gather: dst0[j] = sum_{p in list(j)} src0[p] ([rows,128] -> [R,128]) in list order, and likewise
+ *   src1 -> dst1 (both nullable together).  Rows without pairs get zeros.  The deterministic gather_nd backward of
+ *   attention.py:130,135: the neighbour-row sums of d_a * g' (dx_scatter) and d_pre (t_scatter).
+ * scann_la_backward_pipe_det: scann_la_backward_pipe with dx_scatter a [rows,128] per-pair buffer (d_a * g' stored at
+ *   the pair row), t_scatter unused (d_pre stays per pair in prebuf), dbk [grid][128] and dgamma_g [grid][256]
+ *   (gamma | beta) slots, dbeta_g unused.  attention.py:118-216.
+ * scann_dense_chain2_det / scann_dense_chain_det: scann_dense_chain2 / scann_dense_chain with dgamma / dbeta of every
+ *   mode-4 step [scann_dense_chain2_grid(R) / scann_dense_chain_grid(R)][128] slots (LayerNorm backward,
+ *   attention.py:35,111,113).
+ * scann_wgrad_batch_tc_det / scann_wgrad_batch_reduce: scann_wgrad_batch_tc storing every problem that one CTA owns
+ *   and leaving the partial dW / db of shared problems in slots [grid][2][128*128] / [grid][2][128]; the reduce (same
+ *   grid, table and plan) adds them up in CTA order and stores them.  Dense / einsum kernel gradients
+ *   (attention.py:118-216, scann_model.py:424-447).
+ * scann_geom_init_backward_det: slots [2 * grid][2*20*128 + 2*128] (dWd | dWw | dbd | dbw per half-CTA);
+ *   scann_model.py:376-389.
+ * scann_noupdate_geom_backward_det: slots [2 * grid][21*128] (dWf | dbf per half-CTA); attention.py:155.
+ * scann_embed_backward_det: G_slots [scann_embed_backward_det_slots(R)][n_atoms + 3][128]; scann_model.py:361-374.
+ * scann_cgcnn_embed_backward_det: dense_embed's dWe / dbe into slots [(R + 31) / 32][(E + (ring ? 10 : 0) + 1) * 128];
+ *   scann_model.py:364-374.
+ * scann_ga_head_backward_det: dwp_slots [B][128], dbp_slots [B]; scann_model.py:441-447.
+ * scann_rmse_prepare_det: one CTA over the batch (losses.py:5-6).
+ * scann_adam_step_det: reg_slots 1184 floats (l2 sum per CTA, added up in CTA order); scann_model.py:212.
+ * scann_adam_p2p_step_det: scann_adam_p2p_step with the l2 sum in CTA order (reg_slots: 592 floats); the cross-rank
+ *   sum of the peer-memory exchange is in rank order already.
+ * scann_slot_reduce: table = DEVICE array of nent ScannSlotSum; dst[i] += sum_{s < nslots} slots[s * ld + i] for
+ *   i < count, slots in order; max_count >= every count.  One launch for all slot arrays that only the optimiser reads. */
+typedef struct ScannSlotSum {
+    const float* slots;
+    float* dst;
+    int nslots, count, ld, pad;
+} ScannSlotSum;
+int scann_plan_inverse(const int32_t* ntiles, int tile_stride, long long rows, const int32_t* pair_c, const int32_t* pair_j,
+                       int R, int32_t* inv_ptr, int32_t* inv_idx, int32_t* cnt_ws, int32_t* tmp_ws, void* stream);
+int scann_row_gather(int R, const int32_t* inv_ptr, const int32_t* inv_idx, const float* src0, float* dst0,
+                     const float* src1, float* dst1, void* stream);
+int scann_la_backward_pipe_det(int grid, long long rows, int which, const int32_t* ntiles, const int32_t* pair_c,
+                               const int32_t* pair_j, const float* x, const float* proj, const float* g_in,
+                               const float* g_new, float* kbuf, float* prebuf, const float* W2T, const float* WkT,
+                               const float* gamma_g, const float* d_ctx, float* dg, int dg_has_up, float* dg_out,
+                               float* dq, float* s_pre, float* t_scatter, float* dx_scatter, float* dgamma_g,
+                               float* dbeta_g, float* dbk, const void* attn_drop, int drop_site, int32_t* status,
+                               void* stream);
+int scann_dense_chain2_det(const ScannChainStep* steps, int nsteps, int R, int32_t* status, void* stream);
+int scann_dense_chain2_grid(int R);
+int scann_dense_chain_det(const ScannChainStep* steps, int nsteps, int R, void* stream);
+int scann_dense_chain_grid(int R);
+int scann_wgrad_batch_tc_det(int grid, const ScannWgradProblem* problems, int nprob, const int32_t* ntiles, int tile_stride,
+                             const int32_t* pair_c, const int32_t* pair_j, const int32_t* valid_rows,
+                             const int32_t* valid_j, const int32_t* nvalid, float* slots, float* bslots, void* stream);
+int scann_wgrad_batch_reduce(int grid, const ScannWgradProblem* problems, int nprob, const int32_t* ntiles, int tile_stride,
+                             const int32_t* valid_rows, const int32_t* nvalid, const float* slots, const float* bslots,
+                             void* stream);
+int scann_geom_init_backward_det(const int32_t* ntiles, int grid, int tile_stride, const int32_t* pair_c,
+                                 const float* pair_d, const float* pair_w, const float* centers_d,
+                                 const float* centers_w, const float* Wd, const float* bd, const float* Ww,
+                                 const float* bw, const float* dg0, float* slots, void* stream);
+int scann_embed_backward_det(const int32_t* atomic, const float* ring, int R, int E, int n_atoms,
+                             const float* emb, const float* Wr, const float* br, const float* We,
+                             const float* t0, const float* dx0, float* G_ws, float* G_slots, float* d_emb,
+                             float* dWr, float* dbr, float* dWe, float* dbe, const void* drop_ctl, void* stream);
+int scann_embed_backward_det_slots(int R);
+int scann_noupdate_geom_backward_det(const int32_t* ntiles, int grid, int tile_stride, const int32_t* pair_c,
+                                     const float* pair_d, const float* pair_w, const float* centers_d,
+                                     const float* Wf, const float* bf, const float* dg, float* slots, void* stream);
+int scann_cgcnn_embed_backward_det(const float* atomic92, const float* emb_rows, const float* ring, int R, int F,
+                                   int E, const float* Wr, const float* br, const float* We, const float* t0,
+                                   const float* dx0, float* d_cat_ws, float* dWemb, float* dbemb, float* dWr,
+                                   float* dbr, float* slots, const void* drop_ctl, void* stream);
+int scann_ga_head_backward_det(const float* qk, const uint8_t* atom_mask, int B, int M, int norm,
+                               const float* WbT, const float* wp, const float* tb, const float* dy,
+                               float* d_qk, float* d_tb, float* dwp_slots, float* dbp_slots, void* stream);
+int scann_rmse_prepare_det(const float* y, const float* target, int B, float* dy, float* sse, void* stream);
+int scann_adam_step_det(float* params, const float* grads, float* m, float* v, const float* l2mask, int n,
+                        float* sse, const void* scalars_dev, float* grad_out, int apply, float* reg_slots,
+                        void* stream);
+int scann_adam_p2p_step_det(float* params, float* m, float* v, const float* l2mask, int n, const void* block_dev,
+                            float* sums, const void* scalars_dev, float* grad_out, int apply, float* reg_slots,
+                            void* stream);
+int scann_slot_reduce(const ScannSlotSum* table, int nent, int max_count, void* stream);
+
 /* ---- development probes ------------------------------------------------------------------------
  * Exported only by development builds (nvcc -DSCANN_DEV_PROBES; the production library carries neither these entry
  * points nor the timestamp stores inside its kernels).

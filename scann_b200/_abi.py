@@ -75,6 +75,26 @@ PROTOTYPES = {
     "scann_p2p_close": (ci, [vp]),
     "scann_p2p_begin_step": (ci, [vp, vp, vp]),
     "scann_adam_p2p_step": (ci, [vp, vp, vp, vp, ci, vp, vp, vp, vp, ci, vp]),
+    # deterministic training mode
+    "scann_plan_inverse": (ci, [vp, ci, C.c_longlong, vp, vp, ci, vp, vp, vp, vp, vp]),
+    "scann_row_gather": (ci, [ci, vp, vp, vp, vp, vp, vp, vp]),
+    "scann_la_backward_pipe_det": (ci, [ci, C.c_longlong, ci] + [vp] * 14 + [ci] + [vp] * 8 + [vp, ci, vp, vp]),
+    "scann_dense_chain2_det": (ci, [vp, ci, ci, vp, vp]),
+    "scann_dense_chain2_grid": (ci, [ci]),
+    "scann_wgrad_batch_tc_det": (ci, [ci, vp, ci, vp, ci, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "scann_wgrad_batch_reduce": (ci, [ci, vp, ci, vp, ci, vp, vp, vp, vp, vp]),
+    "scann_geom_init_backward_det": (ci, [vp, ci, ci] + [vp] * 11 + [vp]),
+    "scann_embed_backward_det": (ci, [vp, vp, ci, ci, ci] + [vp] * 13 + [vp, vp]),
+    "scann_embed_backward_det_slots": (ci, [ci]),
+    "scann_ga_head_backward_det": (ci, [vp, vp, ci, ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "scann_rmse_prepare_det": (ci, [vp, vp, ci, vp, vp, vp]),
+    "scann_adam_step_det": (ci, [vp, vp, vp, vp, vp, ci, vp, vp, vp, ci, vp, vp]),
+    "scann_slot_reduce": (ci, [vp, ci, ci, vp]),
+    "scann_dense_chain_det": (ci, [vp, ci, ci, vp]),
+    "scann_dense_chain_grid": (ci, [ci]),
+    "scann_noupdate_geom_backward_det": (ci, [vp, ci, ci] + [vp] * 8 + [vp]),
+    "scann_cgcnn_embed_backward_det": (ci, [vp, vp, vp, ci, ci, ci] + [vp] * 11 + [vp, vp]),
+    "scann_adam_p2p_step_det": (ci, [vp, vp, vp, vp, ci, vp, vp, vp, vp, ci, vp, vp]),
 }
 
 # development probes: exported only by builds with -DSCANN_DEV_PROBES (bound when present)
@@ -122,6 +142,11 @@ class WgradProblem(C.Structure):
     """``ScannWgradProblem`` of include/scann_b200.h (one dW += X^T Y problem of ``scann_wgrad_batch_tc``)."""
     _fields_ = [("X", vp), ("Y", vp), ("xg", vp), ("dW", vp), ("db", vp), ("ldx", ci), ("ldy", ci), ("rows", ci),
                 ("pad", ci)]
+
+
+class SlotSum(C.Structure):
+    """``ScannSlotSum`` of include/scann_b200.h (one slot array of ``scann_slot_reduce``)."""
+    _fields_ = [("slots", vp), ("dst", vp), ("nslots", ci), ("count", ci), ("ld", ci), ("pad", ci)]
 
 
 class ScannAbiError(RuntimeError):

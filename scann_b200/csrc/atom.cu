@@ -114,6 +114,51 @@ __global__ void __launch_bounds__(128) embed_bwd_gather_kernel(const int32_t* __
     }
 }
 
+// Deterministic form of stage 1: thread n owns column n of every per-species row of the CTA's partial G (shared
+// memory, rows in order, no atomics); the partial goes to slot blockIdx.x of Gs ([grid][n_atoms + 3][128]).
+__global__ void __launch_bounds__(128) embed_bwd_gather_det_kernel(const int32_t* __restrict__ atomic,
+                                                                   const float* __restrict__ ring, int R, int n_atoms,
+                                                                   const float* __restrict__ t0,
+                                                                   const float* __restrict__ dx0, float* __restrict__ Gs,
+                                                                   int rows_per_cta, const ScannDropCtl* __restrict__ drop) {
+    extern __shared__ float s_g[];                       // [n_atoms + 3][128]
+    const int n = threadIdx.x, nrow = n_atoms + 3;
+    for (int z = 0; z < nrow; ++z) s_g[z * SCANN_D + n] = 0.f;
+    const int r0 = blockIdx.x * rows_per_cta, r1 = min(R, r0 + rows_per_cta);
+    for (int r = r0; r < r1; ++r) {
+        const float d = dx0[(size_t)r * SCANN_D + n] * drop_mult(drop, 0u, (uint32_t)r * SCANN_D + n) *
+                        swish_grad_f(t0[(size_t)r * SCANN_D + n]);
+        int z = atomic[r];
+        z = (z < 0 || z >= n_atoms) ? 0 : z;
+        s_g[z * SCANN_D + n] += d;
+        s_g[n_atoms * SCANN_D + n] += d;
+        if (ring) {
+            s_g[(n_atoms + 1) * SCANN_D + n] = fmaf(ring[(size_t)r * 2], d, s_g[(n_atoms + 1) * SCANN_D + n]);
+            s_g[(n_atoms + 2) * SCANN_D + n] = fmaf(ring[(size_t)r * 2 + 1], d, s_g[(n_atoms + 2) * SCANN_D + n]);
+        }
+    }
+    float* slot = Gs + (size_t)blockIdx.x * nrow * SCANN_D;
+    for (int z = 0; z < nrow; ++z) slot[z * SCANN_D + n] = s_g[z * SCANN_D + n];
+}
+
+// G[i] = sum over the nslots slots of Gs, in slot order (eight loads in flight)
+__global__ void __launch_bounds__(128) embed_bwd_slot_sum_kernel(const float* __restrict__ Gs, int nslots, int count,
+                                                                 float* __restrict__ G) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    float s = 0.f;
+    int k = 0;
+    for (; k + 8 <= nslots; k += 8) {
+        float v[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) v[u] = Gs[(size_t)(k + u) * count + i];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) s += v[u];
+    }
+    for (; k < nslots; ++k) s += Gs[(size_t)k * count + i];
+    G[i] = s;
+}
+
 // Backward, stage 2 (tiny): dWe = [emb^T G ; br (x) G_all + Wr^T G2], dbe = G_all,
 // d_emb = G We[:E]^T, dWr = G2 We[E:]^T, dbr = G_all We[E:]^T.  Gradients are ACCUMULATED.
 __global__ void __launch_bounds__(128) embed_bwd_final_kernel(int E, int n_atoms, int has_ring,
@@ -189,6 +234,9 @@ __global__ void __launch_bounds__(128) small_dense_fwd_kernel(const float* __res
 // General embedding backward, stage 1 (32 rows per CTA): d_t0 = dx0 * dropout * swish'(t0);
 // dWe[k, :] += cat[r, k] d_t0[r, :], dbe += d_t0, d_cat[r, k] = <d_t0[r, :], We[k, :]>  with
 // cat[r, :] = [emb_rows[r, :E] | br + ring[r] @ Wr].
+// DET (deterministic mode): the CTA's dWe rows and dbe go to its slot of dWe, a [grid][(Kin + 1) * 128] array
+// (dWe rows, then dbe; dbe unused).
+template <bool DET>
 __global__ void __launch_bounds__(128) embed_bwd_rows_kernel(const float* __restrict__ emb_rows,
                                                              const float* __restrict__ ring, int R, int E,
                                                              const float* __restrict__ Wr, const float* __restrict__ br,
@@ -219,12 +267,15 @@ __global__ void __launch_bounds__(128) embed_bwd_rows_kernel(const float* __rest
         }
     }
     __syncthreads();
-    atomicAdd(dbe + n, bsum);
+    float* slot = dWe + (size_t)blockIdx.x * (Kin + 1) * SCANN_D;
+    if constexpr (DET) slot[(size_t)Kin * SCANN_D + n] = bsum;
+    else atomicAdd(dbe + n, bsum);
     for (int k = 0; k < Kin; ++k) {
         float acc = 0.f;
 #pragma unroll 8
         for (int i = 0; i < 32; ++i) acc = fmaf(s_cat[i][k], s_dt[i][n], acc);
-        atomicAdd(dWe + (size_t)k * SCANN_D + n, acc);
+        if constexpr (DET) slot[(size_t)k * SCANN_D + n] = acc;
+        else atomicAdd(dWe + (size_t)k * SCANN_D + n, acc);
     }
     // d_cat[r, k]: thread k, loop over the CTA's rows
     for (int k = n; k < Kin; k += 128) {
@@ -345,6 +396,10 @@ __global__ void __launch_bounds__(256) geom_init_fwd_kernel(const int32_t* __res
 }
 
 // Backward: accumulates dWd, dbd, dWw, dbw from d_g0 (no gradient flows to distances/weights).
+// DET (deterministic mode): every half-CTA stores its partial sums into slot 2 * blockIdx.x + half of dWd, a
+// [2 * grid][GEOM_BWD_SLOT] array laid out as dWd | dWw | dbd | dbw (dbd, dWw, dbw unused).
+#define GEOM_BWD_SLOT (2 * SCANN_RBF * SCANN_D + 2 * SCANN_D)
+template <bool DET>
 __global__ void __launch_bounds__(256, 2) geom_init_bwd_kernel(const int32_t* __restrict__ ntiles, int stride,
                                                             const int32_t* __restrict__ pair_c,
                                                             const float* __restrict__ pair_d,
@@ -417,7 +472,16 @@ __global__ void __launch_bounds__(256, 2) geom_init_bwd_kernel(const int32_t* __
         }
     }
     pdl_trigger();
-    if ((long long)blockIdx.x * GEOM_CR < (long long)nt * stride) {
+    if constexpr (DET) {
+        float* slot = dWd + ((size_t)blockIdx.x * 2 + half) * GEOM_BWD_SLOT;
+#pragma unroll
+        for (int k = 0; k < SCANN_RBF; ++k) {
+            slot[k * SCANN_D + n] = gd[k];
+            slot[(SCANN_RBF + k) * SCANN_D + n] = gw[k];
+        }
+        slot[2 * SCANN_RBF * SCANN_D + n] = gbd;
+        slot[2 * SCANN_RBF * SCANN_D + SCANN_D + n] = gbw;
+    } else if ((long long)blockIdx.x * GEOM_CR < (long long)nt * stride) {
 #pragma unroll
         for (int k = 0; k < SCANN_RBF; ++k) {
             atomicAdd(dWd + k * SCANN_D + n, gd[k]);
@@ -475,6 +539,10 @@ __global__ void __launch_bounds__(256) noupdate_geom_fwd_kernel(const int32_t* _
 // g_update = False (attention.py:155): g' = swish(rbf(d) @ Wf + bf) * w is recomputed in every layer; its only
 // trainable inputs are Wf [20,128] and bf.  dWf += rbf^T d_pre, dbf += sum d_pre with
 // d_pre = dg' * w * swish'(pre), pre = rbf @ Wf + bf (recomputed here from the 8 bytes/pair of raw geometry).
+// DET (deterministic mode): every half-CTA stores its partial sums into slot 2 * blockIdx.x + half of dWf, a
+// [2 * grid][NOUP_BWD_SLOT] array laid out as dWf (20 x 128) | dbf (dbf unused).
+#define NOUP_BWD_SLOT ((SCANN_RBF + 1) * SCANN_D)
+template <bool DET>
 __global__ void __launch_bounds__(256, 2) noupdate_geom_bwd_kernel(const int32_t* __restrict__ ntiles, int stride,
                                                                 const int32_t* __restrict__ pair_c,
                                                                 const float* __restrict__ pair_d,
@@ -535,7 +603,12 @@ __global__ void __launch_bounds__(256, 2) noupdate_geom_bwd_kernel(const int32_t
         }
     }
     pdl_trigger();
-    if ((long long)blockIdx.x * GEOM_CR < (long long)nt * stride) {
+    if constexpr (DET) {
+        float* slot = dWf + ((size_t)blockIdx.x * 2 + half) * NOUP_BWD_SLOT;
+#pragma unroll
+        for (int k = 0; k < SCANN_RBF; ++k) slot[k * SCANN_D + n] = gf[k];
+        slot[SCANN_RBF * SCANN_D + n] = gb;
+    } else if ((long long)blockIdx.x * GEOM_CR < (long long)nt * stride) {
 #pragma unroll
         for (int k = 0; k < SCANN_RBF; ++k) atomicAdd(dWf + k * SCANN_D + n, gf[k]);
         atomicAdd(dbf + n, gb);
@@ -829,6 +902,47 @@ extern "C" int scann_embed_backward(const int32_t* atomic, const float* ring, in
     return scann_check_launch("scann_embed_backward");
 }
 
+extern "C" int scann_device_sm_count(void);
+
+// Deterministic form: G_slots = [scann_embed_backward_det_slots(R)][n_atoms + 3][128] floats of workspace.  Rows per CTA
+// are chosen so that the slots fill about two waves of CTAs: enough parallelism, slot traffic bounded by the SM count.
+static int embed_det_rows(int R) {
+    static int sms = 0;
+    if (sms == 0) sms = scann_device_sm_count();
+    const int ctas = 2 * (sms > 0 ? sms : 148);
+    const int rows = (R + ctas - 1) / ctas;
+    return rows < 16 ? 16 : rows;
+}
+
+extern "C" int scann_embed_backward_det(const int32_t* atomic, const float* ring, int R, int E, int n_atoms,
+                                        const float* emb, const float* Wr, const float* br, const float* We,
+                                        const float* t0, const float* dx0, float* G_ws, float* G_slots, float* d_emb,
+                                        float* dWr, float* dbr, float* dWe, float* dbe, const void* drop_ctl, void* stream) {
+    if (R <= 0) return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int nrow = n_atoms + 3, rows = embed_det_rows(R), nslots = (R + rows - 1) / rows;
+    const size_t smem = (size_t)nrow * SCANN_D * sizeof(float);
+    if (smem > 200 * 1024) { scann_set_error("embed_backward_det: n_atoms=%d too large", n_atoms); return 1; }
+    static size_t configured = 48 * 1024;             // dynamic shared memory the kernel is opted in to
+    if (smem > configured) {
+        if (cudaFuncSetAttribute(embed_bwd_gather_det_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) !=
+            cudaSuccess) {
+            scann_set_error("embed_backward_det: shared-memory opt-in failed");
+            return 1;
+        }
+        configured = 200 * 1024;
+    }
+    embed_bwd_gather_det_kernel<<<nslots, 128, smem, st>>>(atomic, ring, R, n_atoms, t0, dx0, G_slots, rows,
+                                                           (const ScannDropCtl*)drop_ctl);
+    embed_bwd_slot_sum_kernel<<<nrow, 128, 0, st>>>(G_slots, nslots, nrow * SCANN_D, G_ws);
+    embed_bwd_final_kernel<<<64, 128, 0, st>>>(E, n_atoms, ring ? 1 : 0, emb, Wr, br, We, G_ws, d_emb, dWr, dbr, dWe,
+                                               dbe);
+    return scann_check_launch("scann_embed_backward_det");
+}
+
+// Slots of the G workspace scann_embed_backward_det needs for R atom rows.
+extern "C" int scann_embed_backward_det_slots(int R) { return R <= 0 ? 0 : (R + embed_det_rows(R) - 1) / embed_det_rows(R); }
+
 // feature == "cgcnn": emb_rows [R,E] = atomic92 [R,92] @ embed_atom/kernel + bias (feeds scann_embed_forward).
 extern "C" int scann_cgcnn_embed_forward(const float* atomic92, const float* W, const float* b, int R, int F, int E,
                                          float* emb_rows, void* stream) {
@@ -847,10 +961,25 @@ extern "C" int scann_cgcnn_embed_backward(const float* atomic92, const float* em
     if (E > 128) { scann_set_error("cgcnn_embed_backward: embedding width %d too large", E); return 1; }
     if (R <= 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
-    embed_bwd_rows_kernel<<<(R + 31) / 32, 128, 0, st>>>(emb_rows, ring, R, E, Wr, br, We, t0, dx0, d_cat_ws, dWe, dbe,
-                                                       (const ScannDropCtl*)drop_ctl);
+    embed_bwd_rows_kernel<false><<<(R + 31) / 32, 128, 0, st>>>(emb_rows, ring, R, E, Wr, br, We, t0, dx0, d_cat_ws, dWe, dbe,
+                                                              (const ScannDropCtl*)drop_ctl);
     embed_bwd_cols_kernel<<<F + 1 + (ring ? 3 : 0), 128, 0, st>>>(atomic92, ring, R, F, E, d_cat_ws, dWemb, dbemb, dWr, dbr);
     return scann_check_launch("scann_cgcnn_embed_backward");
+}
+
+// Deterministic form: dense_embed's gradients go to slots [(R + 31) / 32][(E + (ring ? 10 : 0) + 1) * 128] (kernel rows,
+// then bias; scann_slot_reduce adds them up); the embed_atom / extra_embed gradients are written by one thread each.
+extern "C" int scann_cgcnn_embed_backward_det(const float* atomic92, const float* emb_rows, const float* ring, int R, int F,
+                                              int E, const float* Wr, const float* br, const float* We, const float* t0,
+                                              const float* dx0, float* d_cat_ws, float* dWemb, float* dbemb, float* dWr,
+                                              float* dbr, float* slots, const void* drop_ctl, void* stream) {
+    if (E > 128) { scann_set_error("cgcnn_embed_backward: embedding width %d too large", E); return 1; }
+    if (R <= 0) return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    embed_bwd_rows_kernel<true><<<(R + 31) / 32, 128, 0, st>>>(emb_rows, ring, R, E, Wr, br, We, t0, dx0, d_cat_ws, slots,
+                                                             (float*)nullptr, (const ScannDropCtl*)drop_ctl);
+    embed_bwd_cols_kernel<<<F + 1 + (ring ? 3 : 0), 128, 0, st>>>(atomic92, ring, R, F, E, d_cat_ws, dWemb, dbemb, dWr, dbr);
+    return scann_check_launch("scann_cgcnn_embed_backward_det");
 }
 
 extern "C" int scann_geom_init_forward(const int32_t* ntiles, int grid, int tile_stride, const int32_t* pair_c, const float* pair_d,
@@ -869,9 +998,21 @@ extern "C" int scann_geom_init_backward(const int32_t* ntiles, int grid, int til
                                         const float* dg0, float* dWd, float* dbd, float* dWw, float* dbw,
                                         void* stream) {
     if (tile_stride != 32 && tile_stride != 64 && tile_stride != 128) { scann_set_error("geom_init: tile_stride must be 64 or 128"); return 1; }
-    scann_launch(geom_init_bwd_kernel, dim3(grid), dim3(256), 0, stream, ntiles, tile_stride, pair_c, pair_d, pair_w, centers_d, centers_w,
+    scann_launch(geom_init_bwd_kernel<false>, dim3(grid), dim3(256), 0, stream, ntiles, tile_stride, pair_c, pair_d, pair_w, centers_d, centers_w,
                  Wd, bd, Ww, bw, dg0, dWd, dbd, dWw, dbw);
     return scann_check_launch("scann_geom_init_backward");
+}
+
+// Deterministic form: slots = [2 * grid][2 * 20 * 128 + 2 * 128] partial sums (dWd | dWw | dbd | dbw per half-CTA), to be
+// added up in slot order (scann_slot_reduce).
+extern "C" int scann_geom_init_backward_det(const int32_t* ntiles, int grid, int tile_stride, const int32_t* pair_c,
+                                            const float* pair_d, const float* pair_w, const float* centers_d,
+                                            const float* centers_w, const float* Wd, const float* bd, const float* Ww,
+                                            const float* bw, const float* dg0, float* slots, void* stream) {
+    if (tile_stride != 32 && tile_stride != 64 && tile_stride != 128) { scann_set_error("geom_init: tile_stride must be 64 or 128"); return 1; }
+    scann_launch(geom_init_bwd_kernel<true>, dim3(grid), dim3(256), 0, stream, ntiles, tile_stride, pair_c, pair_d, pair_w, centers_d,
+                 centers_w, Wd, bd, Ww, bw, dg0, slots, (float*)nullptr, (float*)nullptr, (float*)nullptr);
+    return scann_check_launch("scann_geom_init_backward_det");
 }
 
 // g' = swish(rbf(d) @ Wf + bf) * w of a g_update = False layer as a [tile_cap * tile_stride, 128] tensor (see
@@ -893,9 +1034,21 @@ extern "C" int scann_noupdate_geom_backward(const int32_t* ntiles, int grid, int
                                             const float* Wf, const float* bf, const float* dg, float* dWf, float* dbf,
                                             void* stream) {
     if (tile_stride != 32 && tile_stride != 64 && tile_stride != 128) { scann_set_error("noupdate_geom_backward: tile_stride must be 64 or 128"); return 1; }
-    scann_launch(noupdate_geom_bwd_kernel, dim3(grid), dim3(256), 0, stream, ntiles, tile_stride, pair_c, pair_d, pair_w,
+    scann_launch(noupdate_geom_bwd_kernel<false>, dim3(grid), dim3(256), 0, stream, ntiles, tile_stride, pair_c, pair_d, pair_w,
                  centers_d, Wf, bf, dg, dWf, dbf);
     return scann_check_launch("scann_noupdate_geom_backward");
+}
+
+// Deterministic form: slots = [2 * grid][21 * 128] partial sums (dWf | dbf per half-CTA), added up in slot order by
+// scann_slot_reduce.
+extern "C" int scann_noupdate_geom_backward_det(const int32_t* ntiles, int grid, int tile_stride, const int32_t* pair_c,
+                                                const float* pair_d, const float* pair_w, const float* centers_d,
+                                                const float* Wf, const float* bf, const float* dg, float* slots,
+                                                void* stream) {
+    if (tile_stride != 32 && tile_stride != 64 && tile_stride != 128) { scann_set_error("noupdate_geom_backward: tile_stride must be 64 or 128"); return 1; }
+    scann_launch(noupdate_geom_bwd_kernel<true>, dim3(grid), dim3(256), 0, stream, ntiles, tile_stride, pair_c, pair_d, pair_w,
+                 centers_d, Wf, bf, dg, slots, (float*)nullptr);
+    return scann_check_launch("scann_noupdate_geom_backward_det");
 }
 
 // Generic blocked dense: see DenseArgs.  A/W/bias arrays hold kblk / kblk*nblk / nblk entries.

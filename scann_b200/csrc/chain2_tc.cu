@@ -174,7 +174,9 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
     for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
 }
 
-template <int TR>
+// DET (deterministic mode, DESIGN.md section 4.7): the LayerNorm-backward column sums of a CTA are stored into its slot
+// (dgamma / dbeta point to [grid][128] slot arrays) instead of being added into the gradient arena.
+template <int TR, bool DET>
 __global__ void __launch_bounds__(C2_THREADS, 1) dense_chain2_kernel(const __grid_constant__ C2Args ga) {
     typedef C2Cfg<TR> K;
     extern __shared__ uint8_t smem_raw[];
@@ -588,7 +590,8 @@ __global__ void __launch_bounds__(C2_THREADS, 1) dense_chain2_kernel(const __gri
                     float sum = 0.f;
 #pragma unroll
                     for (int w = 0; w < C2_EPI_WARPS; ++w) sum += *reinterpret_cast<const float*>(base + (size_t)w * K::RPW * 128u);
-                    atomicAdd((which ? st.dbeta : st.dgamma) + p, sum);
+                    if constexpr (DET) (which ? st.dbeta : st.dgamma)[(size_t)blockIdx.x * SCANN_D + p] = sum;
+                    else atomicAdd((which ? st.dbeta : st.dgamma) + p, sum);
                 }
             }
             if (tid == 0) C2CLK(2, si * 6 + 5);
@@ -602,15 +605,15 @@ __global__ void __launch_bounds__(C2_THREADS, 1) dense_chain2_kernel(const __gri
     if (warp == C2_EPI_WARPS) tmem_dealloc(tmem, K::TCOLS);
 }
 
-template <int TR>
+template <int TR, bool DET>
 static int chain2_launch(const C2Args& a, void* stream) {
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(dense_chain2_kernel<TR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C2Cfg<TR>::SMEM);
+        cudaError_t e = cudaFuncSetAttribute(dense_chain2_kernel<TR, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C2Cfg<TR>::SMEM);
         if (e != cudaSuccess) { scann_set_error("dense_chain2: smem opt-in failed: %s", cudaGetErrorString(e)); return 1; }
         configured = true;
     }
-    scann_launch(dense_chain2_kernel<TR>, dim3((a.R + TR - 1) / TR), dim3(C2_THREADS), (size_t)C2Cfg<TR>::SMEM, stream, a);
+    scann_launch(dense_chain2_kernel<TR, DET>, dim3((a.R + TR - 1) / TR), dim3(C2_THREADS), (size_t)C2Cfg<TR>::SMEM, stream, a);
     return scann_check_launch("scann_dense_chain2");
 }
 
@@ -623,7 +626,8 @@ extern "C" int scann_dense_chain2_max_rows(void) {
 
 // Same contract as scann_dense_chain, except that W[kb] of every step points to the weight IMAGE of the block
 // (scann_weight_images; orientation 0 for x @ W, 1 for x @ W^T).
-extern "C" int scann_dense_chain2(const void* steps_host, int nsteps, int R, int32_t* status, void* stream) {
+template <bool DET>
+static int chain2_run(const void* steps_host, int nsteps, int R, int32_t* status, void* stream) {
     if (nsteps < 1 || nsteps > C2_MAX_STEPS) { scann_set_error("dense_chain2: nsteps must be in 1..%d", C2_MAX_STEPS); return 1; }
     if (R <= 0) return 0;
     static_assert(sizeof(C2Args) <= 4096, "kernel parameter space");
@@ -665,6 +669,23 @@ extern "C" int scann_dense_chain2(const void* steps_host, int nsteps, int R, int
     a.nblocks = nb;
     static int sms = 0;
     if (sms == 0) sms = scann_device_sm_count();
-    if ((R + 31) / 32 <= sms) return chain2_launch<32>(a, stream);
-    return chain2_launch<64>(a, stream);
+    if ((R + 31) / 32 <= sms) return chain2_launch<32, DET>(a, stream);
+    return chain2_launch<64, DET>(a, stream);
+}
+
+extern "C" int scann_dense_chain2(const void* steps_host, int nsteps, int R, int32_t* status, void* stream) {
+    return chain2_run<false>(steps_host, nsteps, R, status, stream);
+}
+
+// Deterministic form: dgamma / dbeta of every mode-4 step are [scann_dense_chain2_grid(R)][128] slot arrays.
+extern "C" int scann_dense_chain2_det(const void* steps_host, int nsteps, int R, int32_t* status, void* stream) {
+    return chain2_run<true>(steps_host, nsteps, R, status, stream);
+}
+
+// CTAs of one scann_dense_chain2 launch over R rows (32-row tiles while they fit one wave, else 64-row tiles).
+extern "C" int scann_dense_chain2_grid(int R) {
+    static int sms = 0;
+    if (sms == 0) sms = scann_device_sm_count();
+    if (R <= 0) return 0;
+    return (R + 31) / 32 <= sms ? (R + 31) / 32 : (R + 63) / 64;
 }

@@ -90,7 +90,9 @@ __device__ __forceinline__ void chain_weight_to_tmem(const float* __restrict__ W
     chain_weight_store(w, t_whi, t_wlo, warp);
 }
 
-template <int TR>
+// DET (deterministic mode, DESIGN.md section 4.7): the warps add their LayerNorm-backward column sums into shared memory
+// one warp after the other, and the CTA stores them into its slot (dgamma / dbeta point to [grid][128] slot arrays).
+template <int TR, bool DET>
 __global__ void __launch_bounds__(CH_THREADS, 1) dense_chain_kernel(const __grid_constant__ ChainArgs a) {
     constexpr int XIT = TR / 8;                         // LDG.128 per thread for one activation tile
     constexpr uint32_t IMG = (TR / 8) * TC_RG_STRIDE;   // bytes of one K-major image of TR rows
@@ -420,6 +422,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) dense_chain_kernel(const __grid
         }
         if (mode == 4) {
             // column sums over this CTA's rows -> shared -> global
+            float cg[4][4], cb[4][4];
 #pragma unroll
             for (int it = 0; it < 4; ++it)
 #pragma unroll
@@ -427,15 +430,36 @@ __global__ void __launch_bounds__(CH_THREADS, 1) dense_chain_kernel(const __grid
                     float dg = dgam[it][q], db = dbet[it][q];
                     dg += __shfl_xor_sync(0xffffffffu, dg, 8);  db += __shfl_xor_sync(0xffffffffu, db, 8);
                     dg += __shfl_xor_sync(0xffffffffu, dg, 16); db += __shfl_xor_sync(0xffffffffu, db, 16);
-                    if (rsub == 0) {
+                    if constexpr (DET) {
+                        cg[it][q] = dg; cb[it][q] = db;
+                    } else if (rsub == 0) {
                         atomicAdd(&s_dg[(l8 + 8 * it) * 4 + q], dg);
                         atomicAdd(&s_db[(l8 + 8 * it) * 4 + q], db);
                     }
                 }
-            __syncthreads();
-            if (tid < SCANN_D) {
-                atomicAdd(st.dgamma + tid, s_dg[tid]);
-                atomicAdd(st.dbeta + tid, s_db[tid]);
+            if constexpr (DET) {
+                for (int w = 0; w < CH_THREADS / 32; ++w) {
+                    if (warp == w && rsub == 0) {
+#pragma unroll
+                        for (int it = 0; it < 4; ++it)
+#pragma unroll
+                            for (int q = 0; q < 4; ++q) {
+                                s_dg[(l8 + 8 * it) * 4 + q] += cg[it][q];
+                                s_db[(l8 + 8 * it) * 4 + q] += cb[it][q];
+                            }
+                    }
+                    __syncthreads();
+                }
+                if (tid < SCANN_D) {
+                    st.dgamma[(size_t)blockIdx.x * SCANN_D + tid] = s_dg[tid];
+                    st.dbeta[(size_t)blockIdx.x * SCANN_D + tid] = s_db[tid];
+                }
+            } else {
+                __syncthreads();
+                if (tid < SCANN_D) {
+                    atomicAdd(st.dgamma + tid, s_dg[tid]);
+                    atomicAdd(st.dbeta + tid, s_db[tid]);
+                }
             }
         }
         __syncthreads();        // S and the images are rewritten / read by the next step
@@ -455,7 +479,8 @@ extern "C" int scann_debug_clocks_chain(long long* host_out64) {
 #endif
 
 // Host-side mirror of the public struct (include/scann_b200.h): identical layout to ChainStep.
-extern "C" int scann_dense_chain(const void* steps_host, int nsteps, int R, void* stream) {
+template <bool DET>
+static int chain_run(const void* steps_host, int nsteps, int R, void* stream) {
     if (nsteps < 1 || nsteps > CH_MAX_STEPS) { scann_set_error("dense_chain: nsteps must be in 1..%d", CH_MAX_STEPS); return 1; }
     if (R <= 0) return 0;
     ChainArgs a;
@@ -479,13 +504,13 @@ extern "C" int scann_dense_chain(const void* steps_host, int nsteps, int R, void
     for (int i = nsteps; i < CH_MAX_STEPS; ++i) a.s[i] = ChainStep{};
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(dense_chain_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        cudaError_t e = cudaFuncSetAttribute(dense_chain_kernel<128, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              (int)(3 * TC_TILE_BYTES));
         if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(dense_chain_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            e = cudaFuncSetAttribute(dense_chain_kernel<64, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)(3 * TC_TILE_BYTES / 2));
         if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(dense_chain_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            e = cudaFuncSetAttribute(dense_chain_kernel<32, DET>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)(3 * TC_TILE_BYTES / 4));
         if (e != cudaSuccess) { scann_set_error("dense_chain: smem opt-in failed: %s", cudaGetErrorString(e)); return 1; }
         configured = true;
@@ -497,8 +522,26 @@ extern "C" int scann_dense_chain(const void* steps_host, int nsteps, int R, void
     else if ((R + 63) / 64 <= sms) tr = 64;
     dim3 grid((R + tr - 1) / tr);
     const size_t smem = 3 * (size_t)(tr / 8) * TC_RG_STRIDE;
-    if (tr == 32) scann_launch(dense_chain_kernel<32>, grid, dim3(CH_THREADS), smem, stream, a);
-    else if (tr == 64) scann_launch(dense_chain_kernel<64>, grid, dim3(CH_THREADS), smem, stream, a);
-    else scann_launch(dense_chain_kernel<128>, grid, dim3(CH_THREADS), smem, stream, a);
+    if (tr == 32) scann_launch(dense_chain_kernel<32, DET>, grid, dim3(CH_THREADS), smem, stream, a);
+    else if (tr == 64) scann_launch(dense_chain_kernel<64, DET>, grid, dim3(CH_THREADS), smem, stream, a);
+    else scann_launch(dense_chain_kernel<128, DET>, grid, dim3(CH_THREADS), smem, stream, a);
     return scann_check_launch("scann_dense_chain");
+}
+
+extern "C" int scann_dense_chain(const void* steps_host, int nsteps, int R, void* stream) {
+    return chain_run<false>(steps_host, nsteps, R, stream);
+}
+
+// Deterministic form: dgamma / dbeta of every mode-4 step are [scann_dense_chain_grid(R)][128] slot arrays.
+extern "C" int scann_dense_chain_det(const void* steps_host, int nsteps, int R, void* stream) {
+    return chain_run<true>(steps_host, nsteps, R, stream);
+}
+
+// CTAs of one scann_dense_chain launch over R rows.
+extern "C" int scann_dense_chain_grid(int R) {
+    static int sms = 0;
+    if (sms == 0) sms = scann_device_sm_count();
+    if (R <= 0) return 0;
+    const int tr = (R + 31) / 32 <= sms ? 32 : ((R + 63) / 64 <= sms ? 64 : 128);
+    return (R + tr - 1) / tr;
 }

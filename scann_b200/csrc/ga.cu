@@ -119,6 +119,8 @@ __global__ void __launch_bounds__(GA_THREADS) ga_head_fwd_kernel(const float* __
 
 // Backward of head + global attention for one structure (SURVEY.md appendix A).
 // dy[b] is the upstream gradient of y[b] (mrelu has an identity gradient, custom_layers.py:12-13).
+// DET (deterministic mode): the head gradient of structure b is stored into slot b (dwp: [B][128], dbp: [B]).
+template <bool DET>
 __global__ void __launch_bounds__(GA_THREADS) ga_head_bwd_kernel(
     const float* __restrict__ qk, const uint8_t* __restrict__ atom_mask, int M, int norm,
     const float* __restrict__ WbT, const float* __restrict__ wp, const float* __restrict__ tb,
@@ -143,8 +145,13 @@ __global__ void __launch_bounds__(GA_THREADS) ga_head_bwd_kernel(
     {
         float t = tb[(size_t)b * SCANN_D + tid];
         float hid = swish_f(t);
-        atomicAdd(dwp + tid, g * hid);
-        if (tid == 0) atomicAdd(dbp, g);
+        if constexpr (DET) {
+            dwp[(size_t)b * SCANN_D + tid] = g * hid;
+            if (tid == 0) dbp[b] = g;
+        } else {
+            atomicAdd(dwp + tid, g * hid);
+            if (tid == 0) atomicAdd(dbp, g);
+        }
         float dt = g * wp[tid] * swish_grad_f(t);
         s_dtb[tid] = dt;
         d_tb[(size_t)b * SCANN_D + tid] = dt;
@@ -344,6 +351,7 @@ __global__ void __launch_bounds__(GA2_THREADS, 1) ga_head_fwd_staged_kernel(
     }
 }
 
+template <bool DET>
 __global__ void __launch_bounds__(GA2_THREADS, 1) ga_head_bwd_staged_kernel(
     const float* __restrict__ qk, const uint8_t* __restrict__ atom_mask, int M, int norm,
     const float* __restrict__ WbT, const float* __restrict__ wp, const float* __restrict__ tb,
@@ -372,8 +380,13 @@ __global__ void __launch_bounds__(GA2_THREADS, 1) ga_head_bwd_staged_kernel(
     const float g = dy[b];
     if (tid < 128) {                           // head
         const float t = tb[(size_t)b * SCANN_D + tid];
-        atomicAdd(dwp + tid, g * swish_f(t));
-        if (tid == 0) atomicAdd(dbp, g);
+        if constexpr (DET) {
+            dwp[(size_t)b * SCANN_D + tid] = g * swish_f(t);
+            if (tid == 0) dbp[b] = g;
+        } else {
+            atomicAdd(dwp + tid, g * swish_f(t));
+            if (tid == 0) atomicAdd(dbp, g);
+        }
         const float dt = g * wpc * swish_grad_f(t);
         s_dtb[tid] = dt;
         d_tb[(size_t)b * SCANN_D + tid] = dt;
@@ -446,8 +459,9 @@ static bool ga2_ready() {
     static int state = 0;                      // 0 unknown, 1 ok, -1 failed (fall back to the unstaged kernels)
     if (state == 0) {
         cudaError_t e1 = cudaFuncSetAttribute(ga_head_fwd_staged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GA2_SMEM_MAX);
-        cudaError_t e2 = cudaFuncSetAttribute(ga_head_bwd_staged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GA2_SMEM_MAX);
-        state = (e1 == cudaSuccess && e2 == cudaSuccess) ? 1 : -1;
+        cudaError_t e2 = cudaFuncSetAttribute(ga_head_bwd_staged_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, GA2_SMEM_MAX);
+        cudaError_t e3 = cudaFuncSetAttribute(ga_head_bwd_staged_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GA2_SMEM_MAX);
+        state = (e1 == cudaSuccess && e2 == cudaSuccess && e3 == cudaSuccess) ? 1 : -1;
         if (state < 0) cudaGetLastError();
     }
     return state > 0;
@@ -456,6 +470,8 @@ static bool ga2_ready() {
 // err_b = y_b - t_b ; dy_b = err_b (the 1/(B*RMSE) factor of d sqrt(mean err^2) is applied in the
 // optimiser AFTER the gradient all-reduce, so data-parallel ranks need one collective only);
 // sse[0] += sum err^2, abs_err[0] += sum |err|.
+// DET (deterministic mode, launched as ONE CTA): the sums are stored, not added.
+template <bool DET>
 __global__ void __launch_bounds__(256) rmse_prepare_kernel(const float* __restrict__ y, const float* __restrict__ target,
                                                            int B, float* __restrict__ dy, float* __restrict__ sse) {
     __shared__ float s_a[8], s_b[8];
@@ -475,8 +491,13 @@ __global__ void __launch_bounds__(256) rmse_prepare_kernel(const float* __restri
     if (threadIdx.x == 0) {
         float ta = 0.f, tc = 0.f;
         for (int w = 0; w < (int)(blockDim.x >> 5); ++w) { ta += s_a[w]; tc += s_b[w]; }
-        atomicAdd(sse, ta);
-        atomicAdd(sse + 1, tc);
+        if constexpr (DET) {
+            sse[0] = ta;
+            sse[1] = tc;
+        } else {
+            atomicAdd(sse, ta);
+            atomicAdd(sse + 1, tc);
+        }
     }
 }
 
@@ -496,26 +517,48 @@ extern "C" int scann_ga_head_forward(const float* qk, const uint8_t* atom_mask, 
     return scann_check_launch("scann_ga_head_forward");
 }
 
-extern "C" int scann_ga_head_backward(const float* qk, const uint8_t* atom_mask, int B, int M, int norm,
-                                      const float* WbT, const float* wp, const float* tb, const float* dy,
-                                      float* d_qk, float* d_tb, float* dwp, float* dbp, void* stream) {
+template <bool DET>
+static int ga_head_backward_launch(const float* qk, const uint8_t* atom_mask, int B, int M, int norm, const float* WbT,
+                                   const float* wp, const float* tb, const float* dy, float* d_qk, float* d_tb, float* dwp,
+                                   float* dbp, void* stream) {
     if (B <= 0) return 0;
     if (ga2_smem_bytes(M, true) <= GA2_SMEM_MAX && ga2_ready()) {
-        scann_launch(ga_head_bwd_staged_kernel, dim3(B), dim3(GA2_THREADS), ga2_smem_bytes(M, true), stream, qk, atom_mask, M,
+        scann_launch(ga_head_bwd_staged_kernel<DET>, dim3(B), dim3(GA2_THREADS), ga2_smem_bytes(M, true), stream, qk, atom_mask, M,
                      norm, WbT, wp, tb, dy, d_qk, d_tb, dwp, dbp);
         return scann_check_launch("scann_ga_head_backward");
     }
     size_t smem = (size_t)(3 * SCANN_D + 4 + 3 * M) * sizeof(float);
     if (smem > 48 * 1024) { scann_set_error("ga_head_backward: M=%d too large", M); return 1; }
-    scann_launch(ga_head_bwd_kernel, dim3(B), dim3(GA_THREADS), smem, stream, qk, atom_mask, M, norm, WbT, wp, tb, dy, d_qk,
+    scann_launch(ga_head_bwd_kernel<DET>, dim3(B), dim3(GA_THREADS), smem, stream, qk, atom_mask, M, norm, WbT, wp, tb, dy, d_qk,
                  d_tb, dwp, dbp);
     return scann_check_launch("scann_ga_head_backward");
+}
+
+extern "C" int scann_ga_head_backward(const float* qk, const uint8_t* atom_mask, int B, int M, int norm,
+                                      const float* WbT, const float* wp, const float* tb, const float* dy,
+                                      float* d_qk, float* d_tb, float* dwp, float* dbp, void* stream) {
+    return ga_head_backward_launch<false>(qk, atom_mask, B, M, norm, WbT, wp, tb, dy, d_qk, d_tb, dwp, dbp, stream);
+}
+
+// Deterministic form: dwp_slots [B][128] and dbp_slots [B] receive the head gradient of each structure (scann_slot_reduce
+// adds them up in structure order).
+extern "C" int scann_ga_head_backward_det(const float* qk, const uint8_t* atom_mask, int B, int M, int norm,
+                                          const float* WbT, const float* wp, const float* tb, const float* dy,
+                                          float* d_qk, float* d_tb, float* dwp_slots, float* dbp_slots, void* stream) {
+    return ga_head_backward_launch<true>(qk, atom_mask, B, M, norm, WbT, wp, tb, dy, d_qk, d_tb, dwp_slots, dbp_slots, stream);
 }
 
 extern "C" int scann_rmse_prepare(const float* y, const float* target, int B, float* dy, float* sse, void* stream) {
     if (B <= 0) return 0;
     int grid = (B + 255) / 256;
     if (grid > 64) grid = 64;
-    scann_launch(rmse_prepare_kernel, dim3(grid), dim3(256), 0, stream, y, target, B, dy, sse);
+    scann_launch(rmse_prepare_kernel<false>, dim3(grid), dim3(256), 0, stream, y, target, B, dy, sse);
     return scann_check_launch("scann_rmse_prepare");
+}
+
+// Deterministic form: one CTA walks the whole batch and stores the sums into sse[0..1] in a fixed order.
+extern "C" int scann_rmse_prepare_det(const float* y, const float* target, int B, float* dy, float* sse, void* stream) {
+    if (B <= 0) return 0;
+    scann_launch(rmse_prepare_kernel<true>, dim3(1), dim3(256), 0, stream, y, target, B, dy, sse);
+    return scann_check_launch("scann_rmse_prepare_det");
 }

@@ -55,6 +55,14 @@ struct PipeAttnBwdArgs {
     int32_t* status;
 };
 
+// Deterministic instantiations (DET = true, DESIGN.md section 4.7): d_a * g' is STORED at its pair row of dx_scatter
+// (a [rows,128] per-pair buffer; scann_row_gather sums it per atom row afterwards) instead of being added at the
+// neighbour row, and the column sums leave the CTA as one plain store per CTA slot (dbk: [grid][128]; dgamma_g /
+// dbeta_g: [grid][256], gamma then beta) after the consumer warps have combined their partials in warp order.
+// Geometry: t_scatter is not written at all -- d_pre stays per pair in the pre-activation buffer.
+__device__ __forceinline__ void pb_consumer_sync() { asm volatile("bar.sync 14, %0;" ::"n"(PF_CW * 32) : "memory"); }
+
+template <bool DET>
 __global__ void __launch_bounds__(PF_THREADS, 1) la_attn_bwd_pipe_kernel(const __grid_constant__ PipeAttnBwdArgs a) {
     __shared__ float s_dbk[SCANN_D];
     if (threadIdx.x < SCANN_D) s_dbk[threadIdx.x] = 0.f;
@@ -297,7 +305,11 @@ __global__ void __launch_bounds__(PF_THREADS, 1) la_attn_bwd_pipe_kernel(const _
                 float4 o = make_float4(0.f, 0.f, 0.f, 0.f);
                 if (pc[k] >= 0) {
                     const float4 da = lds4(Lo + off), gp = lds4(G + off), xj = lds4(X + off);
-                    red_add4(a.dx_scatter + (size_t)jj[k] * SCANN_D + lane * 4, da.x * gp.x, da.y * gp.y, da.z * gp.z, da.w * gp.w);
+                    if constexpr (DET)
+                        st4(a.dx_scatter + (rowbase + r) * SCANN_D + lane * 4,
+                            make_float4(da.x * gp.x, da.y * gp.y, da.z * gp.z, da.w * gp.w));
+                    else
+                        red_add4(a.dx_scatter + (size_t)jj[k] * SCANN_D + lane * 4, da.x * gp.x, da.y * gp.y, da.z * gp.z, da.w * gp.w);
                     o = make_float4(da.x * xj.x, da.y * xj.y, da.z * xj.z, da.w * xj.w);
                 }
                 sts4(X + off, o);
@@ -307,13 +319,27 @@ __global__ void __launch_bounds__(PF_THREADS, 1) la_attn_bwd_pipe_kernel(const _
             BCLK(0, 9);
             if (gtid == 0) mbar_arrive(&c.ready[s]);            // d_k and d_a * x[j]: over to the store warp
         }
-        atomicAdd(&s_dbk[lane * 4 + 0], dbk.x); atomicAdd(&s_dbk[lane * 4 + 1], dbk.y);
-        atomicAdd(&s_dbk[lane * 4 + 2], dbk.z); atomicAdd(&s_dbk[lane * 4 + 3], dbk.w);
+        if constexpr (DET) {
+            for (int w = 0; w < PF_CW; ++w) {
+                if (warp == w) {
+                    s_dbk[lane * 4 + 0] += dbk.x; s_dbk[lane * 4 + 1] += dbk.y;
+                    s_dbk[lane * 4 + 2] += dbk.z; s_dbk[lane * 4 + 3] += dbk.w;
+                }
+                pb_consumer_sync();
+            }
+        } else {
+            atomicAdd(&s_dbk[lane * 4 + 0], dbk.x); atomicAdd(&s_dbk[lane * 4 + 1], dbk.y);
+            atomicAdd(&s_dbk[lane * 4 + 2], dbk.z); atomicAdd(&s_dbk[lane * 4 + 3], dbk.w);
+        }
     }
     pdl_trigger();
     tc_fence_before();
     __syncthreads();
-    if (tid < SCANN_D) atomicAdd(a.dbk + tid, s_dbk[tid]);
+    if constexpr (DET) {
+        if (tid < SCANN_D) a.dbk[(size_t)blockIdx.x * SCANN_D + tid] = s_dbk[tid];
+    } else {
+        if (tid < SCANN_D) atomicAdd(a.dbk + tid, s_dbk[tid]);
+    }
     if (warp == PF_CW + 1) tmem_dealloc(tmem, 512);
 }
 
@@ -331,6 +357,7 @@ struct PipeGeomBwdArgs {
     int32_t* status;
 };
 
+template <bool DET>
 __global__ void __launch_bounds__(PF_THREADS, 1) la_geom_bwd_pipe_kernel(const __grid_constant__ PipeGeomBwdArgs a) {
     __shared__ float s_acc[2 * SCANN_D];
     if (threadIdx.x < 2 * SCANN_D) s_acc[threadIdx.x] = 0.f;
@@ -449,7 +476,7 @@ __global__ void __launch_bounds__(PF_THREADS, 1) la_geom_bwd_pipe_kernel(const _
                 const float4 dpre = make_float4(dp[0], dp[1], dp[2], dp[3]);
                 sts4(P + off, dpre);
                 sts4(Lo + off, tf32_lo4(dpre));
-                red_add4(a.t_scatter + (size_t)jr * SCANN_D + lane * 4, dp[0], dp[1], dp[2], dp[3]);
+                if constexpr (!DET) red_add4(a.t_scatter + (size_t)jr * SCANN_D + lane * 4, dp[0], dp[1], dp[2], dp[3]);
             }
             fence_async_smem();
             tc_fence_before();
@@ -509,15 +536,29 @@ __global__ void __launch_bounds__(PF_THREADS, 1) la_geom_bwd_pipe_kernel(const _
             BCLK(1, 7);
             if (gtid == 0) mbar_arrive(&c.ready[s]);            // d_pre and dg: over to the store warp
         }
-        atomicAdd(&s_acc[lane * 4 + 0], dgam.x); atomicAdd(&s_acc[lane * 4 + 1], dgam.y);
-        atomicAdd(&s_acc[lane * 4 + 2], dgam.z); atomicAdd(&s_acc[lane * 4 + 3], dgam.w);
-        atomicAdd(&s_acc[SCANN_D + lane * 4 + 0], dbet.x); atomicAdd(&s_acc[SCANN_D + lane * 4 + 1], dbet.y);
-        atomicAdd(&s_acc[SCANN_D + lane * 4 + 2], dbet.z); atomicAdd(&s_acc[SCANN_D + lane * 4 + 3], dbet.w);
+        if constexpr (DET) {
+            for (int w = 0; w < PF_CW; ++w) {
+                if (warp == w) {
+                    s_acc[lane * 4 + 0] += dgam.x; s_acc[lane * 4 + 1] += dgam.y;
+                    s_acc[lane * 4 + 2] += dgam.z; s_acc[lane * 4 + 3] += dgam.w;
+                    s_acc[SCANN_D + lane * 4 + 0] += dbet.x; s_acc[SCANN_D + lane * 4 + 1] += dbet.y;
+                    s_acc[SCANN_D + lane * 4 + 2] += dbet.z; s_acc[SCANN_D + lane * 4 + 3] += dbet.w;
+                }
+                pb_consumer_sync();
+            }
+        } else {
+            atomicAdd(&s_acc[lane * 4 + 0], dgam.x); atomicAdd(&s_acc[lane * 4 + 1], dgam.y);
+            atomicAdd(&s_acc[lane * 4 + 2], dgam.z); atomicAdd(&s_acc[lane * 4 + 3], dgam.w);
+            atomicAdd(&s_acc[SCANN_D + lane * 4 + 0], dbet.x); atomicAdd(&s_acc[SCANN_D + lane * 4 + 1], dbet.y);
+            atomicAdd(&s_acc[SCANN_D + lane * 4 + 2], dbet.z); atomicAdd(&s_acc[SCANN_D + lane * 4 + 3], dbet.w);
+        }
     }
     pdl_trigger();
     tc_fence_before();
     __syncthreads();
-    if (tid < SCANN_D) {
+    if constexpr (DET) {
+        if (tid < 2 * SCANN_D) a.dgamma_g[(size_t)blockIdx.x * 2 * SCANN_D + tid] = s_acc[tid];
+    } else if (tid < SCANN_D) {
         atomicAdd(a.dgamma_g + tid, s_acc[tid]);
         atomicAdd(a.dbeta_g + tid, s_acc[SCANN_D + tid]);
     }
@@ -525,14 +566,47 @@ __global__ void __launch_bounds__(PF_THREADS, 1) la_geom_bwd_pipe_kernel(const _
 }
 
 // ---- host ---------------------------------------------------------------------------------------------------
+template <bool DET>
 static int la_pipe_bwd_configure() {
     static bool configured = false;
     if (configured) return 0;
-    cudaError_t e = cudaFuncSetAttribute(la_attn_bwd_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PB_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(la_geom_bwd_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PB_SMEM);
+    cudaError_t e = cudaFuncSetAttribute(la_attn_bwd_pipe_kernel<DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PB_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(la_geom_bwd_pipe_kernel<DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PB_SMEM);
     if (e != cudaSuccess) { scann_set_error("la_backward_pipe: smem opt-in failed: %s", cudaGetErrorString(e)); return 1; }
     configured = true;
     return 0;
+}
+
+template <bool DET>
+static int la_pipe_bwd_launch(int grid, long long rows, int which, const int32_t* ntiles, const int32_t* pair_c,
+                              const int32_t* pair_j, const float* x, const float* proj, const float* g_in,
+                              const float* g_new, float* kbuf, float* prebuf, const float* W2T, const float* WkT,
+                              const float* gamma_g, const float* d_ctx, float* dg, int dg_has_up, float* dg_out,
+                              float* dq, float* s_pre, float* t_scatter, float* dx_scatter, float* dgamma_g,
+                              float* dbeta_g, float* dbk, const void* attn_drop, int drop_site, int32_t* status,
+                              void* stream) {
+    if (la_pipe_bwd_configure<DET>()) return 1;
+    if (grid <= 0) return 0;
+    if (which & 1) {
+        PipeAttnBwdArgs ab;
+        memset(&ab, 0, sizeof(ab));
+        if (pipe_encode_tmap(&ab.tm_k, kbuf, rows) || pipe_encode_tmap(&ab.tm_g, g_new, rows) ||
+            pipe_encode_tmap(&ab.tm_dg, dg, rows)) return 1;
+        ab.ntiles = ntiles; ab.pair_c = pair_c; ab.pair_j = pair_j; ab.x = x; ab.proj = proj; ab.WkT = WkT; ab.d_ctx = d_ctx;
+        ab.dq = dq; ab.dx_scatter = dx_scatter; ab.dbk = dbk; ab.dg_accum = dg_has_up ? 1 : 0;
+        ab.drop = (const ScannDropCtl*)attn_drop; ab.drop_site = drop_site; ab.status = status;
+        scann_launch(la_attn_bwd_pipe_kernel<DET>, dim3(grid), dim3(PF_THREADS), PB_SMEM, stream, ab);
+    }
+    if (which & 2) {
+        PipeGeomBwdArgs gb;
+        memset(&gb, 0, sizeof(gb));
+        if (pipe_encode_tmap(&gb.tm_pre, prebuf, rows) || pipe_encode_tmap(&gb.tm_g, g_in, rows) ||
+            pipe_encode_tmap(&gb.tm_dgt, dg, rows) || pipe_encode_tmap(&gb.tm_dgo, dg_out, rows)) return 1;
+        gb.ntiles = ntiles; gb.pair_c = pair_c; gb.pair_j = pair_j; gb.W2T = W2T; gb.gamma_g = gamma_g; gb.s_pre = s_pre;
+        gb.t_scatter = t_scatter; gb.dgamma_g = dgamma_g; gb.dbeta_g = dbeta_g; gb.status = status;
+        scann_launch(la_geom_bwd_pipe_kernel<DET>, dim3(grid), dim3(PF_THREADS), PB_SMEM, stream, gb);
+    }
+    return scann_check_launch("scann_la_backward_pipe");
 }
 
 // Pipelined backward of LocalAttention (TF autodiff of attention.py:118-216 inside keras fit) for pair plans with
@@ -545,26 +619,23 @@ extern "C" int scann_la_backward_pipe(int grid, long long rows, int which, const
                                       float* dq, float* s_pre, float* t_scatter, float* dx_scatter, float* dgamma_g,
                                       float* dbeta_g, float* dbk, const void* attn_drop, int drop_site, int32_t* status,
                                       void* stream) {
-    if (la_pipe_bwd_configure()) return 1;
-    if (grid <= 0) return 0;
-    if (which & 1) {
-        PipeAttnBwdArgs ab;
-        memset(&ab, 0, sizeof(ab));
-        if (pipe_encode_tmap(&ab.tm_k, kbuf, rows) || pipe_encode_tmap(&ab.tm_g, g_new, rows) ||
-            pipe_encode_tmap(&ab.tm_dg, dg, rows)) return 1;
-        ab.ntiles = ntiles; ab.pair_c = pair_c; ab.pair_j = pair_j; ab.x = x; ab.proj = proj; ab.WkT = WkT; ab.d_ctx = d_ctx;
-        ab.dq = dq; ab.dx_scatter = dx_scatter; ab.dbk = dbk; ab.dg_accum = dg_has_up ? 1 : 0;
-        ab.drop = (const ScannDropCtl*)attn_drop; ab.drop_site = drop_site; ab.status = status;
-        scann_launch(la_attn_bwd_pipe_kernel, dim3(grid), dim3(PF_THREADS), PB_SMEM, stream, ab);
-    }
-    if (which & 2) {
-        PipeGeomBwdArgs gb;
-        memset(&gb, 0, sizeof(gb));
-        if (pipe_encode_tmap(&gb.tm_pre, prebuf, rows) || pipe_encode_tmap(&gb.tm_g, g_in, rows) ||
-            pipe_encode_tmap(&gb.tm_dgt, dg, rows) || pipe_encode_tmap(&gb.tm_dgo, dg_out, rows)) return 1;
-        gb.ntiles = ntiles; gb.pair_c = pair_c; gb.pair_j = pair_j; gb.W2T = W2T; gb.gamma_g = gamma_g; gb.s_pre = s_pre;
-        gb.t_scatter = t_scatter; gb.dgamma_g = dgamma_g; gb.dbeta_g = dbeta_g; gb.status = status;
-        scann_launch(la_geom_bwd_pipe_kernel, dim3(grid), dim3(PF_THREADS), PB_SMEM, stream, gb);
-    }
-    return scann_check_launch("scann_la_backward_pipe");
+    return la_pipe_bwd_launch<false>(grid, rows, which, ntiles, pair_c, pair_j, x, proj, g_in, g_new, kbuf, prebuf, W2T, WkT,
+                                     gamma_g, d_ctx, dg, dg_has_up, dg_out, dq, s_pre, t_scatter, dx_scatter, dgamma_g,
+                                     dbeta_g, dbk, attn_drop, drop_site, status, stream);
+}
+
+// Deterministic form (DESIGN.md section 4.7): same arguments, except
+//   dx_scatter : [rows,128] per-pair buffer, d_a * g' stored at the pair row (scann_row_gather sums it per atom row)
+//   t_scatter  : unused (d_pre is left per pair in prebuf)
+//   dbk        : [grid][128] slots; dgamma_g : [grid][256] slots (gamma | beta); dbeta_g : unused
+extern "C" int scann_la_backward_pipe_det(int grid, long long rows, int which, const int32_t* ntiles, const int32_t* pair_c,
+                                          const int32_t* pair_j, const float* x, const float* proj, const float* g_in,
+                                          const float* g_new, float* kbuf, float* prebuf, const float* W2T, const float* WkT,
+                                          const float* gamma_g, const float* d_ctx, float* dg, int dg_has_up, float* dg_out,
+                                          float* dq, float* s_pre, float* t_scatter, float* dx_scatter, float* dgamma_g,
+                                          float* dbeta_g, float* dbk, const void* attn_drop, int drop_site, int32_t* status,
+                                          void* stream) {
+    return la_pipe_bwd_launch<true>(grid, rows, which, ntiles, pair_c, pair_j, x, proj, g_in, g_new, kbuf, prebuf, W2T, WkT,
+                                    gamma_g, d_ctx, dg, dg_has_up, dg_out, dq, s_pre, t_scatter, dx_scatter, dgamma_g,
+                                    dbeta_g, dbk, attn_drop, drop_site, status, stream);
 }

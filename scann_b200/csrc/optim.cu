@@ -16,11 +16,14 @@ struct AdamScalars {      // filled by the host every step (device copy)
     float batch;          // global batch size B
 };
 
+// DET (deterministic mode): the l2 sum of a CTA is combined in warp order and stored into reg_slots[blockIdx.x];
+// adam_reg_sum_kernel adds the slots up in CTA order.
+template <bool DET>
 __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const float* __restrict__ g,
                                                    float* __restrict__ m, float* __restrict__ v,
                                                    const float* __restrict__ l2mask, int n,
                                                    float* __restrict__ sse_rw, const AdamScalars* __restrict__ hs,
-                                                   float* __restrict__ grad_out, int apply) {
+                                                   float* __restrict__ grad_out, int apply, float* __restrict__ reg_slots) {
     const float* sse = sse_rw;
     const AdamScalars h = *hs;
     const float rmse = sqrtf(sse[0] / h.batch);
@@ -58,7 +61,33 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const 
         if (apply) { m[i] = mi; v[i] = vi; p[i] = o; }
     }
     reg = warp_sum(reg);
-    if ((threadIdx.x & 31) == 0) atomicAdd(sse_rw + 2, reg);
+    if constexpr (DET) {
+        __shared__ float s_reg[8];
+        if ((threadIdx.x & 31) == 0) s_reg[threadIdx.x >> 5] = reg;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            float t = 0.f;
+            for (int w = 0; w < 8; ++w) t += s_reg[w];
+            reg_slots[blockIdx.x] = t;
+        }
+    } else {
+        if ((threadIdx.x & 31) == 0) atomicAdd(sse_rw + 2, reg);
+    }
+}
+
+// one CTA: thread i adds slots i, i + 256, ... in order, then the 256 partials are added in thread order
+__global__ void __launch_bounds__(256) adam_reg_sum_kernel(const float* __restrict__ reg_slots, int nslots,
+                                                           float* __restrict__ sse_rw) {
+    __shared__ float s_t[256];
+    float t = 0.f;
+    for (int k = threadIdx.x; k < nslots; k += 256) t += reg_slots[k];
+    s_t[threadIdx.x] = t;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float a = 0.f;
+        for (int i = 0; i < 256; ++i) a += s_t[i];
+        sse_rw[2] += a;
+    }
 }
 
 // out[0] = sqrt(SSE/B) + l2 * sum(mask * p^2) ; out[1] = sqrt(SSE/B) ; out[2] = sum|err| / B.
@@ -75,9 +104,22 @@ extern "C" int scann_adam_step(float* params, const float* grads, float* m, floa
     if (n <= 0) return 0;
     int grid = (n / 4 + 255) / 256 + 1;
     if (grid > 1184) grid = 1184;
-    adam_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(params, grads, m, v, l2mask, n, sse,
-                                                        (const AdamScalars*)scalars_dev, grad_out, apply);
+    adam_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(params, grads, m, v, l2mask, n, sse,
+                                                               (const AdamScalars*)scalars_dev, grad_out, apply, nullptr);
     return scann_check_launch("scann_adam_step");
+}
+
+// Deterministic form: reg_slots = 1184 floats of workspace (the l2 sum per CTA).
+extern "C" int scann_adam_step_det(float* params, const float* grads, float* m, float* v, const float* l2mask, int n,
+                                   float* sse, const void* scalars_dev, float* grad_out, int apply, float* reg_slots,
+                                   void* stream) {
+    if (n <= 0) return 0;
+    int grid = (n / 4 + 255) / 256 + 1;
+    if (grid > 1184) grid = 1184;
+    adam_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(params, grads, m, v, l2mask, n, sse,
+                                                              (const AdamScalars*)scalars_dev, grad_out, apply, reg_slots);
+    adam_reg_sum_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(reg_slots, grid, sse);
+    return scann_check_launch("scann_adam_step_det");
 }
 
 extern "C" int scann_loss_value(const float* params, const float* l2mask, int n, const float* sse, float batch,

@@ -74,11 +74,14 @@ __global__ void __launch_bounds__(32) p2p_begin_step_kernel(const P2PBlock* __re
 }
 
 // sums[0] = global SSE, [1] = global sum |err|, [2] = l2 penalty sum (as sse[0..2] of adam_kernel / loss_value)
+// DET (deterministic mode): the l2 sum of a CTA is combined in warp order and stored into reg_slots[blockIdx.x]; the
+// last CTA of the rank (the ticket below) adds the slots in CTA order and stores sums[2].
+template <bool DET>
 __global__ void __launch_bounds__(256) adam_p2p_kernel(float* __restrict__ p, float* __restrict__ m, float* __restrict__ v,
                                                        const float* __restrict__ l2mask, int n,
                                                        const P2PBlock* __restrict__ blk, float* __restrict__ sums,
                                                        const AdamScalarsP* __restrict__ hs, float* __restrict__ grad_out,
-                                                       int apply) {
+                                                       int apply, float* __restrict__ reg_slots) {
     __shared__ P2PBlock b;
     if (threadIdx.x == 0) b = *blk;
     __syncthreads();
@@ -178,13 +181,30 @@ __global__ void __launch_bounds__(256) adam_p2p_kernel(float* __restrict__ p, fl
         if (apply) { m[i] = mi; v[i] = vi; p[i] = o; }
     }
     reg = warp_sum(reg);
-    if ((threadIdx.x & 31) == 0) atomicAdd(sums + 2, reg);
+    __shared__ float s_reg[8];
+    if constexpr (DET) {
+        if ((threadIdx.x & 31) == 0) s_reg[threadIdx.x >> 5] = reg;
+    } else {
+        if ((threadIdx.x & 31) == 0) atomicAdd(sums + 2, reg);
+    }
     // the last CTA of this rank: every read of the peers' arenas is complete
     __syncthreads();
     if (threadIdx.x == 0) {
+        if constexpr (DET) {
+            float t = 0.f;
+            for (int w = 0; w < 8; ++w) t += s_reg[w];
+            reg_slots[blockIdx.x] = t;
+        }
         __threadfence();
         const uint32_t t = atomicAdd(fl + P2P_TICKET, 1u);
         if (t == gridDim.x - 1) {
+            if constexpr (DET) {
+                __threadfence();
+                const volatile float* rs = reg_slots;
+                float a = 0.f;
+                for (int c = 0; c < (int)gridDim.x; ++c) a += rs[c];
+                sums[2] = a;
+            }
             fl[P2P_TICKET] = 0u;
             fl[P2P_EPOCH] = e;
             __threadfence_system();
@@ -249,7 +269,25 @@ extern "C" int scann_adam_p2p_step(float* params, float* m, float* v, const floa
     }
     int grid = (n / 4 + 255) / 256 + 1;
     if (grid > 592) grid = 592;                  // all CTAs resident at once (they wait for the peers' flags)
-    adam_p2p_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(params, m, v, l2mask, n, (const P2PBlock*)block_dev, sums,
-                                                           (const AdamScalarsP*)scalars_dev, grad_out, apply);
+    adam_p2p_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(params, m, v, l2mask, n, (const P2PBlock*)block_dev, sums,
+                                                                  (const AdamScalarsP*)scalars_dev, grad_out, apply, nullptr);
     return scann_check_launch("scann_adam_p2p_step");
+}
+
+// Deterministic form: reg_slots = 592 floats of workspace (the l2 sum per CTA, added up in CTA order).  The cross-rank
+// sum is already in rank order.
+extern "C" int scann_adam_p2p_step_det(float* params, float* m, float* v, const float* l2mask, int n, const void* block_dev,
+                                       float* sums, const void* scalars_dev, float* grad_out, int apply, float* reg_slots,
+                                       void* stream) {
+    if (n <= 0) return 0;
+    if ((((uintptr_t)params | (uintptr_t)m | (uintptr_t)v | (uintptr_t)l2mask | (uintptr_t)grad_out) & 15) != 0) {
+        scann_set_error("adam_p2p_step: arrays must be 16-byte aligned");
+        return 1;
+    }
+    if (!reg_slots) { scann_set_error("adam_p2p_step_det: reg_slots is required"); return 1; }
+    int grid = (n / 4 + 255) / 256 + 1;
+    if (grid > 592) grid = 592;
+    adam_p2p_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(params, m, v, l2mask, n, (const P2PBlock*)block_dev, sums,
+                                                                 (const AdamScalarsP*)scalars_dev, grad_out, apply, reg_slots);
+    return scann_check_launch("scann_adam_p2p_step_det");
 }

@@ -44,6 +44,8 @@ struct WgArgs {
     const int32_t* valid_rows;   // compact list of the valid pair rows (scann_plan_build), nullable
     const int32_t* valid_j;      // neighbour atom row of each compact entry
     const int32_t* nvalid;       // its length (device)
+    float* slots;                // deterministic form: [grid][2][128*128] partial dW of the shared problems
+    float* bslots;               //                     [grid][2][128]     partial db
 };
 
 __device__ __forceinline__ void wg_split_store(uint8_t* sHi, uint8_t* sLo, uint32_t off, float4 v) {
@@ -89,6 +91,11 @@ struct WgRegs {
 // for the copies, 256 for reading them back and ~200 for the dummy LDS the compiler wraps around LDGSTS, on top of
 // the 512 (split stores) + 752 (tensor-core reads) that are inherent: the kernel ran at 2.4 TB/s, bound by the
 // shared-memory pipe, not by HBM.
+// DET (deterministic mode, DESIGN.md section 4.7): a problem that lies entirely inside this CTA's unit range is STORED
+// into dW / db; the first and the last problem of the range, which neighbouring CTAs may share, go to the CTA's two
+// slots (slot 0: a problem that started before the range, slot 1: one that continues behind it), summed in CTA order
+// by scann_wgrad_batch_reduce.  The bias column sums of the warps are combined in warp order.
+template <bool DET>
 __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_batch_tc_kernel(const WgArgs a) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     // the BASE32B swizzle is a function of the absolute shared address: align the images to 1024 bytes
@@ -200,6 +207,16 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_batch_tc_kernel(const WgA
             if (pending[b]) { mbar_wait(&bars[b], phase[b]); phase[b] ^= 1; tc_fence_after(); pending[b] = false; }
         if (!first) {
             const int m = (warp & 3) * 32 + lane, nbase = (warp >> 2) * 32;
+            // (DET) owned problem: dW itself; shared problem: this CTA's slot
+            float* dW = pr.dW;
+            float* db = pr.db;
+            if constexpr (DET) {
+                const int slot = (int)blockIdx.x * 2 + (s_units[pc] < u_lo ? 0 : 1);
+                if (!(s_units[pc] >= u_lo && s_units[pc + 1] <= u_hi)) {
+                    dW = a.slots + (size_t)slot * SCANN_D * SCANN_D;
+                    db = a.bslots + (size_t)slot * SCANN_D;
+                }
+            }
             const uint32_t lane_base = (uint32_t)((warp & 3) * 32) << 16;
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
@@ -208,19 +225,44 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_batch_tc_kernel(const WgA
                 tmem_ld16(t_dc + lane_base + nbase + h * 16, c);
                 tmem_ld_wait();
 #pragma unroll
-                for (int q = 0; q < 16; q += 4)
-                    red_add4(pr.dW + (size_t)m * SCANN_D + nbase + h * 16 + q, v[q] + c[q], v[q + 1] + c[q + 1],
-                             v[q + 2] + c[q + 2], v[q + 3] + c[q + 3]);
+                for (int q = 0; q < 16; q += 4) {
+                    if constexpr (DET)
+                        st4(dW + (size_t)m * SCANN_D + nbase + h * 16 + q,
+                            make_float4(v[q] + c[q], v[q + 1] + c[q + 1], v[q + 2] + c[q + 2], v[q + 3] + c[q + 3]));
+                    else
+                        red_add4(pr.dW + (size_t)m * SCANN_D + nbase + h * 16 + q, v[q] + c[q], v[q + 1] + c[q + 1],
+                                 v[q + 2] + c[q + 2], v[q + 3] + c[q + 3]);
+                }
             }
-            if (pr.db) {
-                atomicAdd(&s_db[lane * 4 + 0], colsum.x); atomicAdd(&s_db[lane * 4 + 1], colsum.y);
-                atomicAdd(&s_db[lane * 4 + 2], colsum.z); atomicAdd(&s_db[lane * 4 + 3], colsum.w);
+            if constexpr (DET) {
+                if (pr.db) {
+                    for (int w = 0; w < WG_WARPS; ++w) {
+                        if (warp == w) {
+                            s_db[lane * 4 + 0] += colsum.x; s_db[lane * 4 + 1] += colsum.y;
+                            s_db[lane * 4 + 2] += colsum.z; s_db[lane * 4 + 3] += colsum.w;
+                        }
+                        __syncthreads();
+                    }
+                }
+                tc_fence_before();
+                __syncthreads();             // every warp has read the accumulators; s_db is complete
+                tc_fence_after();
+                if (pr.db && tid < SCANN_D) {
+                    db[tid] = s_db[tid];
+                    s_db[tid] = 0.f;
+                }
+                __syncthreads();
+            } else {
+                if (pr.db) {
+                    atomicAdd(&s_db[lane * 4 + 0], colsum.x); atomicAdd(&s_db[lane * 4 + 1], colsum.y);
+                    atomicAdd(&s_db[lane * 4 + 2], colsum.z); atomicAdd(&s_db[lane * 4 + 3], colsum.w);
+                }
+                tc_fence_before();
+                __syncthreads();                 // every warp has read the accumulators; s_db is complete
+                tc_fence_after();
+                if (pr.db && tid < SCANN_D) { atomicAdd(pr.db + tid, s_db[tid]); s_db[tid] = 0.f; }
+                __syncthreads();
             }
-            tc_fence_before();
-            __syncthreads();                 // every warp has read the accumulators; s_db is complete
-            tc_fence_after();
-            if (pr.db && tid < SCANN_D) { atomicAdd(pr.db + tid, s_db[tid]); s_db[tid] = 0.f; }
-            __syncthreads();
         }
         first = true;
         colsum = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -305,22 +347,101 @@ __global__ void __launch_bounds__(WG_THREADS, 1) wgrad_batch_tc_kernel(const WgA
 
 #define WG_SMEM (WG_NIMG * 4 * WG_MNT + 1024)
 
-// problems: DEVICE array of nprob ScannWgradProblem (include/scann_b200.h).  Gradients are accumulated
-// (atomics) into dW / db, which the caller zeroes at the start of the step.
-extern "C" int scann_wgrad_batch_tc(int grid, const void* problems_dev, int nprob, const int32_t* ntiles, int tile_stride,
-                                    const int32_t* pair_c, const int32_t* pair_j, const int32_t* valid_rows,
-                                    const int32_t* valid_j, const int32_t* nvalid, void* stream) {
+// Sums the slots of every problem that several CTAs of a deterministic scann_wgrad_batch_tc_det launch of `grid` CTAs
+// shared, in CTA order, and stores the result into dW / db.  One CTA per (problem, 2048 elements of dW).
+__global__ void __launch_bounds__(256) wgrad_slot_reduce_kernel(const WgProblem* __restrict__ prob, int nprob, int grid,
+                                                                const int32_t* __restrict__ ntiles, int stride,
+                                                                const int32_t* __restrict__ nvalid,
+                                                                const float* __restrict__ slots,
+                                                                const float* __restrict__ bslots) {
+    __shared__ int s_ub, s_ue, s_total;
+    pdl_wait();
+    const int p = blockIdx.y;
+    if (threadIdx.x == 0) {
+        const int pair_rows = nvalid ? *nvalid : *ntiles * stride;
+        int run = 0, ub = 0, ue = 0;
+        for (int q = 0; q < nprob; ++q) {
+            if (q == p) ub = run;
+            const int rows = prob[q].rows >= 0 ? prob[q].rows : pair_rows;
+            run += (rows + WG_UR - 1) / WG_UR;
+            if (q == p) ue = run;
+        }
+        s_ub = ub; s_ue = ue; s_total = run;
+    }
+    __syncthreads();
+    const int ub = s_ub, ue = s_ue;
+    const long long total = s_total, G = grid;
+    if (ub >= ue) return;
+    auto lo = [&](long long c) { return (int)(total * c / G); };
+    int c0 = (int)((long long)ub * G / total);                  // the CTA whose range holds unit ub
+    while (c0 + 1 < grid && lo(c0 + 1) <= ub) ++c0;
+    while (c0 > 0 && lo(c0) > ub) --c0;
+    if (lo(c0 + 1) >= ue) return;                                // one CTA owns the problem: it stored dW itself
+    const WgProblem pr = prob[p];
+    const int i = (blockIdx.x * blockDim.x + threadIdx.x) * 8;  // 8 consecutive elements of dW per thread
+    float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, bacc = 0.f;
+    const bool bias = pr.db && blockIdx.x == 0 && threadIdx.x < SCANN_D;
+    for (int c = c0; c < grid && lo(c) < ue; ++c) {
+        if (lo(c) == lo(c + 1)) continue;                         // a CTA without units
+        const size_t slot = (size_t)c * 2 + (ub < lo(c) ? 0 : 1);
+        const float4 v0 = ld4(slots + slot * SCANN_D * SCANN_D + i), v1 = ld4(slots + slot * SCANN_D * SCANN_D + i + 4);
+        acc[0] += v0.x; acc[1] += v0.y; acc[2] += v0.z; acc[3] += v0.w;
+        acc[4] += v1.x; acc[5] += v1.y; acc[6] += v1.z; acc[7] += v1.w;
+        if (bias) bacc += bslots[slot * SCANN_D + threadIdx.x];
+    }
+    st4(pr.dW + i, make_float4(acc[0], acc[1], acc[2], acc[3]));
+    st4(pr.dW + i + 4, make_float4(acc[4], acc[5], acc[6], acc[7]));
+    if (bias) pr.db[threadIdx.x] = bacc;
+    pdl_trigger();
+}
+
+template <bool DET>
+static int wgrad_batch_launch(int grid, const void* problems_dev, int nprob, const int32_t* ntiles, int tile_stride,
+                              const int32_t* pair_c, const int32_t* pair_j, const int32_t* valid_rows,
+                              const int32_t* valid_j, const int32_t* nvalid, float* slots, float* bslots, void* stream) {
     if (nprob < 1 || nprob > WG_MAX_PROBLEMS) { scann_set_error("wgrad_batch_tc: nprob must be in 1..%d", WG_MAX_PROBLEMS); return 1; }
     if (tile_stride != 32 && tile_stride != 64 && tile_stride != 128) { scann_set_error("wgrad_batch_tc: tile_stride must be 64 or 128"); return 1; }
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(wgrad_batch_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WG_SMEM);
+        cudaError_t e = cudaFuncSetAttribute(wgrad_batch_tc_kernel<DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WG_SMEM);
         if (e != cudaSuccess) { scann_set_error("wgrad_batch_tc: smem opt-in failed: %s", cudaGetErrorString(e)); return 1; }
         configured = true;
     }
     if (grid <= 0) return 0;
     WgArgs a{(const WgProblem*)problems_dev, nprob, ntiles, tile_stride, pair_c, pair_j, valid_rows, valid_j,
-             valid_rows ? nvalid : nullptr};
-    wgrad_batch_tc_kernel<<<grid, WG_THREADS, WG_SMEM, (cudaStream_t)stream>>>(a);
+             valid_rows ? nvalid : nullptr, slots, bslots};
+    wgrad_batch_tc_kernel<DET><<<grid, WG_THREADS, WG_SMEM, (cudaStream_t)stream>>>(a);
     return scann_check_launch("scann_wgrad_batch_tc");
+}
+
+// problems: DEVICE array of nprob ScannWgradProblem (include/scann_b200.h).  Gradients are accumulated
+// (atomics) into dW / db, which the caller zeroes at the start of the step.
+extern "C" int scann_wgrad_batch_tc(int grid, const void* problems_dev, int nprob, const int32_t* ntiles, int tile_stride,
+                                    const int32_t* pair_c, const int32_t* pair_j, const int32_t* valid_rows,
+                                    const int32_t* valid_j, const int32_t* nvalid, void* stream) {
+    return wgrad_batch_launch<false>(grid, problems_dev, nprob, ntiles, tile_stride, pair_c, pair_j, valid_rows, valid_j,
+                                     nvalid, nullptr, nullptr, stream);
+}
+
+// Deterministic form: dW / db are STORED (each is written by exactly one problem); slots [grid][2][128*128] and
+// bslots [grid][2][128] hold the partial sums of the problems that several CTAs share, which
+// scann_wgrad_batch_reduce (same grid, table and plan) adds up afterwards.
+extern "C" int scann_wgrad_batch_tc_det(int grid, const void* problems_dev, int nprob, const int32_t* ntiles, int tile_stride,
+                                        const int32_t* pair_c, const int32_t* pair_j, const int32_t* valid_rows,
+                                        const int32_t* valid_j, const int32_t* nvalid, float* slots, float* bslots,
+                                        void* stream) {
+    if (!slots || !bslots) { scann_set_error("wgrad_batch_tc_det: slots and bslots are required"); return 1; }
+    return wgrad_batch_launch<true>(grid, problems_dev, nprob, ntiles, tile_stride, pair_c, pair_j, valid_rows, valid_j,
+                                    nvalid, slots, bslots, stream);
+}
+
+extern "C" int scann_wgrad_batch_reduce(int grid, const void* problems_dev, int nprob, const int32_t* ntiles, int tile_stride,
+                                        const int32_t* valid_rows, const int32_t* nvalid, const float* slots,
+                                        const float* bslots, void* stream) {
+    if (nprob < 1 || nprob > WG_MAX_PROBLEMS) { scann_set_error("wgrad_batch_reduce: nprob must be in 1..%d", WG_MAX_PROBLEMS); return 1; }
+    if (grid <= 0) return 0;
+    scann_launch(wgrad_slot_reduce_kernel, dim3(SCANN_D * SCANN_D / (256 * 8), nprob), dim3(256), 0, stream,
+                 (const WgProblem*)problems_dev, nprob, grid, ntiles, tile_stride, valid_rows ? nvalid : (const int32_t*)nullptr,
+                 slots, bslots);
+    return scann_check_launch("scann_wgrad_batch_reduce");
 }

@@ -31,6 +31,17 @@ ERR_BITS = {1: "plan tile capacity exceeded", 2: "an atom has more than 128 vali
             16: "a bounded mbarrier wait of a pipelined kernel (local attention, chained Dense) gave up"}
 
 
+def deterministic_mode(deterministic: Optional[bool] = None, environ=None) -> bool:
+    """Whether an engine trains in the deterministic mode (DESIGN.md section 4.7).  An explicit ``deterministic``
+    wins; None reads the environment: ``SCANN_DETERMINISTIC=1``, or the reference's own switch
+    ``TF_DETERMINISTIC_OPS`` set to ``1`` / ``true`` (the reference's train.py:16-25 sets it)."""
+    if deterministic is not None:
+        return bool(deterministic)
+    env = os.environ if environ is None else environ
+    return (env.get("SCANN_DETERMINISTIC", "0") == "1"
+            or env.get("TF_DETERMINISTIC_OPS", "").strip().lower() in ("1", "true"))
+
+
 def _p(t: Optional[torch.Tensor], off_elems: int = 0) -> int:
     if t is None:
         return 0
@@ -49,8 +60,11 @@ class Batch:
 
 class Engine:
     def __init__(self, spec: ModelSpec, arena: Optional[np.ndarray] = None, device: Optional[torch.device] = None,
-                 seed: int = 1):
+                 seed: int = 1, deterministic: Optional[bool] = None):
+        """``deterministic``: bitwise-reproducible train steps (DESIGN.md section 4.7); None reads the environment
+        (``deterministic_mode``).  Fixed for the life of the engine."""
         check_kernel_support(spec)
+        self.deterministic = deterministic_mode(deterministic)
         self.sm_count = _abi.require_gpu()
         self.device = device or torch.device("cuda", torch.cuda.current_device())
         self.spec = spec
@@ -164,6 +178,35 @@ class Engine:
         self._wimg_dirty = True
         # every weight-gradient GEMM of the step in one persistent launch at the end of the backward pass
         self.use_wgrad_batch = os.environ.get("SCANN_WGRAD_BATCH", "1") == "1" and self.use_chain and self.tc_la_bwd
+        self._nccl_warned = False
+
+    # ------------------------------------------------------------------ deterministic mode
+    def _check_deterministic_support(self) -> None:
+        """The deterministic mode exists for the default engine only: refuse every setting it cannot guarantee.  (Checked
+        when training starts: inference is deterministic with every setting.)"""
+        why = None
+        if not (self.tc_dense and self.tc_la_fwd and self.tc_la_bwd):
+            why = "the SIMT / round-1 kernels (SCANN_ENGINE=simt, SCANN_DENSE, SCANN_LA_FWD, SCANN_LA_BWD)"
+        elif not self.use_chain or not self.use_chain2:
+            why = "the unchained engine (SCANN_CHAIN=0 / SCANN_CHAIN2=0)"
+        elif not self.use_wgrad_batch:
+            why = "the per-layer weight-gradient kernels (SCANN_WGRAD_BATCH=0)"
+        elif self.la_pipe != self.la_pipe_built:
+            why = "the round-1 local-attention kernels (SCANN_LA_PIPE other than 15)"
+        elif not self.noup_pipe:
+            why = "the round-1 local-attention kernels (SCANN_NOUP_PIPE=0)"
+        elif self.tile_stride_pref not in (0, 32):
+            why = "tile slots other than 32 rows (SCANN_TILE_STRIDE)"
+        elif self._skip:
+            why = "SCANN_DEBUG_SKIP"
+        if why is not None:
+            raise NotImplementedError("deterministic mode is not available with " + why)
+
+    def _check_deterministic_batch(self, b: "Batch") -> None:
+        if b.stride != 32:
+            raise NotImplementedError(
+                f"deterministic mode needs the 32-row pipelined pair plan: this batch has up to {b.N} neighbours per "
+                "atom (at most 32 are supported)")
 
     # ------------------------------------------------------------------ helpers
     def _ev(self, name: str, begin: bool) -> None:
@@ -460,6 +503,7 @@ class Engine:
         # 4 ints per plan group (four-kernel form) + the 64-bit look-back words of the one-launch form, which rely
         # on the buffer being zero when it is first used (scann_plan_build)
         b.scratch = torch.zeros(6 * ngroups + 16, **i32)
+        b.inv_ptr = None            # inverse neighbour CSR (deterministic mode, scann_plan_inverse)
         b.graphs = {}
         return b
 
@@ -524,6 +568,16 @@ class Engine:
                                    self._stream()), "plan_build")
         # one launch (look-back over the plan groups), or count / group / scan / fill with SCANN_LA4 bit 5
         self.launches += 4 if (self.la_groups4 & 32) else 1
+        if self.deterministic and b.stride == 32:
+            if b.inv_ptr is None:
+                i32 = dict(dtype=torch.int32, device=self.device)
+                b.inv_ptr = torch.empty(b.R + 1, **i32)
+                b.inv_idx = torch.empty(b.rows, **i32)
+                b.inv_cnt = torch.empty(b.R, **i32)
+                b.inv_tmp = torch.empty(b.rows, **i32)
+            check(lib.scann_plan_inverse(_p(b.ntiles), b.stride, b.rows, _p(b.pair_c), _p(b.pair_j), b.R, _p(b.inv_ptr),
+                                         _p(b.inv_idx), _p(b.inv_cnt), _p(b.inv_tmp), self._stream()), "plan_inverse")
+            self.launches += 4
 
     # ------------------------------------------------------------------ workspaces
     def _workspace(self, b: Batch, training: bool) -> dict:
@@ -572,12 +626,92 @@ class Engine:
             ws["dy"] = torch.empty(b.B, **f)
             ws["wpart"] = torch.empty(self.la_grid, 2, D, D, **f)
             ws["G"] = torch.empty(self.spec.n_atoms + 3, D, **f)
+        if training and self.deterministic:
+            self._det_workspace(b, ws)
         ws["xa"] = torch.empty(R, D, **f)
         ws["qk"] = torch.empty(R, 2 * D, **f)
         ws["ga"] = torch.empty(R, **f)
         ws["y"] = torch.empty(b.B, **f)
         self._ws[key] = ws
         return ws
+
+    def _det_workspace(self, b: Batch, ws: dict) -> None:
+        """Per-pair buffer and per-CTA slot arrays of the deterministic mode, and the table of slot arrays that
+        scann_slot_reduce adds into the gradient arena before the optimiser."""
+        sp, dev = self.spec, self.device
+        L, R, G = sp.n_attention, b.R, self.la_grid
+        f = dict(dtype=torch.float32, device=dev)
+        ws["pairbuf"] = torch.empty(b.rows, D, **f)                   # d_a * g' per pair, reused by every layer
+        ws["dbk_slots"] = torch.empty(L, G, D, **f)
+        if sp.g_update:
+            ws["lng_slots"] = torch.empty(L, G, 2 * D, **f)           # layer_norm_g gamma | beta
+        # CTAs of the chained launches over R rows: the warp-specialised form up to one wave, else the round-1 form
+        cg = (lib.scann_dense_chain2_grid(R) if self.use_chain2 and R <= self.chain2_max_rows
+              else lib.scann_dense_chain_grid(R))
+        ws["ln_slots"] = torch.empty(L, 2, 2, cg, D, **f)             # [layer][layer_norm, residual_norm][gamma, beta]
+        ws["wg_slots"] = torch.empty(G, 2, D * D, **f)
+        ws["wg_bslots"] = torch.empty(G, 2, D, **f)
+        gi = G * self.gi_bwd_mult
+        gslot = 2 * N_RBF * D + 2 * D                                  # geometry initialisation: dWd | dWw | dbd | dbw
+        nslot = (N_RBF + 1) * D                                        # g_update=False filter: dWf | dbf
+        if sp.g_update:
+            ws["gi_slots"] = torch.empty(2 * gi, gslot, **f)
+        else:
+            ws["noup_slots"] = torch.empty(L, 2 * gi, nslot, **f)
+        kin = sp.embedding_dim + (10 if sp.use_ring else 0)
+        if sp.feature == "cgcnn":
+            ws["cg_slots"] = torch.empty((R + 31) // 32, (kin + 1) * D, **f)    # dense_embed kernel rows | bias
+        else:
+            ns = lib.scann_embed_backward_det_slots(R)
+            ws["emb_slots"] = torch.empty(ns, sp.n_atoms + 3, D, **f)
+        ws["head_slots"] = torch.empty(b.B, D, **f)                   # predict_property kernel, per structure
+        ws["head_bslots"] = torch.empty(b.B, **f)                     # predict_property bias, per structure
+        ws["reg_slots"] = torch.empty(1184, **f)
+        ents = []
+
+        def add(slots: torch.Tensor, nslots: int, count: int, ld: int, dst: int, off: int = 0) -> None:
+            e = _abi.SlotSum()
+            e.slots, e.dst, e.nslots, e.count, e.ld, e.pad = _p(slots, off), dst, nslots, count, ld, 0
+            ents.append(e)
+
+        for l in range(L):
+            la = layer_name("local_attention", l)
+            rn = layer_name("residual_norm", l)
+            add(ws["dbk_slots"][l], G, D, D, self.gw(f"{la}/key/bias"))
+            if sp.g_update:
+                add(ws["lng_slots"][l], G, D, 2 * D, self.gw(f"{la}/layer_norm_g/gamma"))
+                add(ws["lng_slots"][l], G, D, 2 * D, self.gw(f"{la}/layer_norm_g/beta"), D)
+            else:
+                add(ws["noup_slots"][l], 2 * gi, N_RBF * D, nslot, self.gw(f"{la}/filter_geo/kernel"))
+                add(ws["noup_slots"][l], 2 * gi, D, nslot, self.gw(f"{la}/filter_geo/bias"), N_RBF * D)
+            add(ws["ln_slots"][l, 0, 0], cg, D, D, self.gw(f"{la}/layer_norm/gamma"))
+            add(ws["ln_slots"][l, 0, 1], cg, D, D, self.gw(f"{la}/layer_norm/beta"))
+            if sp.use_attn_norm:
+                add(ws["ln_slots"][l, 1, 0], cg, D, D, self.gw(f"{rn}/layer_norm/gamma"))
+                add(ws["ln_slots"][l, 1, 1], cg, D, D, self.gw(f"{rn}/layer_norm/beta"))
+        if sp.g_update:
+            gs = ws["gi_slots"]
+            add(gs, 2 * gi, N_RBF * D, gslot, self.gw("neighbor_d/kernel"))
+            add(gs, 2 * gi, N_RBF * D, gslot, self.gw("neighbor_w/kernel"), N_RBF * D)
+            add(gs, 2 * gi, D, gslot, self.gw("neighbor_d/bias"), 2 * N_RBF * D)
+            add(gs, 2 * gi, D, gslot, self.gw("neighbor_w/bias"), 2 * N_RBF * D + D)
+        if sp.feature == "cgcnn":
+            cs = ws["cg_slots"]
+            add(cs, cs.shape[0], kin * D, (kin + 1) * D, self.gw("dense_embed/kernel"))
+            add(cs, cs.shape[0], D, (kin + 1) * D, self.gw("dense_embed/bias"), kin * D)
+        add(ws["head_slots"], b.B, D, D, self.gw("predict_property/kernel"))
+        add(ws["head_bslots"], b.B, 1, 1, self.gw("predict_property/bias"))
+        arr = (_abi.SlotSum * len(ents))(*ents)
+        ws["slot_table"] = torch.frombuffer(bytearray(bytes(arr)), dtype=torch.uint8).to(dev)
+        ws["slot_count"] = len(ents)
+        ws["slot_max"] = max(e.count for e in ents)
+
+    def _ln_grads(self, ws: dict, l: int, which: int, name: str) -> dict:
+        """dgamma / dbeta of a LayerNorm-backward chain step: the gradient arena, or the slot arrays of the deterministic
+        mode (which: 0 the attention output's LayerNorm, 1 the ResidualNorm's)."""
+        if self.deterministic:
+            return dict(dgamma=_p(ws["ln_slots"][l, which, 0]), dbeta=_p(ws["ln_slots"][l, which, 1]))
+        return dict(dgamma=self.gw(f"{name}/layer_norm/gamma"), dbeta=self.gw(f"{name}/layer_norm/beta"))
 
     # ------------------------------------------------------------------ thin kernel wrappers
     def _dense(self, A, lda, W, bias, kblk, nblk, R, C, ldc, mode=0, resid=None, ldres=D, pre_in=None, pre_out=None,
@@ -616,12 +750,13 @@ class Engine:
                 for kb in range(s.kblk):
                     s.W[kb] = self._wimg_ptr(s.W[kb])
             arr = (ChainStep * len(steps))(*steps)
-            check(lib.scann_dense_chain2(ctypes.cast(arr, ctypes.c_void_p), len(steps), R, _p(self.status), self._stream()),
-                  "dense_chain2")
+            fn = lib.scann_dense_chain2_det if self.deterministic else lib.scann_dense_chain2
+            check(fn(ctypes.cast(arr, ctypes.c_void_p), len(steps), R, _p(self.status), self._stream()), "dense_chain2")
             self.launches += 1
             return
         arr = (ChainStep * len(steps))(*steps)
-        check(lib.scann_dense_chain(ctypes.cast(arr, ctypes.c_void_p), len(steps), R, self._stream()), "dense_chain")
+        fn = lib.scann_dense_chain_det if self.deterministic else lib.scann_dense_chain
+        check(fn(ctypes.cast(arr, ctypes.c_void_p), len(steps), R, self._stream()), "dense_chain")
         self.launches += 1
 
     def _wgrad(self, A, lda, G, ldg, kblk, nblk, R, dW, db):
@@ -958,13 +1093,16 @@ class Engine:
             self._backward_prep(ws, st)
             ws["scat_all"].zero_()
         self._pdl(False)
-        check(lib.scann_rmse_prepare(_p(ws["y"]), _p(target), b.B, _p(ws["dy"]), _p(self.grads, n), st), "rmse_prepare")
+        det = self.deterministic
+        check((lib.scann_rmse_prepare_det if det else lib.scann_rmse_prepare)(
+            _p(ws["y"]), _p(target), b.B, _p(ws["dy"]), _p(self.grads, n), st), "rmse_prepare")
         self._pdl(True)
         self._ev("ga_backward", True)
-        check(lib.scann_ga_head_backward(_p(ws["qk"]), _p(b.atom_mask), b.B, b.M, int(sp.use_ga_norm),
-                                         self.wT("bf_property/kernel"), self.w("predict_property/kernel"),
-                                         _p(ws["tb"]), _p(ws["dy"]), _p(ws["d_qk"]), _p(ws["d_tb"]),
-                                         self.gw("predict_property/kernel"), self.gw("predict_property/bias"), st),
+        head = (_p(ws["head_slots"]), _p(ws["head_bslots"])) if det else \
+            (self.gw("predict_property/kernel"), self.gw("predict_property/bias"))
+        check((lib.scann_ga_head_backward_det if det else lib.scann_ga_head_backward)(
+            _p(ws["qk"]), _p(b.atom_mask), b.B, b.M, int(sp.use_ga_norm), self.wT("bf_property/kernel"),
+            self.w("predict_property/kernel"), _p(ws["tb"]), _p(ws["dy"]), _p(ws["d_qk"]), _p(ws["d_tb"]), *head, st),
               "ga_head_backward")
         self._ev("ga_backward", False)
         self.launches += 2
@@ -1077,35 +1215,45 @@ class Engine:
                 ev.record(main)
                 side.wait_event(ev)
                 gst = side.cuda_stream
-            check(lib.scann_geom_init_backward(_p(b.ntiles), self.la_grid * self.gi_bwd_mult, b.stride, _p(b.pair_c), _p(b.pair_d), _p(b.pair_w),
-                                               _p(self.centers_d), _p(self.centers_w), self.w("neighbor_d/kernel"),
-                                               self.w("neighbor_d/bias"), self.w("neighbor_w/kernel"),
-                                               self.w("neighbor_w/bias"), _p(dg_up), self.gw("neighbor_d/kernel"),
-                                               self.gw("neighbor_d/bias"), self.gw("neighbor_w/kernel"),
-                                               self.gw("neighbor_w/bias"), gst), "geom_init_backward")
+            if self.deterministic:
+                check(lib.scann_geom_init_backward_det(
+                    _p(b.ntiles), self.la_grid * self.gi_bwd_mult, b.stride, _p(b.pair_c), _p(b.pair_d), _p(b.pair_w),
+                    _p(self.centers_d), _p(self.centers_w), self.w("neighbor_d/kernel"), self.w("neighbor_d/bias"),
+                    self.w("neighbor_w/kernel"), self.w("neighbor_w/bias"), _p(dg_up), _p(ws["gi_slots"]), gst),
+                      "geom_init_backward_det")
+            else:
+                check(lib.scann_geom_init_backward(_p(b.ntiles), self.la_grid * self.gi_bwd_mult, b.stride, _p(b.pair_c), _p(b.pair_d), _p(b.pair_w),
+                                                   _p(self.centers_d), _p(self.centers_w), self.w("neighbor_d/kernel"),
+                                                   self.w("neighbor_d/bias"), self.w("neighbor_w/kernel"),
+                                                   self.w("neighbor_w/bias"), _p(dg_up), self.gw("neighbor_d/kernel"),
+                                                   self.gw("neighbor_d/bias"), self.gw("neighbor_w/kernel"),
+                                                   self.gw("neighbor_w/bias"), gst), "geom_init_backward")
         E = sp.embedding_dim
         ring = sp.use_ring
         if sp.feature == "cgcnn":
-            check(lib.scann_cgcnn_embed_backward(
+            # deterministic mode: dense_embed's gradients go to per-CTA slots (scann_slot_reduce)
+            dense = (_p(ws["cg_slots"]),) if self.deterministic else \
+                (self.gw("dense_embed/kernel"), self.gw("dense_embed/bias"))
+            check((lib.scann_cgcnn_embed_backward_det if self.deterministic else lib.scann_cgcnn_embed_backward)(
                 _p(b.atomic92), _p(ws["emb_rows"]), _p(b.ring) if ring else 0, R, 92, E,
                 self.w("extra_embed/kernel") if ring else 0, self.w("extra_embed/bias") if ring else 0,
                 self.w("dense_embed/kernel"), _p(ws["t0"]), _p(dx), _p(ws["d_cat"]), self.gw("embed_atom/kernel"),
                 self.gw("embed_atom/bias"), self.gw("extra_embed/kernel") if ring else 0,
-                self.gw("extra_embed/bias") if ring else 0, self.gw("dense_embed/kernel"), self.gw("dense_embed/bias"),
-                _p(self.adam_scalars, 8), st), "cgcnn_embed_backward")
+                self.gw("extra_embed/bias") if ring else 0, *dense, _p(self.adam_scalars, 8), st), "cgcnn_embed_backward")
             self.launches += 2
             if side is not main:
                 ev = torch.cuda.Event()
                 ev.record(side)
                 main.wait_event(ev)
             return
-        check(lib.scann_embed_backward(_p(b.atomic), _p(b.ring) if ring else 0, R, E, sp.n_atoms,
-                                       self.w("embed_atom/embeddings"), self.w("extra_embed/kernel") if ring else 0,
-                                       self.w("extra_embed/bias") if ring else 0,
-                                       self.w("dense_embed/kernel"), _p(ws["t0"]), _p(dx), _p(ws["G"]),
-                                       self.gw("embed_atom/embeddings"), self.gw("extra_embed/kernel") if ring else 0,
-                                       self.gw("extra_embed/bias") if ring else 0, self.gw("dense_embed/kernel"),
-                                       self.gw("dense_embed/bias"), _p(self.adam_scalars, 8), st), "embed_backward")
+        Gslots = (_p(ws["emb_slots"]),) if self.deterministic else ()
+        check((lib.scann_embed_backward_det if self.deterministic else lib.scann_embed_backward)(
+            _p(b.atomic), _p(b.ring) if ring else 0, R, E, sp.n_atoms, self.w("embed_atom/embeddings"),
+            self.w("extra_embed/kernel") if ring else 0, self.w("extra_embed/bias") if ring else 0,
+            self.w("dense_embed/kernel"), _p(ws["t0"]), _p(dx), _p(ws["G"]), *Gslots,
+            self.gw("embed_atom/embeddings"), self.gw("extra_embed/kernel") if ring else 0,
+            self.gw("extra_embed/bias") if ring else 0, self.gw("dense_embed/kernel"), self.gw("dense_embed/bias"),
+            _p(self.adam_scalars, 8), st), "embed_backward")
         self.launches += 4
         if side is not main:             # join: the optimiser needs every weight gradient
             ev = torch.cuda.Event()
@@ -1127,8 +1275,7 @@ class Engine:
             la = layer_name("local_attention", l)
             rn = layer_name("residual_norm", l)
             la_ln = dict(mode=4, pre_in=_p(ws["ctxpre"][l]), gamma=self.w(f"{la}/layer_norm/gamma"),
-                         dgamma=self.gw(f"{la}/layer_norm/gamma"), dbeta=self.gw(f"{la}/layer_norm/beta"),
-                         C_=_p(ws["d_ctx"]), C2=_p(ws["dq"][l]))
+                         **self._ln_grads(ws, l, 0, la), C_=_p(ws["d_ctx"]), C2=_p(ws["dq"][l]))
             if not sp.use_attn_norm:
                 return [chain_step(**head, **la_ln)]
             d_v2, d_t1 = ws["d_v2"][l], ws["d_t1"][l]
@@ -1136,8 +1283,7 @@ class Engine:
                 # d_v2 (residual branch) and d_v2 * dropout mask (gradient of the dense_1 output, also the operand
                 # of the next step and of the dense_1 weight gradient)
                 chain_step(**head, mode=4, pre_in=_p(ws["v2"][l]), gamma=self.w(f"{rn}/layer_norm/gamma"),
-                           dgamma=self.gw(f"{rn}/layer_norm/gamma"), dbeta=self.gw(f"{rn}/layer_norm/beta"),
-                           C_=_p(d_v2), C2=_p(ws["d_v2m"][l]), to_image=True,
+                           **self._ln_grads(ws, l, 1, rn), C_=_p(d_v2), C2=_p(ws["d_v2m"][l]), to_image=True,
                            drop=_p(self.adam_scalars, 8), drop_site=1 + l),
                 chain_step(W=[self.wT(f"{rn}/dense_1/kernel")], mode=2, pre_in=_p(ws["t1"][l]), C_=_p(d_t1), to_image=True),
                 chain_step(W=[self.wT(f"{rn}/dense/kernel")], resid=_p(d_v2), **la_ln),
@@ -1171,7 +1317,14 @@ class Engine:
             self._ev("la_backward", True)
             if not sp.g_update:
                 # SCANN without geometry update: attention part only, then the filter_geo [20,128] gradient
-                if self.noup_pipe and b.stride == 32:
+                if self.deterministic:
+                    # d_a * g' stored per pair, summed per atom row in list order behind the filter gradient
+                    check(lib.scann_la_backward_pipe_det(
+                        self.la_grid, b.rows, 1, _p(b.ntiles), _p(b.pair_c), _p(b.pair_j), _p(ws["x"][l]), _p(ws["proj"][l]),
+                        0, _p(ws["gsave"][l]), _p(ws["kk"][l]), 0, 0, self.wT(f"{la}/key/kernel"), 0, _p(ws["d_ctx"]),
+                        _p(ws["dg"][0]), 0, 0, _p(dq), 0, 0, _p(ws["pairbuf"]), 0, 0, _p(ws["dbk_slots"][l]),
+                        *self._adrop(True, l), _p(self.status), st), "la_backward_pipe_det")
+                elif self.noup_pipe and b.stride == 32:
                     check(lib.scann_la_backward_pipe(
                         self.la_grid, b.rows, 1, _p(b.ntiles), _p(b.pair_c), _p(b.pair_j), _p(ws["x"][l]), _p(ws["proj"][l]),
                         0, _p(ws["gsave"][l]), _p(ws["kk"][l]), 0, 0, self.wT(f"{la}/key/kernel"), 0, _p(ws["d_ctx"]),
@@ -1183,10 +1336,19 @@ class Engine:
                         _p(b.pair_c), _p(b.pair_j), _p(ws["x"][l]), _p(ws["proj"][l]), _p(ws["gsave"][l]), _p(ws["kk"][l]),
                         self.wT(f"{la}/key/kernel"), _p(ws["d_ctx"]), _p(ws["dg"][0]), _p(dq), _p(dx_sc),
                         self.gw(f"{la}/key/bias"), *self._adrop(True, l), st), "la_backward_noupdate_tc")
-                check(lib.scann_noupdate_geom_backward(
-                    _p(b.ntiles), self.la_grid * self.gi_bwd_mult, b.stride, _p(b.pair_c), _p(b.pair_d), _p(b.pair_w), _p(self.centers_d),
-                    self.w(fg), self.w(f"{la}/filter_geo/bias"), _p(ws["dg"][0]), self.gw(fg),
-                    self.gw(f"{la}/filter_geo/bias"), st), "noupdate_geom_backward")
+                if self.deterministic:
+                    check(lib.scann_noupdate_geom_backward_det(
+                        _p(b.ntiles), self.la_grid * self.gi_bwd_mult, b.stride, _p(b.pair_c), _p(b.pair_d), _p(b.pair_w),
+                        _p(self.centers_d), self.w(fg), self.w(f"{la}/filter_geo/bias"), _p(ws["dg"][0]),
+                        _p(ws["noup_slots"][l]), st), "noupdate_geom_backward_det")
+                    check(lib.scann_row_gather(R, _p(b.inv_ptr), _p(b.inv_idx), _p(ws["pairbuf"]), _p(dx_sc), 0, 0, st),
+                          "row_gather")
+                    self.launches += 1
+                else:
+                    check(lib.scann_noupdate_geom_backward(
+                        _p(b.ntiles), self.la_grid * self.gi_bwd_mult, b.stride, _p(b.pair_c), _p(b.pair_d), _p(b.pair_w), _p(self.centers_d),
+                        self.w(fg), self.w(f"{la}/filter_geo/bias"), _p(ws["dg"][0]), self.gw(fg),
+                        self.gw(f"{la}/filter_geo/bias"), st), "noupdate_geom_backward")
                 self.launches += 2
             elif "la_bwd" not in self._skip:
                 plan_args = (_p(b.ntiles), _p(b.tile_a0), _p(b.tile_a1), _p(b.cnt), _p(b.rowptr), _p(b.pair_c), _p(b.pair_j))
@@ -1196,7 +1358,18 @@ class Engine:
                         _p(dg_out), _p(dq), _p(s_pre), _p(t_sc), _p(dx_sc))
                 grads = (self.gw(f"{la}/layer_norm_g/gamma"), self.gw(f"{la}/layer_norm_g/beta"), self.gw(f"{la}/key/bias"))
                 pipe = (self.la_pipe >> 2) & 3 if b.stride == 32 else 0
-                for part in (1, 2):                   # attention kernel, then geometry kernel: pipelined or round-1 form
+                if self.deterministic:
+                    # d_a * g' stored per pair, d_pre left per pair in pre[l]; both summed per atom row in list order
+                    data = data[:-1] + (_p(ws["pairbuf"]),)
+                    grads = (_p(ws["lng_slots"][l]), 0, _p(ws["dbk_slots"][l]))
+                    check(lib.scann_la_backward_pipe_det(self.la_grid, b.rows, 3, plan_args[0], plan_args[5], plan_args[6],
+                                                         *data, *grads, *self._adrop(True, l), _p(self.status), st),
+                          "la_backward_pipe_det")
+                    check(lib.scann_row_gather(R, _p(b.inv_ptr), _p(b.inv_idx), _p(ws["pairbuf"]), _p(dx_sc),
+                                               _p(ws["pre"][l]), _p(t_sc), st), "row_gather")
+                    pipe = 0
+                    self.launches += 1
+                for part in ((1, 2) if not self.deterministic else ()):   # attention kernel, then geometry kernel
                     if pipe & part:
                         check(lib.scann_la_backward_pipe(self.la_grid, b.rows, part, plan_args[0], plan_args[5], plan_args[6],
                                                          *data, *grads, *self._adrop(True, l), _p(self.status), st),
@@ -1236,8 +1409,17 @@ class Engine:
             table, count = self._wgrad_table(b, ws)
             self._pdl(False)
             self._ev("wgrad_batch", True)
-            check(lib.scann_wgrad_batch_tc(self.la_grid, _p(table), count, _p(b.ntiles), b.stride, _p(b.pair_c),
-                                           _p(b.pair_j), _p(b.valid_rows), _p(b.valid_j), _p(b.nvalid), st),
+            if self.deterministic:
+                check(lib.scann_wgrad_batch_tc_det(self.la_grid, _p(table), count, _p(b.ntiles), b.stride, _p(b.pair_c),
+                                                   _p(b.pair_j), _p(b.valid_rows), _p(b.valid_j), _p(b.nvalid),
+                                                   _p(ws["wg_slots"]), _p(ws["wg_bslots"]), st), "wgrad_batch_tc_det")
+                check(lib.scann_wgrad_batch_reduce(self.la_grid, _p(table), count, _p(b.ntiles), b.stride,
+                                                   _p(b.valid_rows), _p(b.nvalid), _p(ws["wg_slots"]),
+                                                   _p(ws["wg_bslots"]), st), "wgrad_batch_reduce")
+                self.launches += 1
+            else:
+                check(lib.scann_wgrad_batch_tc(self.la_grid, _p(table), count, _p(b.ntiles), b.stride, _p(b.pair_c),
+                                               _p(b.pair_j), _p(b.valid_rows), _p(b.valid_j), _p(b.nvalid), st),
                       "wgrad_batch_tc")
             self._ev("wgrad_batch", False)
             self.launches += 1
@@ -1378,6 +1560,14 @@ class Engine:
 
     def _train_body(self, b: Batch, allreduce, apply: bool, want_grads: bool, replan: bool, exchange: bool = True) -> None:
         p2p = self.p2p if exchange else None
+        if self.deterministic:
+            self._check_deterministic_support()
+            self._check_deterministic_batch(b)
+            if allreduce is not None and not self._nccl_warned:
+                import warnings
+                warnings.warn("deterministic mode: the cross-rank gradient sum of the NCCL all-reduce runs in NCCL's "
+                              "order, which this package does not control", RuntimeWarning)
+                self._nccl_warned = True
         if self.p2p is not None:
             # no peer still reads the arena that is zeroed next (scann_b200/csrc/p2p.cu); also in the local warm pass
             check(lib.scann_p2p_begin_step(_p(self.p2p.block), _p(self.p2p.sums), self._stream()), "p2p_begin_step")
@@ -1397,20 +1587,38 @@ class Engine:
         self.forward(b, training=True, replan=replan, side_work=prep)
         self.backward(b, b.target)
         n = self.layout.total
+        if self.deterministic:
+            self._pdl(False)
+            check(lib.scann_slot_reduce(_p(ws["slot_table"]), ws["slot_count"], ws["slot_max"], self._stream()),
+                  "slot_reduce")
+            self.launches += 1
         if p2p is not None:
-            check(lib.scann_adam_p2p_step(_p(self.params), _p(self.adam_m), _p(self.adam_v), _p(self.l2mask), n,
-                                          _p(self.p2p.block), _p(self.p2p.sums), _p(self.adam_scalars),
-                                          _p(self.grad_out) if want_grads else 0, int(apply), self._stream()),
-                  "adam_p2p_step")
+            if self.deterministic:
+                check(lib.scann_adam_p2p_step_det(_p(self.params), _p(self.adam_m), _p(self.adam_v), _p(self.l2mask), n,
+                                                  _p(self.p2p.block), _p(self.p2p.sums), _p(self.adam_scalars),
+                                                  _p(self.grad_out) if want_grads else 0, int(apply), _p(ws["reg_slots"]),
+                                                  self._stream()), "adam_p2p_step_det")
+            else:
+                check(lib.scann_adam_p2p_step(_p(self.params), _p(self.adam_m), _p(self.adam_v), _p(self.l2mask), n,
+                                              _p(self.p2p.block), _p(self.p2p.sums), _p(self.adam_scalars),
+                                              _p(self.grad_out) if want_grads else 0, int(apply), self._stream()),
+                      "adam_p2p_step")
             self.launches += 1
             return
         if allreduce is not None and exchange:
             # (not in the local warm-up pass of a new shape class, whose result is discarded: ranks that meet new
             # shapes at different steps must still issue the same number of collectives)
             allreduce(self.grads)
-        check(lib.scann_adam_step(_p(self.params), _p(self.grads), _p(self.adam_m), _p(self.adam_v), _p(self.l2mask), n,
-                                  _p(self.grads, n), _p(self.adam_scalars), _p(self.grad_out) if want_grads else 0,
-                                  int(apply), self._stream()), "adam_step")
+        if self.deterministic:
+            check(lib.scann_adam_step_det(_p(self.params), _p(self.grads), _p(self.adam_m), _p(self.adam_v), _p(self.l2mask),
+                                          n, _p(self.grads, n), _p(self.adam_scalars),
+                                          _p(self.grad_out) if want_grads else 0, int(apply), _p(ws["reg_slots"]),
+                                          self._stream()), "adam_step_det")
+            self.launches += 1
+        else:
+            check(lib.scann_adam_step(_p(self.params), _p(self.grads), _p(self.adam_m), _p(self.adam_v), _p(self.l2mask), n,
+                                      _p(self.grads, n), _p(self.adam_scalars), _p(self.grad_out) if want_grads else 0,
+                                      int(apply), self._stream()), "adam_step")
         self.launches += 1
 
     def predict_step(self, b: Batch, replan: bool = False):

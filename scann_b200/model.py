@@ -140,10 +140,11 @@ class ScannKerasModel:
     input_names = ["atomic", "atom_mask", "neighbors", "neighbor_mask", "neighbor_weight", "neighbor_distance"]
 
     def __init__(self, spec: ModelSpec, arena: Optional[np.ndarray] = None, infer: bool = False, seed: int = 1,
-                 device: Optional[torch.device] = None):
+                 device: Optional[torch.device] = None, deterministic: Optional[bool] = None):
         self.spec = spec
         self.infer = infer
-        self.engine = Engine(spec, arena, device=device, seed=seed)
+        # deterministic: bitwise-reproducible training (Engine); None = SCANN_DETERMINISTIC / TF_DETERMINISTIC_OPS
+        self.engine = Engine(spec, arena, device=device, seed=seed, deterministic=deterministic)
         self.layout: ParamLayout = self.engine.layout
         self.lr = 1e-3
         self.allreduce = None
@@ -384,9 +385,10 @@ class ScannKerasModel:
         return self
 
 
-def create_model(config: dict, seed: int = 1, infer: bool = False, arena: Optional[np.ndarray] = None) -> ScannKerasModel:
-    """Counterpart of ``create_model(config)`` (scann_model.py:329-453)."""
-    return ScannKerasModel(model_spec(config), arena=arena, infer=infer, seed=seed)
+def create_model(config: dict, seed: int = 1, infer: bool = False, arena: Optional[np.ndarray] = None,
+                 deterministic: Optional[bool] = None) -> ScannKerasModel:
+    """Counterpart of ``create_model(config)`` (scann_model.py:329-453).  ``deterministic``: see ``Engine``."""
+    return ScannKerasModel(model_spec(config), arena=arena, infer=infer, seed=seed, deterministic=deterministic)
 
 
 class SCANN:
