@@ -384,6 +384,31 @@ int scann_voronoi_neighbors(const double* lattice, const double* coords, const i
                             int n_centres, int allow_pathological, int cap, void* slots, int32_t* slot_count,
                             void* blob, void* host_blob, int32_t* status, void* stream);
 
+/* ---- Voronoi facets -> the model's batch, on the device ----------------------------------------------------------
+ * Replaces the host steps between the cell search and the padded input: the per-site thresholding of
+ * compute_voronoi_neighbor (scann/utils/voronoi_neighbor.py:11-61), the neighbour-list half of prepare_input_pmt
+ * (scann/utils/general.py:206-246) and the CSR batch DataIterator builds (scann/utils/datagenerator.py:69-135).
+ * scann_voronoi_select reads the blob of scann_voronoi_neighbors (n_centres centres) and, for every centre c, orders
+ * its records by (distance, site, n0, n1, n2) -- fp64 distance, image components decoded -- keeps those with
+ * distance <= d_thresh and normalized >= w_thresh (fp64) and writes them to row r = centre_row[c] of the staging arrays:
+ * sel_count[r], and at r * 64 + i: sel_idx = site, sel_w = (float)solid_angle (weight_column 0) or (float)normalized
+ * (weight_column 1), sel_d = (float)distance, all rounded to nearest.  One warp per centre, rank by counting; a centre
+ * whose cell was dropped (flag 1 without allow_pathological) has no record and writes count 0.
+ * status |= SCANN_ERR_VORONOI_CAPACITY if a centre has more than 64 records.
+ * scann_voronoi_batch_csr writes structures s0 .. s0 + n_structs - 1 (struct_atom_off [S+1] and z [A] over the same
+ * atom rows as the staging arrays; atom0 = struct_atom_off[s0] and n_atoms, known to the caller) as the CSR batch of
+ * scann_pack_batch into the device blob `csr` at the byte offsets off_*: struct_atom_off [n_structs+1] (from 0),
+ * atom_nbr_off [n_atoms+1], z [n_atoms], nbr_idx / nbr_w / nbr_d [n_atoms * 64 at most].  sizes [2 * n_structs]
+ * int32: the largest kept neighbour count of each structure, then its kept pair count -- what the caller copies back
+ * to size the padded buffers.  Integer arithmetic only: the output does not depend on scheduling. */
+int scann_voronoi_select(const void* blob, const int32_t* centre_row, int n_centres, double d_thresh, double w_thresh,
+                         int weight_column, int32_t* sel_count, int32_t* sel_idx, float* sel_w, float* sel_d,
+                         int32_t* status, void* stream);
+int scann_voronoi_batch_csr(const int32_t* struct_atom_off, const int32_t* z, int s0, int n_structs, int atom0,
+                            int n_atoms, const int32_t* sel_count, const int32_t* sel_idx, const float* sel_w,
+                            const float* sel_d, void* csr, long long off_sa, long long off_an, long long off_z,
+                            long long off_idx, long long off_w, long long off_d, int32_t* sizes, void* stream);
+
 /* ---- NCCL gradient all-reduce (SURVEY.md 8b / 8e) ---------------------------------------------------------------
  * One process per GPU, one communicator per process.  Rank 0: scann_allreduce_unique_id(out128) -> 128 HOST bytes
  * (ncclUniqueId) that the caller sends to the other ranks; every rank, with its device current:

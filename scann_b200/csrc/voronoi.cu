@@ -497,3 +497,150 @@ extern "C" int scann_voronoi_neighbors(const double* lattice, const double* coor
     }
     return 0;
 }
+
+// ---- facet records -> the model's neighbour lists ---------------------------------------------------------------
+// What the host does per centre between the cell search and the model's input (voronoi.py voronoi_polyhedra +
+// compute_voronoi_neighbors, DataIterator): order the facets by (distance, site, n0, n1, n2), keep distance <= d_thresh
+// and normalised solid angle >= w_thresh (fp64), and write (site, (float)weight, (float)distance).
+#define VOR_SEL_WARPS 8
+
+// Facet a before facet b in the host's np.lexsort order.  The image components compare as stored: (x & 1023) and
+// (x & 1023) - 512 order alike, but the packed word itself would compare n2 first.
+__device__ __forceinline__ bool vor_before(double da, int sa, int ia, double db, int sb, int ib) {
+    if (da != db) return da < db;
+    if (sa != sb) return sa < sb;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const int na = (ia >> (10 * k)) & 1023, nb = (ib >> (10 * k)) & 1023;
+        if (na != nb) return na < nb;
+    }
+    return false;
+}
+
+// One warp per centre: up to 64 records, two per lane; the rank of a kept record is the number of kept records before
+// it in the host's order (ties, which would be one facet listed twice, by record position: a stable sort).
+__global__ void __launch_bounds__(32 * VOR_SEL_WARPS) vor_select_kernel(
+        const int32_t* __restrict__ off, const VorFacet* __restrict__ rec, const int32_t* __restrict__ centre_row, int n,
+        double d_thresh, double w_thresh, int column, int32_t* __restrict__ sel_count, int32_t* __restrict__ sel_idx,
+        float* __restrict__ sel_w, float* __restrict__ sel_d, int32_t* __restrict__ status) {
+    __shared__ double s_d[VOR_SEL_WARPS][VOR_FMAX];
+    __shared__ int s_site[VOR_SEL_WARPS][VOR_FMAX], s_img[VOR_SEL_WARPS][VOR_FMAX];
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int c = blockIdx.x * VOR_SEL_WARPS + w;
+    if (c >= n) return;                         // whole warps only: the kernel has no block-level barrier
+    const int o = off[c];
+    int k = off[c + 1] - o;
+    if (k > VOR_FMAX) {
+        if (lane == 0) atomicOr(status, SCANN_ERR_VORONOI_CAPACITY);
+        k = VOR_FMAX;
+    }
+    VorFacet r[2];
+    bool keep[2];
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        const int i = lane + 32 * h;
+        keep[h] = false;
+        if (i < k) {
+            r[h] = rec[o + i];
+            keep[h] = r[h].distance <= d_thresh && r[h].normalized >= w_thresh;
+            // a dropped record takes no part in the ranking: site -1 marks it
+            s_d[w][i] = r[h].distance;
+            s_site[w][i] = keep[h] ? r[h].site : -1;
+            s_img[w][i] = r[h].image;
+        }
+    }
+    __syncwarp();
+    const size_t row = (size_t)centre_row[c] * VOR_FMAX;
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        const int i = lane + 32 * h;
+        if (!keep[h]) continue;
+        const double di = r[h].distance;
+        const int si = r[h].site, ii = r[h].image;
+        int rank = 0;
+        for (int j = 0; j < k; ++j) {
+            const int sj = s_site[w][j];
+            if (sj < 0 || j == i) continue;
+            const double dj = s_d[w][j];
+            const int ij = s_img[w][j];
+            rank += vor_before(dj, sj, ij, di, si, ii) || (j < i && !vor_before(di, si, ii, dj, sj, ij));
+        }
+        sel_idx[row + rank] = si;
+        sel_w[row + rank] = __double2float_rn(column ? r[h].normalized : r[h].solid_angle);
+        sel_d[row + rank] = __double2float_rn(di);
+    }
+    const int kept = __popc(__ballot_sync(0xffffffffu, keep[0])) + __popc(__ballot_sync(0xffffffffu, keep[1]));
+    if (lane == 0) sel_count[centre_row[c]] = kept;
+}
+
+extern "C" int scann_voronoi_select(const void* blob, const int32_t* centre_row, int n_centres, double d_thresh,
+                                    double w_thresh, int weight_column, int32_t* sel_count, int32_t* sel_idx,
+                                    float* sel_w, float* sel_d, int32_t* status, void* stream) {
+    if (n_centres < 0 || (weight_column != 0 && weight_column != 1)) {
+        scann_set_error("scann_voronoi_select: n_centres %d, weight_column %d (0 or 1)", n_centres, weight_column);
+        return 1;
+    }
+    if (n_centres == 0) return 0;
+    const int32_t* off = (const int32_t*)blob;
+    const VorFacet* rec = (const VorFacet*)((const char*)blob + vor_header_bytes(n_centres));
+    vor_select_kernel<<<(n_centres + VOR_SEL_WARPS - 1) / VOR_SEL_WARPS, 32 * VOR_SEL_WARPS, 0, (cudaStream_t)stream>>>(
+        off, rec, centre_row, n_centres, d_thresh, w_thresh, weight_column, sel_count, sel_idx, sel_w, sel_d, status);
+    return scann_check_launch("scann_voronoi_select");
+}
+
+// One warp per atom of the batch: its selected neighbours -> nbr_idx / nbr_w / nbr_d at atom_nbr_off[atom]; lane 0
+// raises the structure's largest count (integer atomics: the result does not depend on the order).  The first threads
+// also write the batch's struct_atom_off and z.
+__global__ void vor_batch_fill_kernel(const int32_t* __restrict__ sa, const int32_t* __restrict__ z, int s0, int n_structs,
+                                      int a0, int A, const int32_t* __restrict__ sel_count, const int32_t* __restrict__ sel_idx,
+                                      const float* __restrict__ sel_w, const float* __restrict__ sel_d,
+                                      const int32_t* __restrict__ an, int32_t* __restrict__ sa_out,
+                                      int32_t* __restrict__ z_out, int32_t* __restrict__ idx_out,
+                                      float* __restrict__ w_out, float* __restrict__ d_out, int32_t* __restrict__ sizes) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t <= n_structs) sa_out[t] = sa[s0 + t] - a0;
+    const int a = t >> 5, lane = t & 31;
+    if (a >= A) return;
+    const int row = a0 + a, k = sel_count[row], p = an[a];
+    for (int i = lane; i < k; i += 32) {
+        idx_out[p + i] = sel_idx[(size_t)row * VOR_FMAX + i];
+        w_out[p + i] = sel_w[(size_t)row * VOR_FMAX + i];
+        d_out[p + i] = sel_d[(size_t)row * VOR_FMAX + i];
+    }
+    if (lane == 0) {
+        z_out[a] = z[row];
+        int lo = s0, hi = s0 + n_structs - 1;           // structure of the atom: last s with sa[s] <= row
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (sa[mid] <= row) lo = mid; else hi = mid - 1;
+        }
+        atomicMax(&sizes[lo - s0], k);
+        atomicAdd(&sizes[n_structs + lo - s0], k);
+    }
+}
+
+extern "C" int scann_voronoi_batch_csr(const int32_t* struct_atom_off, const int32_t* z, int s0, int n_structs,
+                                       int atom0, int n_atoms, const int32_t* sel_count, const int32_t* sel_idx,
+                                       const float* sel_w, const float* sel_d, void* csr, long long off_sa,
+                                       long long off_an, long long off_z, long long off_idx, long long off_w,
+                                       long long off_d, int32_t* sizes, void* stream) {
+    if (n_structs <= 0 || n_atoms < 0 || s0 < 0 || atom0 < 0) {
+        scann_set_error("scann_voronoi_batch_csr: s0 %d, n_structs %d, atom0 %d, n_atoms %d", s0, n_structs, atom0,
+                        n_atoms);
+        return 1;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    char* p = (char*)csr;
+    int32_t* an = (int32_t*)(p + off_an);
+    cudaError_t e = cudaMemsetAsync(sizes, 0, sizeof(int32_t) * 2 * (size_t)n_structs, st);
+    if (e != cudaSuccess) {
+        scann_set_error("scann_voronoi_batch_csr: %s", cudaGetErrorString(e));
+        return 2;
+    }
+    vor_scan_kernel<<<1, 1024, 0, st>>>(sel_count + atom0, n_atoms, an);
+    const long long threads = max((long long)n_atoms * 32, (long long)n_structs + 1);
+    vor_batch_fill_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(
+        struct_atom_off, z, s0, n_structs, atom0, n_atoms, sel_count, sel_idx, sel_w, sel_d, an, (int32_t*)(p + off_sa),
+        (int32_t*)(p + off_z), (int32_t*)(p + off_idx), (float*)(p + off_w), (float*)(p + off_d), sizes);
+    return scann_check_launch("scann_voronoi_batch_csr");
+}

@@ -116,6 +116,9 @@ class Engine:
         self.use_graphs = os.environ.get("SCANN_GRAPHS", "1") == "1"
         self.la_grid = self.sm_count
         self.launches = 0
+        # shape classes dropped from the LRU above, CUDA graphs captured (train and inference)
+        self.shape_class_evictions = 0
+        self.graph_captures = 0
         self.prof: Optional[dict] = None
         # engine selection (tensor-core kernels are the default; SCANN_ENGINE=simt keeps the fp32 SIMT path)
         eng = os.environ.get("SCANN_ENGINE", "tc")
@@ -386,6 +389,7 @@ class Engine:
         if b is None:
             while len(self._batches) >= self.max_shape_classes:      # least recently used class: buffers, graphs
                 old_key, old = self._batches.popitem(last=False)
+                self.shape_class_evictions += 1
                 old.graphs.clear()
                 for k in [k for k in self._pinned if k[1] == old_key]:
                     del self._pinned[k]
@@ -445,18 +449,41 @@ class Engine:
             b.csr_event = torch.cuda.Event()
             b.csr_event.record(main)
         b.h2d_bytes = off
-        b.host_dirty = False
-        check(lib.scann_pack_batch(_p(b.csr_dev), offs["sa"], offs["an"], offs["z"], offs["idx"], offs["w"], offs["d"],
-                                   offs.get("ring", -1), offs.get("target", -1), B, M, N, _p(b.atomic), _p(b.atom_mask),
-                                   _p(b.nbr), _p(b.nmask), _p(b.weight), _p(b.dist), _p(b.ring), _p(b.target),
-                                   self._stream()), "pack_batch")
-        self.launches += 1
+        self._pack_csr(b, b.csr_dev, offs)
         if self.overlap_h2d:
             b.csr_packed = torch.cuda.Event()
             b.csr_packed.record(main)
         if plan:
             self._plan(b)
         return b
+
+    def load_batch_device_csr(self, csr: Dict[str, object], M: Optional[int] = None, N: Optional[int] = None,
+                              plan: bool = True) -> Batch:
+        """``load_batch_csr`` for a CSR batch that is already on the device (``voronoi.NeighborSelection.csr``): one
+        blob ``csr["blob"]`` with the byte offsets ``csr["offsets"]`` (keys sa, an, z, idx, w, d) and the host sizes
+        ``B`` / ``M`` / ``N`` / ``P``.  ``M`` / ``N`` may be raised above the batch's own (shape classes); the padding
+        is masked.  Nothing crosses to or from the host."""
+        B, P = int(csr["B"]), int(csr["P"])
+        M = int(csr["M"]) if M is None else int(M)
+        N = int(csr["N"]) if N is None else int(N)
+        if M < int(csr["M"]) or N < int(csr["N"]):
+            raise ValueError(f"M={M}, N={N} below the batch's own {csr['M']}, {csr['N']}")
+        b = self._get_batch(B, M, N, P)
+        b.P_host = P
+        b.h2d_bytes = 0
+        self._pack_csr(b, csr["blob"], csr["offsets"])
+        if plan:
+            self._plan(b)
+        return b
+
+    def _pack_csr(self, b: Batch, blob: torch.Tensor, offs: Dict[str, int]) -> None:
+        """CSR blob on the device -> the padded buffers of the batch's shape class (scann_pack_batch)."""
+        b.host_dirty = False            # the pinned mirror is stale: it must not be copied over what is packed here
+        check(lib.scann_pack_batch(_p(blob), offs["sa"], offs["an"], offs["z"], offs["idx"], offs["w"], offs["d"],
+                                   offs.get("ring", -1), offs.get("target", -1), b.B, b.M, b.N, _p(b.atomic),
+                                   _p(b.atom_mask), _p(b.nbr), _p(b.nmask), _p(b.weight), _p(b.dist), _p(b.ring),
+                                   _p(b.target), self._stream()), "pack_batch")
+        self.launches += 1
 
     def _new_batch(self, B: int, M: int, N: int, tile_cap: int, ngroups: int, stride: int = TILE) -> Batch:
         dev = self.device
@@ -1551,6 +1578,7 @@ class Engine:
                     self._train_body(b, allreduce, apply, want_grads, replan)
                 g.n_launches = self.launches - n0
                 b.graphs[key] = g
+                self.graph_captures += 1
             else:
                 self.launches += g.n_launches
             g.replay()
@@ -1639,6 +1667,7 @@ class Engine:
                 self.forward(b, training=False, replan=replan)
             g.n_launches = self.launches - n0
             b.graphs[key] = g
+            self.graph_captures += 1
         else:
             self.launches += g.n_launches
         g.replay()

@@ -8,6 +8,7 @@ Arithmetic runs in the sm_100a kernels behind ``libscann_b200.so``; there is no 
 """
 from __future__ import annotations
 
+import functools
 import math
 import os
 from typing import Dict, Iterable, Optional
@@ -39,6 +40,33 @@ class History:
 
     def add(self, key: str, v: float) -> None:
         self.history.setdefault(key, []).append(float(v))
+
+
+MAX_STRUCTURE_ATOMS = 1000      # predict_structures: a site index of 1000 would read as the padding marker
+_CHUNK_ATOMS = 1 << 16          # predict_structures: sites whose neighbour lists are staged on the device at once
+
+
+def shape_class(M: int, N: int):
+    """Padded (M, N) of a ``predict_structures`` batch: atoms up to a multiple of 8; neighbours up to a multiple of 4
+    while <= 32 (a batch within 32 keeps the pipelined 32-row plan), else of 8 (at most 64, the facet capacity)."""
+    M = max(8, (M + 7) // 8 * 8)
+    N = max(4, (N + 3) // 4 * 4) if N <= 32 else (N + 7) // 8 * 8
+    return M, N
+
+
+def _structure_chunks(n_atoms, batch_size: int):
+    """Runs of whole batches with about _CHUNK_ATOMS sites (at least one batch): [(first, end)]."""
+    out, c0, atoms = [], 0, 0
+    for s0 in range(0, len(n_atoms), batch_size):
+        s1 = min(s0 + batch_size, len(n_atoms))
+        n = sum(n_atoms[s0:s1])
+        if s0 > c0 and atoms + n > _CHUNK_ATOMS:
+            out.append((c0, s0))
+            c0, atoms = s0, 0
+        atoms += n
+    if c0 < len(n_atoms):
+        out.append((c0, len(n_atoms)))
+    return out
 
 
 def _ragged_capable(seq) -> bool:
@@ -174,6 +202,64 @@ class ScannKerasModel:
 
     def __call__(self, inputs, training: bool = False):
         return self.predict(inputs)
+
+    def predict_structures(self, structs, d_t: float = 4.0, w_t: float = 0.4, angle: Optional[bool] = None,
+                           batch_size: int = 128, cutoff: float = 13.0, allow_pathological: bool = False):
+        """Structures in, ``[target [S, 1], ga_score]`` out: the README flow (``compute_voronoi_neighbor`` ->
+        ``prepare_input_pmt`` -> ``predict``) for many structures, with the neighbour lists selected and batched on
+        the device (``voronoi.select_neighbors``).  ``ga_score`` is a list of S float32 arrays, one value per atom,
+        in input order.  The outputs equal those of ``predict`` on the same batches built on the host.
+
+        ``angle``: the weight column, as in ``prepare_input_pmt`` (True = raw solid angle, False = normalised).  None
+        picks the column ``DataIterator`` trains this model on: the raw solid angle iff ``g_update``.  (The README
+        example passes ``angle=False`` to a ``g_update`` model; that feeds it a column it was not trained on.)
+        ``d_t`` / ``w_t`` / ``cutoff`` / ``allow_pathological``: as in ``compute_voronoi_neighbors``.
+
+        Batches of ``batch_size`` structures are padded to shape classes (atoms to a multiple of 8, neighbours to a
+        multiple of 4 up to 32, then of 8), so that structures of different sizes replay a handful of CUDA graphs
+        instead of capturing one per batch.  The padding is masked and trimmed from the outputs.
+
+        Refused: ring-feature models (the ring / aromatic flags come from openbabel, not from the geometry) and
+        ``feature='cgcnn'`` models -- use ``predict`` on ``DataIterator`` batches for those -- and structures with
+        more than 1000 atoms (1000 is the reference's neighbour padding marker)."""
+        from . import voronoi as V
+        spec = self.spec
+        if spec.use_ring:
+            raise NotImplementedError("predict_structures: use_ring models need the ring / aromatic flags of openbabel, "
+                                      "which the geometry does not give; build the batches with DataIterator(..., "
+                                      "use_ring=True) and call predict")
+        if spec.feature == "cgcnn":
+            raise NotImplementedError("predict_structures: feature='cgcnn' batches carry per-atom feature vectors; build "
+                                      "them with DataIterator(..., feature='cgcnn') and call predict")
+        structs = list(structs)
+        checked = V._arrays(structs)
+        for k, X in enumerate(checked[1]):
+            if len(X) == 0:
+                raise ValueError(f"structure {k} has no sites")
+            if len(X) > MAX_STRUCTURE_ATOMS:
+                raise ValueError(f"structure {k} has {len(X)} sites: at most {MAX_STRUCTURE_ATOMS} (a neighbour index "
+                                 "of 1000 is the reference's padding marker and would be masked); predict such "
+                                 "structures from host-built batches: compute_voronoi_neighbors + DataIterator + predict")
+        if batch_size < 1:
+            raise ValueError("batch_size must be >= 1")
+        column = bool(spec.g_update) if angle is None else bool(angle)
+        eng = self.engine
+        y_out = np.zeros((len(structs), 1), np.float32)
+        ga_out = []
+        for c0, c1 in _structure_chunks([len(X) for X in checked[1]], batch_size):
+            sel = V.select_neighbors(structs[c0:c1], d_t, w_t, column, cutoff, allow_pathological, first_index=c0,
+                                     _checked=(checked[0][c0:c1], checked[1][c0:c1]))
+            for s0 in range(0, c1 - c0, batch_size):
+                s1 = min(s0 + batch_size, c1 - c0)
+                csr = sel.csr(s0, s1)
+                M, N = shape_class(csr["M"], csr["N"])
+                b = eng.load_batch_device_csr(csr, M=M, N=N, plan=False)
+                y, ga = eng.predict_step(b, replan=True)
+                y_out[c0 + s0:c0 + s1, 0] = y.cpu().numpy()           # synchronises the stream
+                ga_h = ga.cpu().numpy().reshape(b.B, b.M)
+                ga_out.extend(ga_h[i, :n].copy() for i, n in enumerate(csr["n_atoms"]))
+        eng.check_status()
+        return [y_out, ga_out]
 
     # ---- training --------------------------------------------------------------------------
     def compile(self, loss=None, optimizer=None, metrics=None, learning_rate=None):
@@ -434,6 +520,22 @@ class SCANN:
         if len(out) == 2:
             return out[0] * self.std + self.mean, out[1]
         return out * self.std + self.mean
+
+    def _predict_structures(self, structs, d_t: float = 4.0, w_t: float = 0.4, angle: Optional[bool] = None,
+                            batch_size: int = 128, cutoff: float = 13.0, allow_pathological: bool = False):
+        """``ScannKerasModel.predict_structures`` with the target scaled back like ``predict_data``."""
+        y, ga = self.model.predict_structures(structs, d_t=d_t, w_t=w_t, angle=angle, batch_size=batch_size,
+                                              cutoff=cutoff, allow_pathological=allow_pathological)
+        return y * self.std + self.mean, ga
+
+    @property
+    def predict_structures(self):
+        """``predict_structures(structs, d_t=4.0, w_t=0.4, angle=None, batch_size=128, cutoff=13.0,
+        allow_pathological=False)``: ``ScannKerasModel.predict_structures`` with the target scaled back like
+        ``predict_data``.  (A property, not a plain method: the record of SCANN's plain public methods in
+        tests/golden/reference/graph_public_surface.npz stays the surface that was compared with the reference's SCANN,
+        which has no such method.)"""
+        return functools.partial(SCANN._predict_structures, self)
 
     # ---- training shell (scann_model.py:163-313) ------------------------------------------------------------
     def _run_dir(self) -> str:

@@ -168,3 +168,179 @@ def compute_voronoi_neighbor(struct, d_thresh: float = 4.0, w_thresh: float = 0.
     """The reference's ``compute_voronoi_neighbor(struct, d_thresh, w_thresh)`` for one structure (see
     ``compute_voronoi_neighbors``)."""
     return compute_voronoi_neighbors([struct], d_thresh, w_thresh, cutoff, allow_pathological)[0]
+
+
+# ------------------------------------------------------------------------------------------ neighbour lists on the device
+# The same lists as compute_voronoi_neighbors + DataIterator, without the facet records leaving the device:
+# scann_voronoi_select orders and thresholds each centre's records into per-atom staging rows, and
+# scann_voronoi_batch_csr writes any run of structures as the CSR batch that Engine.load_batch_device_csr packs.
+# Only the per-centre flags (retry / error) and a few sizes per batch come back to the host.
+_SEL = _CAP                     # staging slots per atom row (the kernel's facet capacity)
+_ALIGN = 16
+
+# optional CUDA-event log (tools/structure_predict_bench.py): name -> list of (start, end) event pairs
+event_log = None
+
+
+def _timed(name, stream, fn):
+    if event_log is None:
+        return fn()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record(stream)
+    out = fn()
+    e1.record(stream)
+    event_log.setdefault(name, []).append((e0, e1))
+    return out
+
+
+class NeighborSelection:
+    """Selected neighbour lists of a run of structures, resident on the device (``select_neighbors``): per atom row up
+    to 64 ``(site, weight, distance)`` in the order of ``compute_voronoi_neighbors``.  ``csr(s0, s1)`` writes
+    structures ``s0 .. s1 - 1`` as one CSR batch."""
+
+    def __init__(self, sa_off, d_sa, d_z, count, idx, w, d):
+        self.struct_atom_off = sa_off            # host, int64 [S+1]
+        self._d_sa, self._d_z = d_sa, d_z
+        self.sel_count, self.sel_idx, self.sel_w, self.sel_d = count, idx, w, d
+
+    def __len__(self):
+        return len(self.struct_atom_off) - 1
+
+    def csr(self, s0: int = 0, s1: int = None) -> dict:
+        """Structures ``s0 .. s1 - 1`` as the CSR batch of ``DataIterator.csr_item`` in ONE device blob (``"blob"``,
+        byte offsets ``"offsets"``; device views ``struct_atom_off``, ``atom_nbr_off``, ``z``, ``nbr_idx``, ``nbr_w``,
+        ``nbr_d``).  Host side: ``B``, ``M`` (most atoms), ``N`` (most kept neighbours), ``P`` (kept pairs) and per
+        structure ``n_atoms``, ``nmax``, ``npairs``."""
+        s1 = len(self) if s1 is None else s1
+        B = s1 - s0
+        sa = self.struct_atom_off
+        a0, nA = int(sa[s0]), int(sa[s1] - sa[s0])
+        dev = self.sel_count.device
+        sizes_b = [("sa", 4 * (B + 1)), ("an", 4 * (nA + 1)), ("z", 4 * nA), ("idx", 4 * nA * _SEL), ("w", 4 * nA * _SEL),
+                   ("d", 4 * nA * _SEL)]
+        offs, off = {}, 0
+        for name, nb in sizes_b:
+            offs[name] = off
+            off += (nb + _ALIGN - 1) // _ALIGN * _ALIGN
+        blob = torch.empty(max(off, _ALIGN), dtype=torch.uint8, device=dev)
+        sizes = torch.empty(2 * B, dtype=torch.int32, device=dev)
+        stream = torch.cuda.current_stream(dev)
+        _timed("voronoi_batch_csr", stream, lambda: _abi.check(_abi.lib.scann_voronoi_batch_csr(
+            self._d_sa.data_ptr(), self._d_z.data_ptr(), s0, B, a0, nA, self.sel_count.data_ptr(),
+            self.sel_idx.data_ptr(), self.sel_w.data_ptr(), self.sel_d.data_ptr(), blob.data_ptr(), offs["sa"],
+            offs["an"], offs["z"], offs["idx"], offs["w"], offs["d"], sizes.data_ptr(),
+            ctypes.c_void_p(stream.cuda_stream)), "scann_voronoi_batch_csr"))
+        host = torch.empty(2 * B, dtype=torch.int32, pin_memory=True)
+        host.copy_(sizes, non_blocking=True)
+        stream.synchronize()
+        h = host.numpy()
+        nmax, npairs = h[:B].copy(), h[B:].copy()
+        n_atoms = np.diff(sa[s0:s1 + 1])
+        P = int(npairs.sum())
+
+        def view(name, dt, n):
+            return blob[offs[name]:offs[name] + 4 * n].view(dt)
+        return {"blob": blob, "offsets": offs, "B": B, "M": int(n_atoms.max()), "N": int(nmax.max()), "P": P,
+                "n_atoms": n_atoms, "nmax": nmax, "npairs": npairs,
+                "struct_atom_off": view("sa", torch.int32, B + 1), "atom_nbr_off": view("an", torch.int32, nA + 1),
+                "z": view("z", torch.int32, nA), "nbr_idx": view("idx", torch.int32, P),
+                "nbr_w": view("w", torch.float32, P), "nbr_d": view("d", torch.float32, P)}
+
+
+def _select_pass(d_lat, d_x, d_sa, sa_off, atoms, cut, allow_pathological, d_t, w_t, column, sel):
+    """One cell search over the listed centres, its records thresholded into the staging rows -> flags [C] (host)."""
+    dev = d_x.device
+    C = len(atoms)
+    cs = np.searchsorted(sa_off, atoms, side="right") - 1
+    # one upload of the per-centre inputs: atom rows, structures (int32), cutoffs (float64, 8-byte aligned after 2C ints)
+    head = np.empty(2 * C, np.int32)
+    head[:C], head[C:] = atoms, cs
+    up = torch.from_numpy(np.concatenate([head.view(np.uint8), np.ascontiguousarray(cut, np.float64).view(np.uint8)]))
+    d_up = up.to(dev)
+    d_at, d_cs = d_up[:4 * C].view(torch.int32), d_up[4 * C:8 * C].view(torch.int32)
+    d_cut = d_up[8 * C:].view(torch.float64)
+    hb = (4 * (2 * C + 1) + 31) // 32 * 32
+    slots = torch.empty(FACET.itemsize * C * _CAP, dtype=torch.uint8, device=dev)
+    count = torch.empty(C, dtype=torch.int32, device=dev)
+    blob = torch.empty(hb + FACET.itemsize * C * _CAP, dtype=torch.uint8, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    stream = torch.cuda.current_stream(dev)
+    st = ctypes.c_void_p(stream.cuda_stream)
+    _timed("voronoi_neighbors", stream, lambda: _abi.check(_abi.lib.scann_voronoi_neighbors(
+        d_lat.data_ptr(), d_x.data_ptr(), d_sa.data_ptr(), d_at.data_ptr(), d_cs.data_ptr(), d_cut.data_ptr(), C,
+        1 if allow_pathological else 0, _CAP, slots.data_ptr(), count.data_ptr(), blob.data_ptr(), None,
+        status.data_ptr(), st), "scann_voronoi_neighbors"))
+    count_, idx, w, d = sel
+    _timed("voronoi_select", stream, lambda: _abi.check(_abi.lib.scann_voronoi_select(
+        blob.data_ptr(), d_at.data_ptr(), C, float(d_t), float(w_t), 0 if column else 1, count_.data_ptr(),
+        idx.data_ptr(), w.data_ptr(), d.data_ptr(), status.data_ptr(), st), "scann_voronoi_select"))
+    host = torch.empty(C + 1, dtype=torch.int32, pin_memory=True)
+    host[:C].copy_(blob[4 * (C + 1):4 * (2 * C + 1)].view(torch.int32), non_blocking=True)
+    host[C:].copy_(status, non_blocking=True)
+    stream.synchronize()
+    h = host.numpy()
+    if h[C] & ERR_CAPACITY and not (h[:C] & ERR_CAPACITY).any():
+        raise _abi.ScannAbiError("scann_voronoi_select: a centre has more records than the staging rows hold")
+    return h[:C].copy()
+
+
+def select_neighbors(structs: Sequence, d_thresh: float = 4.0, w_thresh: float = 0.4, angle: bool = True,
+                     cutoff: float = 13.0, allow_pathological: bool = False, first_index: int = 0,
+                     _checked=None) -> NeighborSelection:
+    """``compute_voronoi_neighbors`` kept on the device: the cell search of every site, pymatgen's retry loop (only the
+    per-site flags come back; flagged sites run again with a wider cutoff, their records replace the first ones), then
+    the selection of ``scann_voronoi_select``.  ``angle`` picks the weight column as ``prepare_input_pmt`` does: True =
+    solid angle, False = normalised solid angle.  Atomic numbers come from ``struct.atomic_numbers``.  A bad structure
+    raises the ``ValueError`` of ``voronoi_polyhedra``, numbered ``first_index + k``."""
+    _abi.require_gpu()
+    lats, xs = _checked if _checked is not None else _arrays(structs)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    nat = np.array([len(X) for X in xs], np.int64)
+    sa_off = np.zeros(len(xs) + 1, np.int64)
+    np.cumsum(nat, out=sa_off[1:])
+    A = int(sa_off[-1])
+    z = np.fromiter((int(v) for st in structs for v in st.atomic_numbers), np.int32) if A else np.zeros(0, np.int32)
+    if len(z) != A:
+        raise ValueError("every structure needs one atomic number per site (struct.atomic_numbers)")
+    sel = (torch.zeros(A, dtype=torch.int32, device=dev), torch.empty(A * _SEL, dtype=torch.int32, device=dev),
+           torch.empty(A * _SEL, dtype=torch.float32, device=dev), torch.empty(A * _SEL, dtype=torch.float32, device=dev))
+    d_sa = torch.from_numpy(sa_off.astype(np.int32)).to(dev)
+    d_z = torch.from_numpy(z).to(dev)
+    out = NeighborSelection(sa_off, d_sa, d_z, *sel)
+    if A == 0:
+        return out
+    d_lat = torch.from_numpy(np.ascontiguousarray(np.stack(lats).reshape(-1, 9))).to(dev)
+    d_x = torch.from_numpy(np.ascontiguousarray(np.concatenate(xs))).to(dev)
+    sid = np.repeat(np.arange(len(xs)), nat)
+    tops = np.array([max_cutoff(L) for L in lats])
+    cut = np.full(A, float(cutoff))
+    todo = np.arange(A)
+    while len(todo):
+        again = []
+        for c0 in range(0, len(todo), _CHUNK):
+            atoms = todo[c0:c0 + _CHUNK]
+            flags = _select_pass(d_lat, d_x, d_sa, sa_off, atoms, cut[atoms], allow_pathological, d_thresh, w_thresh,
+                                 angle, sel)
+            for k in np.flatnonzero(flags):         # the checks of voronoi_polyhedra, in the same order
+                a = int(atoms[k])
+                err = int(flags[k]) & ~_INFINITE
+                s, site = int(sid[a]), int(a - sa_off[sid[a]])
+                if err:
+                    why = "; ".join(m for b, m in _MESSAGES.items() if err & b)
+                    raise ValueError(f"structure {first_index + s}, site {site}: {why}")
+                if not allow_pathological:
+                    if cut[a] >= tops[s]:
+                        raise ValueError(f"structure {first_index + s}, site {site}: infinite Voronoi facet at the "
+                                         f"largest cutoff {cut[a]:.3f} Angstrom")
+                    cut[a] = min(2 * cut[a], tops[s] + 0.001)
+                    again.append(a)
+        todo = np.array(again, np.int64)
+    return out
+
+
+def neighbor_csr(structs: Sequence, d_t: float = 4.0, w_t: float = 0.4, angle: bool = True, cutoff: float = 13.0,
+                 allow_pathological: bool = False) -> dict:
+    """All ``structs`` as one CSR batch on the device: what ``DataIterator(..., g_update=angle).csr_item`` builds from
+    ``compute_voronoi_neighbors(structs, d_t, w_t)``, bit for bit, without the per-site host work (see
+    ``NeighborSelection.csr`` for the keys)."""
+    return select_neighbors(structs, d_t, w_t, angle, cutoff, allow_pathological).csr()
