@@ -89,6 +89,16 @@ int scann_pack_batch(const void* csr, long long off_sa, long long off_an, long l
                      long long off_w, long long off_d, long long off_ring, long long off_target, int B, int M, int N,
                      int32_t* atomic, uint8_t* atom_mask, int32_t* neighbors, uint8_t* neighbor_mask, float* weight,
                      float* dist, float* ring_out, float* target, void* stream);
+/* The same padding for batch structures picked out of a device-resident data set (DataIterator.__getitem__ over a
+ * shuffled epoch, scann/utils/datagenerator.py:69-135): struct_atom_off [S+1] and atom_nbr_off [A+1] from 0, z [A],
+ * nbr_idx / nbr_w / nbr_d [P], ring [A,2] int32 or NULL, target_in [S] float32 or NULL.  Batch structure b is data-set
+ * structure sel[b] (sel: B int32 device indices, e.g. a slice of the epoch's permutation); target[b] = target_in[sel[b]].
+ * B, M, N > 0 and B * M * N < 2^31; integer arithmetic only, every buffer caller-allocated. */
+int scann_gather_batch(const int32_t* struct_atom_off, const int32_t* atom_nbr_off, const int32_t* z,
+                       const int32_t* nbr_idx, const float* nbr_w, const float* nbr_d, const int32_t* ring,
+                       const float* target_in, const int32_t* sel, int B, int M, int N, int32_t* atomic,
+                       uint8_t* atom_mask, int32_t* neighbors, uint8_t* neighbor_mask, float* weight, float* dist,
+                       float* ring_out, float* target, void* stream);
 
 /* ---- input embedding: Embedding + (extra_embed) + dense_embed swish -----------------------
  * scann/models/scann_model.py:361-374.  ring may be NULL (use_ring False). t0 (pre-activation,

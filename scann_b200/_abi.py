@@ -27,6 +27,7 @@ PROTOTYPES = {
     "scann_set_la_groups4": (ci, [ci]),
     "scann_plan_build": (ci, [vp, vp, vp, vp, ci, ci, ci, ci, ci, ci] + [vp] * 13 + [vp, ci, vp, vp]),
     "scann_pack_batch": (ci, [vp] + [C.c_longlong] * 8 + [ci, ci, ci] + [vp] * 8 + [vp]),
+    "scann_gather_batch": (ci, [vp] * 9 + [ci, ci, ci] + [vp] * 8 + [vp]),
     "scann_embed_forward": (ci, [vp, vp, ci, ci, ci] + [vp] * 7 + [vp, vp, vp, vp]),
     "scann_cgcnn_embed_forward": (ci, [vp, vp, vp, ci, ci, ci, vp, vp]),
     "scann_cgcnn_embed_backward": (ci, [vp, vp, vp, ci, ci, ci] + [vp] * 12 + [vp, vp]),

@@ -302,44 +302,61 @@ __global__ void __launch_bounds__(PLAN_GSZ) plan_chain_kernel(
 
 // ---------------------------------------------------------------------------------------------
 // Ragged (CSR) batch -> padded device buffers: DataIterator.__getitem__ (scann/utils/datagenerator.py:69-135) on
-// the device.  One thread per padded atom row (b, m).  Neighbour value 1000 is the reference's padding marker
-// (mask = idx != 1000, index reset to 0; datagenerator.py:82-90); weights / distances are zero padded;
-// atom_mask = Z != 0.  The CSR arrays arrive in one blob (one host->device copy of the valid data only).
+// the device.  One thread per padded neighbour slot (b, m, n), so that the [R, N] stores of a warp are contiguous;
+// the n == 0 thread of a row also writes the row's atom fields.  Neighbour value 1000 is the reference's padding
+// marker (mask = idx != 1000, index reset to 0; datagenerator.py:82-90); weights / distances are zero padded;
+// atom_mask = Z != 0.
+// kGather = false (scann_pack_batch): batch structure b is structure b of the CSR batch (offsets from 0, one blob
+// copied from the host).  kGather = true (scann_gather_batch): batch structure b is structure sel[b] of a
+// device-resident data set, and target[b] = tgt[sel[b]].
 // ---------------------------------------------------------------------------------------------
-__global__ void pack_batch_kernel(const int32_t* __restrict__ sa, const int32_t* __restrict__ an,
-                                  const int32_t* __restrict__ z, const int32_t* __restrict__ idx,
-                                  const float* __restrict__ w, const float* __restrict__ d,
-                                  const int32_t* __restrict__ ring, const float* __restrict__ tgt, int B, int M, int N,
+template <bool kGather>
+__global__ void pack_batch_kernel(const int32_t* __restrict__ sel, const int32_t* __restrict__ sa,
+                                  const int32_t* __restrict__ an, const int32_t* __restrict__ z,
+                                  const int32_t* __restrict__ idx, const float* __restrict__ w,
+                                  const float* __restrict__ d, const int32_t* __restrict__ ring,
+                                  const float* __restrict__ tgt, int B, int M, int N,
                                   int32_t* __restrict__ atomic, uint8_t* __restrict__ atom_mask,
                                   int32_t* __restrict__ nbr, uint8_t* __restrict__ nmask, float* __restrict__ weight,
                                   float* __restrict__ dist, float* __restrict__ ring_out, float* __restrict__ target) {
-    const int r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (tgt && r < B) target[r] = tgt[r];
-    if (r >= B * M) return;
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (tgt && t < B) target[t] = tgt[kGather ? sel[t] : t];
+    if (t >= B * M * N) return;
+    const int r = t / N, n = t - r * N;
     const int b = r / M, m = r - b * M;
-    const int a0 = sa[b], n_at = sa[b + 1] - a0;
-    int Z = 0, p0 = 0, k = 0, a = -1;
-    if (m < n_at) { a = a0 + m; Z = z[a]; p0 = an[a]; k = an[a + 1] - p0; }
-    atomic[r] = Z;
-    atom_mask[r] = Z != 0;
-    if (ring_out) {
-        ring_out[(size_t)r * 2] = a >= 0 ? (float)ring[(size_t)a * 2] : 0.f;
-        ring_out[(size_t)r * 2 + 1] = a >= 0 ? (float)ring[(size_t)a * 2 + 1] : 0.f;
-    }
-    for (int n = 0; n < N; ++n) {
-        const size_t s = (size_t)r * N + n;
-        int j = 0;
-        bool valid = false;
-        float wv = 0.f, dv = 0.f;
-        if (n < k) {
-            j = idx[p0 + n];
-            valid = j != 1000;
-            if (!valid) j = 0;
-            wv = w[p0 + n];
-            dv = d[p0 + n];
+    const int s = kGather ? sel[b] : b;
+    const int a0 = sa[s], n_at = sa[s + 1] - a0;
+    int p0 = 0, k = 0, a = -1;
+    if (m < n_at) { a = a0 + m; p0 = an[a]; k = an[a + 1] - p0; }
+    if (n == 0) {
+        const int Z = a >= 0 ? z[a] : 0;
+        atomic[r] = Z;
+        atom_mask[r] = Z != 0;
+        if (ring_out) {
+            ring_out[(size_t)r * 2] = a >= 0 ? (float)ring[(size_t)a * 2] : 0.f;
+            ring_out[(size_t)r * 2 + 1] = a >= 0 ? (float)ring[(size_t)a * 2 + 1] : 0.f;
         }
-        nbr[s] = j; nmask[s] = valid; weight[s] = wv; dist[s] = dv;
     }
+    int j = 0;
+    bool valid = false;
+    float wv = 0.f, dv = 0.f;
+    if (n < k) {
+        j = idx[p0 + n];
+        valid = j != 1000;
+        if (!valid) j = 0;
+        wv = w[p0 + n];
+        dv = d[p0 + n];
+    }
+    nbr[t] = j; nmask[t] = valid; weight[t] = wv; dist[t] = dv;
+}
+
+static int pack_shape_ok(const char* who, int B, int M, int N) {
+    if (B <= 0 || M <= 0 || N <= 0) { scann_set_error("%s: bad shape B=%d M=%d N=%d", who, B, M, N); return 0; }
+    if ((long long)B * M * N > 0x7fffffffLL) {
+        scann_set_error("%s: B*M*N = %lld neighbour slots exceed int32", who, (long long)B * M * N);
+        return 0;
+    }
+    return 1;
 }
 
 // csr: device blob; off_*: byte offsets of struct_atom_off [B+1], atom_nbr_off [A+1], z [A], nbr_idx / nbr_w / nbr_d [P],
@@ -348,15 +365,29 @@ extern "C" int scann_pack_batch(const void* csr, long long off_sa, long long off
                                 long long off_w, long long off_d, long long off_ring, long long off_target, int B, int M,
                                 int N, int32_t* atomic, uint8_t* atom_mask, int32_t* neighbors, uint8_t* neighbor_mask,
                                 float* weight, float* dist, float* ring_out, float* target, void* stream) {
-    if (B <= 0 || M <= 0 || N <= 0) { scann_set_error("pack_batch: bad shape B=%d M=%d N=%d", B, M, N); return 1; }
+    if (!pack_shape_ok("pack_batch", B, M, N)) return 1;
     const char* p = (const char*)csr;
-    const int R = B * M;
-    pack_batch_kernel<<<(max(R, B) + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        (const int32_t*)(p + off_sa), (const int32_t*)(p + off_an), (const int32_t*)(p + off_z),
+    const int T = B * M * N;
+    pack_batch_kernel<false><<<(max(T, B) + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
+        nullptr, (const int32_t*)(p + off_sa), (const int32_t*)(p + off_an), (const int32_t*)(p + off_z),
         (const int32_t*)(p + off_idx), (const float*)(p + off_w), (const float*)(p + off_d),
         off_ring >= 0 ? (const int32_t*)(p + off_ring) : nullptr, off_target >= 0 ? (const float*)(p + off_target) : nullptr,
         B, M, N, atomic, atom_mask, neighbors, neighbor_mask, weight, dist, off_ring >= 0 ? ring_out : nullptr, target);
     return scann_check_launch("scann_pack_batch");
+}
+
+extern "C" int scann_gather_batch(const int32_t* struct_atom_off, const int32_t* atom_nbr_off, const int32_t* z,
+                                  const int32_t* nbr_idx, const float* nbr_w, const float* nbr_d, const int32_t* ring,
+                                  const float* target_in, const int32_t* sel, int B, int M, int N, int32_t* atomic,
+                                  uint8_t* atom_mask, int32_t* neighbors, uint8_t* neighbor_mask, float* weight,
+                                  float* dist, float* ring_out, float* target, void* stream) {
+    if (!pack_shape_ok("gather_batch", B, M, N)) return 1;
+    if (!sel) { scann_set_error("gather_batch: sel is NULL"); return 1; }
+    const int T = B * M * N;
+    pack_batch_kernel<true><<<(max(T, B) + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
+        sel, struct_atom_off, atom_nbr_off, z, nbr_idx, nbr_w, nbr_d, ring, target_in, B, M, N, atomic, atom_mask,
+        neighbors, neighbor_mask, weight, dist, ring ? ring_out : nullptr, target_in ? target : nullptr);
+    return scann_check_launch("scann_gather_batch");
 }
 
 extern "C" int scann_plan_build(const uint8_t* neighbor_mask, const int32_t* neighbors, const float* dist,

@@ -17,7 +17,7 @@ index, ``n[2]`` = solid angle, ``n[3]`` = normalised solid angle, ``n[-1]`` = di
 from __future__ import annotations
 
 from math import ceil
-from typing import Dict, Tuple
+from typing import Dict, Optional, Tuple
 
 import numpy as np
 
@@ -118,6 +118,267 @@ class DataIterator:
         if self.feature == "cgcnn":        # datagenerator.py:107-110: the mask comes from the atomic numbers, then the
             inputs["atomic"] = ATOMIC_FEATURES[inputs["atomic"]]      # numbers are replaced by their feature vectors
         return inputs, energy
+
+
+_INT32_MAX = 0x7fffffff
+_DEVICE_ARRAYS = ("struct_atom_off", "atom_nbr_off", "z", "nbr_idx", "nbr_w", "nbr_d", "ring", "target")
+
+
+def _refuse_structures_route(who: str, use_ring: bool, feature: str) -> None:
+    if feature == "cgcnn":
+        raise NotImplementedError(f"{who}: feature='cgcnn' batches carry per-atom feature vectors; train from "
+                                  "DataIterator(..., feature='cgcnn') (padded batches)")
+    if use_ring:
+        raise NotImplementedError(f"{who}: use_ring models need the ring / aromatic flags of openbabel, which the "
+                                  "geometry does not give; build a DataIterator(..., use_ring=True) from the "
+                                  "reference's data files and convert it with DeviceDataIterator.from_data_iterator")
+
+
+def _check_int32_offsets(atom_off: np.ndarray, pair_off: Optional[np.ndarray] = None) -> None:
+    """The device offsets are int32: refuse a data set whose atom or pair offsets reach 2^31, naming the first
+    structure that does not fit."""
+    for what, off in (("atoms", atom_off), ("neighbour pairs", pair_off)):
+        if off is not None and int(off[-1]) > _INT32_MAX:
+            s = int(np.searchsorted(off[1:], _INT32_MAX, side="right"))
+            raise ValueError(f"structure {s}: the data set's {what} exceed int32 offsets ({int(off[-1])} in all, at most "
+                             f"{_INT32_MAX}); split it into data sets below 2^31 {what}")
+
+
+class DeviceDataIterator:
+    """``DataIterator`` with the whole data set resident on the GPU: the CSR arrays and the targets are uploaded once,
+    the epoch's shuffle order once per epoch, and ``Engine.load_batch_gather`` pads a batch straight out of them
+    (``scann_gather_batch``, csrc/plan.cu).  A training step then copies nothing from the host and does O(batch) host
+    work: the batch's M / N / P come from per-structure sizes kept on the host.
+
+    Same Sequence protocol and semantics as ``DataIterator`` (``batch_size``, ``shuffle``, ``converter``,
+    ``use_ring``, ``g_update`` -> weight column, ``len``, ``on_epoch_end`` with ``np.random.shuffle`` of the global
+    generator): the batches, and the generator's stream, are those of the host iterator.  ``ScannKerasModel.fit`` and
+    ``SCANN.evaluate`` take the device route for it; ``csr_item`` / ``__getitem__`` return the host forms of
+    ``DataIterator`` (copied back from the device) for any other consumer.
+
+    Build it with ``from_data_iterator`` (the reference's ``.npy`` flow) or ``from_structures`` (Voronoi neighbour
+    lists selected on the device; nothing per site reaches the host).  ``feature='cgcnn'`` is not supported."""
+
+    def __init__(self, arrays: Dict[str, object], energy: np.ndarray, atom_off: np.ndarray, pair_off: np.ndarray,
+                 nmax: np.ndarray, npairs: np.ndarray, batch_size: int = 32, shuffle: bool = False,
+                 use_ring: bool = False, weight_index: int = 3, converter: float = 1.0, indexes=None):
+        """Low-level constructor.  ``arrays``: device tensors ``struct_atom_off`` [S+1] / ``atom_nbr_off`` [A+1] (int32,
+        from 0), ``z`` [A], ``nbr_idx`` / ``nbr_w`` / ``nbr_d`` [P], ``ring`` [A, 2] int32 or None, ``target`` [S]
+        float32.  Host: ``energy`` [S] float32 (the targets), ``atom_off`` / ``pair_off`` [S+1] int64 (first atom /
+        pair of each structure), ``nmax`` [S] (longest neighbour list, 1000 entries included) and ``npairs`` [S]
+        (entries other than 1000).  ``indexes``: the current epoch order (default: a first ``on_epoch_end``, as
+        ``DataIterator`` does)."""
+        self.batch_size, self.shuffle, self.use_ring, self.feature = batch_size, shuffle, use_ring, "atomic"
+        self.weight_index, self.converter = weight_index, converter
+        for k in _DEVICE_ARRAYS:
+            setattr(self, k, arrays.get(k))
+        self.energy = np.asarray(energy, np.float32)
+        self.atom_off, self.pair_off = np.asarray(atom_off, np.int64), np.asarray(pair_off, np.int64)
+        self.n_atoms = np.diff(self.atom_off)
+        self.nmax, self.npairs = np.asarray(nmax, np.int64), np.asarray(npairs, np.int64)
+        self._perm = None
+        if indexes is None:
+            self.on_epoch_end()
+        else:
+            self.indexes, self._perm_stale = np.array(indexes, copy=True), True
+
+    # ------------------------------------------------------------------ constructors
+    @classmethod
+    def from_data_iterator(cls, it: "DataIterator", device=None) -> "DeviceDataIterator":
+        """Upload a host ``DataIterator``'s flat arrays once and take over its settings and its current order."""
+        _refuse_structures_route("DeviceDataIterator", False, getattr(it, "feature", "atomic"))
+        atom_off = np.asarray(it.atom_off, np.int64)
+        nbr_off = np.asarray(it.nbr_off, np.int64)
+        _check_int32_offsets(atom_off, nbr_off[atom_off])
+        pair_off, nmax, npairs = cls.host_sizes(atom_off, nbr_off, it.nbr_idx)
+        from . import _abi
+        import torch
+        _abi.require_gpu()
+        dev = device or torch.device("cuda", torch.cuda.current_device())
+
+        def up(a, dt):
+            return torch.from_numpy(np.ascontiguousarray(a, dt)).to(dev)
+        arrays = {"struct_atom_off": up(atom_off, np.int32), "atom_nbr_off": up(nbr_off, np.int32), "z": up(it.z, np.int32),
+                  "nbr_idx": up(it.nbr_idx, np.int32), "nbr_w": up(it.nbr_w, np.float32),
+                  "nbr_d": up(it.nbr_d, np.float32), "target": up(it.energy, np.float32),
+                  "ring": up(it.ring, np.int32) if it.use_ring else None}
+        return cls(arrays, it.energy, atom_off, pair_off, nmax, npairs, batch_size=it.batch_size, shuffle=it.shuffle,
+                   use_ring=it.use_ring, weight_index=it.weight_index, converter=it.converter, indexes=it.indexes)
+
+    @staticmethod
+    def host_sizes(atom_off, nbr_off, nbr_idx):
+        """Per-structure host arrays of a data set in ``DataIterator``'s CSR form: ``(pair_off [S+1], nmax [S],
+        npairs [S])``, the first pair row, the longest neighbour list (1000 entries included, as ``csr_item``'s ``N``)
+        and the entries other than 1000 (as ``load_batch_csr``'s pair count)."""
+        atom_off, nbr_off = np.asarray(atom_off, np.int64), np.asarray(nbr_off, np.int64)
+        pair_off = nbr_off[atom_off]
+        n_nb = np.append(np.diff(nbr_off), 0)
+        nmax = np.maximum.reduceat(n_nb, atom_off[:-1]) if len(atom_off) > 1 else np.zeros(0, np.int64)
+        nmax[np.diff(atom_off) == 0] = 0
+        valid = np.zeros(len(nbr_idx) + 1, np.int64)
+        np.cumsum(np.asarray(nbr_idx) != 1000, out=valid[1:])
+        return pair_off, nmax, valid[pair_off[1:]] - valid[pair_off[:-1]]
+
+    @classmethod
+    def from_structures(cls, structs, targets, batch_size: int = 32, shuffle: bool = False, g_update: bool = True,
+                        d_t: float = 4.0, w_t: float = 0.4, angle=None, cutoff: float = 13.0,
+                        allow_pathological: bool = False, converter: bool = False, use_ring: bool = False,
+                        feature: str = "atomic", device=None) -> "DeviceDataIterator":
+        """The iterator ``DataIterator(data_energy, compute_voronoi_neighbors(structs, d_t, w_t), ...)`` would be, with
+        the neighbour lists selected and flattened on the device (``voronoi.select_neighbors``, in the chunks of
+        ``predict_structures``): no facet record and no neighbour list reaches the host.  ``targets``: one value per
+        structure.  ``angle``: the weight column (True = solid angle, False = normalised); None picks the one
+        ``DataIterator`` trains a model with this ``g_update`` on.  ``d_t`` / ``w_t`` / ``cutoff`` /
+        ``allow_pathological``: as in ``compute_voronoi_neighbors``.
+
+        Refused: ``use_ring`` and ``feature='cgcnn'`` (``NotImplementedError``); structures without sites or with more
+        than 1000 (1000 is the reference's neighbour padding marker) (``ValueError``, naming the structure)."""
+        from . import voronoi as V
+        from .model import MAX_STRUCTURE_ATOMS, _structure_chunks
+        _refuse_structures_route("DeviceDataIterator.from_structures", use_ring, feature)
+        structs = list(structs)
+        targets = list(np.asarray(targets, dtype=object).reshape(-1))
+        if len(targets) != len(structs):
+            raise ValueError(f"{len(structs)} structures but {len(targets)} targets")
+        if batch_size < 1:
+            raise ValueError("batch_size must be >= 1")
+        lats, xs = V._arrays(structs)
+        for k, X in enumerate(xs):
+            if len(X) == 0:
+                raise ValueError(f"structure {k} has no sites")
+            if len(X) > MAX_STRUCTURE_ATOMS:
+                raise ValueError(f"structure {k} has {len(X)} sites: at most {MAX_STRUCTURE_ATOMS} (a neighbour index "
+                                 "of 1000 is the reference's padding marker and would be masked); train on such "
+                                 "structures from host-built batches: compute_voronoi_neighbors + DataIterator")
+        n_atoms = np.array([len(X) for X in xs], np.int64)
+        atom_off = np.zeros(len(structs) + 1, np.int64)
+        np.cumsum(n_atoms, out=atom_off[1:])
+        _check_int32_offsets(atom_off)
+        conv = 1000 if converter else 1.0
+        energy = np.array([float(t) * conv for t in targets], "float32")
+        column = bool(g_update) if angle is None else bool(angle)
+        import torch
+        from . import _abi
+        _abi.require_gpu()
+        dev = device or torch.device("cuda", torch.cuda.current_device())
+        A = int(atom_off[-1])
+        an = torch.empty(A + 1, dtype=torch.int32, device=dev)
+        z = torch.empty(A, dtype=torch.int32, device=dev)
+        parts, nmax, npairs, pbase = [], [], [], 0
+        for c0, c1 in _structure_chunks(n_atoms, batch_size):
+            sel = V.select_neighbors(structs[c0:c1], d_t, w_t, column, cutoff, allow_pathological, first_index=c0,
+                                     _checked=(lats[c0:c1], xs[c0:c1]))
+            csr = sel.csr()
+            a0, a1 = int(atom_off[c0]), int(atom_off[c1])
+            if pbase + csr["P"] > _INT32_MAX:
+                s = c0 + int(np.searchsorted(np.cumsum(csr["npairs"]), _INT32_MAX - pbase, side="right"))
+                raise ValueError(f"structure {s}: the data set's neighbour pairs exceed int32 offsets (at most "
+                                 f"{_INT32_MAX}); split it into data sets below 2^31 pairs")
+            an[a0:a1] = csr["atom_nbr_off"][:-1] + pbase      # rebased onto the whole data set's pair rows
+            z[a0:a1] = csr["z"]
+            parts.append((csr["nbr_idx"].clone(), csr["nbr_w"].clone(), csr["nbr_d"].clone()))
+            nmax.append(csr["nmax"])
+            npairs.append(csr["npairs"])
+            pbase += csr["P"]
+        an[A] = pbase
+        npairs = np.concatenate(npairs).astype(np.int64)
+        pair_off = np.zeros(len(structs) + 1, np.int64)
+        np.cumsum(npairs, out=pair_off[1:])
+
+        def cat(k, dt):
+            return torch.cat([p[k] for p in parts]) if parts else torch.empty(0, dtype=dt, device=dev)
+        arrays = {"struct_atom_off": torch.from_numpy(atom_off.astype(np.int32)).to(dev), "atom_nbr_off": an, "z": z,
+                  "nbr_idx": cat(0, torch.int32), "nbr_w": cat(1, torch.float32), "nbr_d": cat(2, torch.float32),
+                  "target": torch.from_numpy(energy).to(dev), "ring": None}
+        return cls(arrays, energy, atom_off, pair_off, np.concatenate(nmax), npairs, batch_size=batch_size,
+                   shuffle=shuffle, use_ring=False, weight_index=2 if column else 3, converter=conv)
+
+    # ------------------------------------------------------------------ Sequence protocol
+    def on_epoch_end(self):
+        self.indexes = np.arange(len(self.energy))                # exactly DataIterator.on_epoch_end
+        if self.shuffle:
+            np.random.shuffle(self.indexes)
+        self._perm_stale = True
+
+    def __len__(self):
+        return ceil(len(self.energy) / self.batch_size)
+
+    @property
+    def perm(self):
+        """The epoch's order on the device (int32 [S]); uploaded with one plain copy after each ``on_epoch_end``."""
+        import torch
+        if self._perm is None:
+            self._perm = torch.empty(len(self.energy), dtype=torch.int32, device=self.struct_atom_off.device)
+        if self._perm_stale:
+            self._perm.copy_(torch.from_numpy(self.indexes.astype(np.int32)))
+            self._perm_stale = False
+        return self._perm
+
+    def batch_shape(self, idx: int) -> Tuple[int, int, int, int, int]:
+        """``(start, B, M, N, P)`` of batch ``idx``: its first position in the epoch's order, its structures, most
+        atoms, longest neighbour list and valid pairs -- the arguments of ``Engine.load_batch_gather``."""
+        start = idx * self.batch_size
+        sel = self.indexes[start:start + self.batch_size]
+        if len(sel) == 0:
+            raise IndexError(f"batch {idx} out of range ({len(self)} batches)")
+        return (start, len(sel), int(self.n_atoms[sel].max()), int(self.nmax[sel].max()),
+                int(self.npairs[sel].sum()))
+
+    def batch_target(self, idx: int) -> np.ndarray:
+        return self.energy[self.indexes[idx * self.batch_size:(idx + 1) * self.batch_size]]
+
+    # ------------------------------------------------------------------ host forms (copied back from the device)
+    def csr_item(self, idx: int) -> Tuple[Dict[str, np.ndarray], np.ndarray]:
+        """``DataIterator.csr_item``: the batch's CSR slice, gathered from the device arrays."""
+        import torch
+        start, B, M, N, _ = self.batch_shape(idx)
+        sel = self.indexes[start:start + B]
+        dev = self.struct_atom_off.device
+        atoms = np.concatenate([np.arange(self.atom_off[s], self.atom_off[s + 1]) for s in sel])
+        pairs = np.concatenate([np.arange(self.pair_off[s], self.pair_off[s + 1]) for s in sel])
+        d_atoms = torch.from_numpy(atoms).to(dev)
+        d_pairs = torch.from_numpy(pairs).to(dev)
+        an = self.atom_nbr_off
+        n_nb = (an[d_atoms + 1] - an[d_atoms]).cpu().numpy()
+        sa = np.zeros(B + 1, np.int32)
+        np.cumsum(self.n_atoms[sel], out=sa[1:])
+        ao = np.zeros(len(atoms) + 1, np.int32)
+        np.cumsum(n_nb, out=ao[1:])
+        csr = {"struct_atom_off": sa, "atom_nbr_off": ao, "z": self.z[d_atoms].cpu().numpy(),
+               "nbr_idx": self.nbr_idx[d_pairs].cpu().numpy(), "nbr_w": self.nbr_w[d_pairs].cpu().numpy(),
+               "nbr_d": self.nbr_d[d_pairs].cpu().numpy(), "M": M, "N": N}
+        if self.use_ring:
+            csr["ring"] = self.ring[d_atoms].cpu().numpy()
+        return csr, self.energy[sel]
+
+    def __getitem__(self, idx: int):
+        """``DataIterator.__getitem__``: the padded batch, gathered by ``scann_gather_batch`` and copied back."""
+        import torch
+        from ._abi import check, lib
+        start, B, M, N, _ = self.batch_shape(idx)
+        dev = self.struct_atom_off.device
+        i32, f32, u8 = (dict(dtype=t, device=dev) for t in (torch.int32, torch.float32, torch.uint8))
+        atomic, amask = torch.empty(B * M, **i32), torch.empty(B * M, **u8)
+        nbr, nmask = torch.empty(B * M * N, **i32), torch.empty(B * M * N, **u8)
+        w, d = torch.empty(B * M * N, **f32), torch.empty(B * M * N, **f32)
+        ring = torch.empty(B * M * 2, **f32) if self.use_ring else None
+        tgt = torch.empty(B, **f32)
+        perm = self.perm
+        check(lib.scann_gather_batch(self.struct_atom_off.data_ptr(), self.atom_nbr_off.data_ptr(), self.z.data_ptr(),
+                                     self.nbr_idx.data_ptr(), self.nbr_w.data_ptr(), self.nbr_d.data_ptr(),
+                                     self.ring.data_ptr() if self.use_ring else None, self.target.data_ptr(),
+                                     perm.data_ptr() + 4 * start, B, M, N, atomic.data_ptr(), amask.data_ptr(),
+                                     nbr.data_ptr(), nmask.data_ptr(), w.data_ptr(), d.data_ptr(),
+                                     ring.data_ptr() if ring is not None else None, tgt.data_ptr(),
+                                     torch.cuda.current_stream(dev).cuda_stream), "gather_batch")
+        atomic = atomic.cpu().numpy().reshape(B, M)
+        out = {"atomic": atomic, "atom_mask": amask.cpu().numpy().reshape(B, M, 1).astype(bool),
+               "neighbors": nbr.cpu().numpy().reshape(B, M, N),
+               "neighbor_mask": nmask.cpu().numpy().reshape(B, M, N).astype(bool),
+               "neighbor_weight": w.cpu().numpy().reshape(B, M, N), "neighbor_distance": d.cpu().numpy().reshape(B, M, N)}
+        if ring is not None:
+            out["ring_aromatic"] = ring.cpu().numpy().reshape(B, M, 2).astype(np.int32)
+        return out, tgt.cpu().numpy()
 
 
 def pack_padded(csr: Dict[str, np.ndarray]) -> Dict[str, np.ndarray]:

@@ -476,6 +476,37 @@ class Engine:
             self._plan(b)
         return b
 
+    def load_batch_gather(self, data, start: int, B: int, M: int, N: int, P: int, plan: bool = True) -> Batch:
+        """Batch of structures ``data.perm[start:start + B]`` of a device-resident data set
+        (``datagenerator.DeviceDataIterator``), padded by ``scann_gather_batch`` into the buffers of the shape class
+        ``(B, M, N, P)`` -- the exact sizes of the batch, so that it shares the class and the captured graphs of the
+        same structures loaded by ``load_batch_csr``.  The targets go to ``b.target``.  Nothing crosses to or from the
+        host."""
+        B, M, N, P = int(B), int(M), int(N), int(P)
+        if B <= 0 or M <= 0 or N <= 0:
+            raise ValueError(f"gather_batch: bad shape B={B} M={M} N={N}")
+        if start < 0 or start + B > data.perm.numel():
+            raise ValueError(f"gather_batch: structures {start}..{start + B} outside the permutation of "
+                             f"{data.perm.numel()}")
+        b = self._get_batch(B, M, N, P)
+        b.P_host = P
+        b.h2d_bytes = 0
+        b.host_dirty = False            # the pinned mirror is stale: it must not be copied over what is gathered here
+        use_ring = self.spec.use_ring
+        if use_ring and data.ring is None:
+            raise ValueError("this model reads ring / aromatic flags: the data set has none (use_ring=False)")
+        self._ev("gather_batch", True)
+        check(lib.scann_gather_batch(_p(data.struct_atom_off), _p(data.atom_nbr_off), _p(data.z), _p(data.nbr_idx),
+                                     _p(data.nbr_w), _p(data.nbr_d), _p(data.ring) if use_ring else 0, _p(data.target),
+                                     _p(data.perm, start), B, M, N, _p(b.atomic), _p(b.atom_mask), _p(b.nbr),
+                                     _p(b.nmask), _p(b.weight), _p(b.dist), _p(b.ring), _p(b.target), self._stream()),
+              "gather_batch")
+        self._ev("gather_batch", False)
+        self.launches += 1
+        if plan:
+            self._plan(b)
+        return b
+
     def _pack_csr(self, b: Batch, blob: torch.Tensor, offs: Dict[str, int]) -> None:
         """CSR blob on the device -> the padded buffers of the batch's shape class (scann_pack_batch)."""
         b.host_dirty = False            # the pinned mirror is stale: it must not be copied over what is packed here

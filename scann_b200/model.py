@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from .config import ModelSpec, fill_cli_defaults, model_spec
-from .engine import Engine
+from .engine import Batch, Engine
 from .params import ParamLayout
 
 
@@ -67,6 +67,13 @@ def _structure_chunks(n_atoms, batch_size: int):
     if c0 < len(n_atoms):
         out.append((c0, len(n_atoms)))
     return out
+
+
+def _batch_errors(y, y_true) -> Dict[str, float]:
+    """MAE / RMSE of one batch's predictions (``evaluate_batch``)."""
+    y = np.asarray(y).reshape(-1)
+    t = np.asarray(y_true, np.float32).reshape(-1)
+    return {"mae": float(np.abs(y - t).mean()), "rmse": float(np.sqrt(((y - t) ** 2).mean()))}
 
 
 def _ragged_capable(seq) -> bool:
@@ -280,7 +287,9 @@ class ScannKerasModel:
         -- Keras' fit does the same with its asynchronous metric tensors."""
         eng = self.engine
         eng.train_dropout = bool(self.dropout) and eng.use_chain and eng.use_wgrad_batch
-        if "struct_atom_off" in inputs:
+        if isinstance(inputs, Batch):             # gathered on the device (Engine.load_batch_gather), targets included
+            b, y_true = inputs, inputs.target
+        elif "struct_atom_off" in inputs:
             b = eng.load_batch_csr(inputs, target=y_true, plan=False)
             y_true = b.target
         else:
@@ -310,14 +319,25 @@ class ScannKerasModel:
 
     def evaluate_batch(self, inputs, y_true) -> Dict[str, float]:
         y = self.predict(inputs)
-        y = (y[0] if isinstance(y, list) else y).reshape(-1)
-        t = np.asarray(y_true, np.float32).reshape(-1)
-        return {"mae": float(np.abs(y - t).mean()), "rmse": float(np.sqrt(((y - t) ** 2).mean()))}
+        return _batch_errors(y[0] if isinstance(y, list) else y, y_true)
+
+    def predict_device_batch(self, data, idx: int):
+        """Predictions of batch ``idx`` of a ``DeviceDataIterator``, gathered on the device: ``(y [B, 1], targets
+        [B])`` as host float32 arrays -- the same values ``predict(data[idx][0])`` gives."""
+        eng = self.engine
+        b = eng.load_batch_gather(data, *data.batch_shape(idx), plan=False)
+        y, _ = eng.predict_step(b, replan=True)
+        y_h = y.cpu().numpy().reshape(b.B, 1)          # synchronises the stream
+        self.last_e2e_bytes = (0, y.numel() * 4)
+        return y_h, data.batch_target(idx)
 
     def fit(self, x, epochs: int = 1, validation_data=None, callbacks=None, verbose: int = 2, shuffle: bool = False,
             **_ignored) -> History:
         """``model.fit(trainIter, epochs, validation_data=validIter, ...)`` (scann_model.py:232-241) over a
-        ``Sequence``-like iterator (``len``, ``__getitem__`` -> (inputs, target), ``on_epoch_end``)."""
+        ``Sequence``-like iterator (``len``, ``__getitem__`` -> (inputs, target), ``on_epoch_end``).  A
+        ``DeviceDataIterator`` (as ``x`` or as ``validation_data``) has its batches gathered on the device."""
+        from .datagenerator import DeviceDataIterator
+        on_device = isinstance(x, DeviceDataIterator)
         hist = History()
         callbacks = list(callbacks or [])
         self.stop_training = False
@@ -343,8 +363,11 @@ class ScannKerasModel:
             eng.overlap_h2d = True
             try:
                 for i in range(len(x)):
-                    # iterators that can hand out the ragged CSR form skip the host-side padding altogether
-                    inputs, target = x.csr_item(i) if _ragged_capable(x) else x[i]
+                    if on_device:                 # a device-resident data set: no host->device copy at all
+                        inputs, target = eng.load_batch_gather(x, *x.batch_shape(i), plan=False), None
+                    else:
+                        # iterators that can hand out the ragged CSR form skip the host-side padding altogether
+                        inputs, target = x.csr_item(i) if _ragged_capable(x) else x[i]
                     pending.append(self._train_on_batch_async(inputs, target))
                     harvest(4)                    # results older than 4 steps (long finished; ring of 8 slots)
                 harvest(0)
@@ -354,7 +377,12 @@ class ScannKerasModel:
             hist.add("loss", float(np.mean(losses)))
             hist.add("mae", float(np.mean(maes)))
             if validation_data is not None:
-                v = [self.evaluate_batch(*validation_data[i]) for i in range(len(validation_data))]
+                if isinstance(validation_data, DeviceDataIterator):
+                    v = [_batch_errors(*self.predict_device_batch(validation_data, i))
+                         for i in range(len(validation_data))]
+                    eng.check_status()
+                else:
+                    v = [self.evaluate_batch(*validation_data[i]) for i in range(len(validation_data))]
                 hist.add("val_mae", float(np.mean([m["mae"] for m in v])))
             if hasattr(x, "on_epoch_end"):
                 x.on_epoch_end()
@@ -547,10 +575,24 @@ class SCANN:
         ``hyper.data_nei_path``, written by the reference's preprocessing), standardise the target when
         ``hyper.scaler`` is set (float32 mean / std, recorded in the config as strings like the reference), split it
         with the global numpy generator and attach ``trainIter`` / ``validIter`` / ``testIter`` (or ``dataIter``)."""
-        from .datagenerator import DataIterator, load_dataset, split_data
+        from .datagenerator import DataIterator, load_dataset
         hy, cm = self.config["hyper"], self.config["model"]
         data_energy, data_neighbor = load_dataset(hy["data_energy_path"], hy["data_nei_path"], hy["target"],
                                                   use_ref=hy["use_ref"], use_ring=cm["use_ring"])
+        self._scale_targets(data_energy)
+
+        def iterator(indices=None, shuffle=False):
+            return DataIterator(batch_size=hy["batch_size"], use_ring=cm["use_ring"], shuffle=shuffle,
+                                feature=cm["feature"], g_update=cm["g_update"],
+                                data_neighbor=data_neighbor if indices is None else data_neighbor[indices],
+                                data_energy=data_energy if indices is None else data_energy[indices])
+
+        return self._attach_iterators(len(data_energy), iterator, split)
+
+    def _scale_targets(self, data_energy) -> None:
+        """Standardise column 1 of the rows in place when ``hyper.scaler`` is set (float32 mean / std) and record the
+        scaling and the data-set size in the config (scann_model.py:117-131)."""
+        hy = self.config["hyper"]
         if hy["scaler"]:
             values = [row[1] for row in data_energy]
             self.mean, self.std = np.mean(values, dtype="float32"), np.std(values, dtype="float32")
@@ -559,16 +601,14 @@ class SCANN:
         hy["target_mean"], hy["target_std"] = str(self.mean), str(self.std)
         hy["data_size"] = len(data_energy)
 
-        def iterator(indices=None, shuffle=False):
-            return DataIterator(batch_size=hy["batch_size"], use_ring=cm["use_ring"], shuffle=shuffle,
-                                feature=cm["feature"], g_update=cm["g_update"],
-                                data_neighbor=data_neighbor if indices is None else data_neighbor[indices],
-                                data_energy=data_energy if indices is None else data_energy[indices])
-
+    def _attach_iterators(self, n: int, iterator, split: bool):
+        """``dataIter``, or the train | valid | test split of the global numpy generator (scann_model.py:133-161)."""
+        from .datagenerator import split_data
+        hy = self.config["hyper"]
         if not split:
             self.dataIter = iterator()
             return None
-        train, valid, test, extra = split_data(len_data=len(data_energy), test_percent=hy["test_percent"],
+        train, valid, test, extra = split_data(len_data=n, test_percent=hy["test_percent"],
                                                train_size=hy["train_size"], test_size=hy["test_size"])
         assert len(extra) == 0, "Split was inexact {} {} {} {}".format(len(train), len(valid), len(test), len(extra))
         print("Number of train data : ", len(train), " , Number of valid data: ", len(valid),
@@ -577,6 +617,39 @@ class SCANN:
         self.trainIter, self.validIter, self.testIter = [iterator(ix, shuffle=(len(ix) == len(train)))
                                                          for ix in (train, valid, test)]
         return train, valid, test
+
+    def _prepare_structures(self, structs, targets, split: bool = True, **voronoi_args):
+        """``SCANN.prepare_structures``: see the property."""
+        from .datagenerator import DeviceDataIterator, _refuse_structures_route
+        hy, cm = self.config["hyper"], self.config["model"]
+        _refuse_structures_route("SCANN.prepare_structures", cm["use_ring"], cm["feature"])
+        structs = list(structs)
+        targets = list(np.asarray(targets, dtype=object).reshape(-1))
+        if len(targets) != len(structs):
+            raise ValueError(f"{len(structs)} structures but {len(targets)} targets")
+        rows = np.empty((len(structs), 2), dtype=object)          # the rows of load_dataset: [atoms, target]
+        rows[:, 1] = [float(t) for t in targets]
+        self._scale_targets(rows)
+
+        def iterator(indices=None, shuffle=False):
+            ix = range(len(structs)) if indices is None else indices
+            return DeviceDataIterator.from_structures([structs[k] for k in ix], rows[list(ix), 1],
+                                                      batch_size=hy["batch_size"], shuffle=shuffle,
+                                                      g_update=cm["g_update"], use_ring=cm["use_ring"],
+                                                      feature=cm["feature"], **voronoi_args)
+
+        return self._attach_iterators(len(structs), iterator, split)
+
+    @property
+    def prepare_structures(self):
+        """``prepare_structures(structs, targets, split=True, **voronoi_args)``: ``prepare_dataset`` for structures
+        and their targets instead of the reference's data files.  The same target scaling (``hyper.scaler``), config
+        entries and split of the global numpy generator; ``trainIter`` / ``validIter`` / ``testIter`` (or ``dataIter``)
+        are ``DeviceDataIterator.from_structures`` (``voronoi_args``: ``d_t``, ``w_t``, ``angle``, ``cutoff``,
+        ``allow_pathological``, ``converter``), so training and evaluation gather their batches on the device.
+        Refused for ``use_ring`` and ``feature='cgcnn'`` models.  (A property for the same reason as
+        ``predict_structures``.)"""
+        return functools.partial(SCANN._prepare_structures, self)
 
     def create_callbacks(self):
         """ModelCheckpoint(best val_mae) + EarlyStopping(patience 200) + SGDRC / lr logging (scann_model.py:163-197)."""
@@ -616,16 +689,22 @@ class SCANN:
                 self.model = create_model(self.config)
             self.model.load_weights(best)
             self._evaluate_from_checkpoint = False
+        from .datagenerator import DeviceDataIterator
         data = self.dataIter if hasattr(self, "dataIter") else self.testIter
         y, y_predict = [], []
         for i in range(len(data)):
-            inputs, target = data[i]
-            out = self.model.predict(inputs)
-            out = out[0] if isinstance(out, list) else out
+            if isinstance(data, DeviceDataIterator):
+                out, target = self.model.predict_device_batch(data, i)
+            else:
+                inputs, target = data[i]
+                out = self.model.predict(inputs)
+                out = out[0] if isinstance(out, list) else out
             y.extend(np.asarray(target, np.float64).reshape(-1).tolist())
             y_predict.extend(np.asarray(out, np.float64).reshape(-1).tolist())
             if i % 10 == 0:
                 print(f"{i}/{len(data)}")
+        if isinstance(data, DeviceDataIterator):
+            self.model.engine.check_status()
         ya, yp = np.asarray(y), np.asarray(y_predict)
         mae = float(np.abs(ya - yp).mean()) * self.std
         ss_tot = float(((ya - ya.mean()) ** 2).sum())
