@@ -100,6 +100,24 @@ int scann_gather_batch(const int32_t* struct_atom_off, const int32_t* atom_nbr_o
                        uint8_t* atom_mask, int32_t* neighbors, uint8_t* neighbor_mask, float* weight, float* dist,
                        float* ring_out, float* target, void* stream);
 
+/* ---- local-attention scores -> user layouts ----------------------------------------------------------------------
+ * attn [L, rows, 8] fp32: what the local-attention forward kernels store through their `attn` pointer for the L layers
+ * of one batch (layer l at attn + l * rows * 8, 16-byte aligned; pair-plan row p, head h at [p * 8 + h]), with the
+ * plan of scann_plan_build.  Integer index arithmetic only; outputs caller-allocated.
+ * scann_attn_to_padded writes out [L][B][8][M][N], the layout of the first output of the reference's
+ * LocalAttention.call (attn[B,H,M,N], scann/layers/attention.py:186-189, :216): valid slot (r, n) holds the value of
+ * plan row rowptr[r] + k, k = the valid slots of row r before n; a masked slot is exactly 0; a row with cnt[r] == 0
+ * (a padded atom or an atom without valid neighbours) is 1/N, the reference's fp32 softmax over N logits that the
+ * mask's -1e9 makes equal.  B, M, N > 0 and B * 8 * M * N < 2^31.
+ * scann_attn_to_csr writes out [L][8][ld]: entry i < *nvalid (<= ld) of the plan's compact list valid_rows is pair i
+ * of the batch in atom-row order and, per atom, in slot order.  PRECONDITION: for a batch packed by scann_pack_batch,
+ * that is the order of the CSR neighbour lists only if they hold no padding marker 1000 (true of the lists of
+ * scann_voronoi_batch_csr); a marker's slot is masked and has no entry.  Entries at and above *nvalid are not written. */
+int scann_attn_to_padded(const float* attn, int L, long long rows, const int32_t* cnt, const int32_t* rowptr,
+                         const uint8_t* neighbor_mask, int B, int M, int N, float* out, void* stream);
+int scann_attn_to_csr(const float* attn, int L, long long rows, const int32_t* valid_rows, const int32_t* nvalid, int ld,
+                      float* out, void* stream);
+
 /* ---- input embedding: Embedding + (extra_embed) + dense_embed swish -----------------------
  * scann/models/scann_model.py:361-374.  ring may be NULL (use_ring False). t0 (pre-activation,
  * saved for backward) may be NULL. */

@@ -28,6 +28,8 @@ PROTOTYPES = {
     "scann_plan_build": (ci, [vp, vp, vp, vp, ci, ci, ci, ci, ci, ci] + [vp] * 13 + [vp, ci, vp, vp]),
     "scann_pack_batch": (ci, [vp] + [C.c_longlong] * 8 + [ci, ci, ci] + [vp] * 8 + [vp]),
     "scann_gather_batch": (ci, [vp] * 9 + [ci, ci, ci] + [vp] * 8 + [vp]),
+    "scann_attn_to_padded": (ci, [vp, ci, C.c_longlong, vp, vp, vp, ci, ci, ci, vp, vp]),
+    "scann_attn_to_csr": (ci, [vp, ci, C.c_longlong, vp, vp, ci, vp, vp]),
     "scann_embed_forward": (ci, [vp, vp, ci, ci, ci] + [vp] * 7 + [vp, vp, vp, vp]),
     "scann_cgcnn_embed_forward": (ci, [vp, vp, vp, ci, ci, ci, vp, vp]),
     "scann_cgcnn_embed_backward": (ci, [vp, vp, vp, ci, ci, ci] + [vp] * 12 + [vp, vp]),

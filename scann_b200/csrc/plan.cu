@@ -438,3 +438,93 @@ extern "C" int scann_plan_build(const uint8_t* neighbor_mask, const int32_t* nei
                                                      pair_w, valid_rows, valid_j, gcbase);
     return scann_check_launch("scann_plan_build");
 }
+
+// ---------------------------------------------------------------------------------------------
+// Local-attention scores: pair-plan order -> the user's layouts.  The forward kernels store the softmax of every
+// valid pair through their `attn` pointer, [rows, 8] per layer in plan order (layer l at attn + l * rows * 8).
+// ---------------------------------------------------------------------------------------------
+
+// out [L][B][8][M][N], the first output of LocalAttention.call (scann/layers/attention.py:186-189, :216).  One thread
+// per padded slot (b, m, n) and layer (blockIdx.y): it reads the slot's 8 heads in one 32-byte row and writes them to
+// 8 planes, so the stores of a warp are contiguous in n and m.  The plan keeps an atom's pairs contiguous and in slot
+// order (plan_fill_kernel), so valid slot n of row r is plan row rowptr[r] + (valid slots of row r before n).
+__global__ void attn_to_padded_kernel(const float* __restrict__ attn, long long rows, const int32_t* __restrict__ cnt,
+                                      const int32_t* __restrict__ rowptr, const uint8_t* __restrict__ nmask, int B,
+                                      int M, int N, float* __restrict__ out) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    const int T = B * M * N;
+    if (t >= T) return;
+    const int l = blockIdx.y;
+    const int r = t / N, n = t - r * N;
+    const int b = r / M, mn = t - b * M * N;
+    const size_t plane = (size_t)M * N;
+    float* o = out + ((size_t)l * B + b) * 8 * plane + mn;
+    const int c = cnt[r];
+    if (c == 0) {
+        // no valid neighbour: the mask adds -1e9 to every logit, which absorbs |s| < 32 in fp32, so the softmax of
+        // the N equal logits is uniform
+        const float u = 1.0f / (float)N;
+#pragma unroll
+        for (int h = 0; h < 8; ++h) o[h * plane] = u;
+        return;
+    }
+    const uint8_t* m = nmask + (size_t)r * N;
+    if (!m[n]) {
+#pragma unroll
+        for (int h = 0; h < 8; ++h) o[h * plane] = 0.0f;
+        return;
+    }
+    int k = 0;
+    for (int j = 0; j < n; ++j) k += m[j] != 0;
+    const float4* a = reinterpret_cast<const float4*>(attn + ((size_t)l * rows + rowptr[r] + k) * 8);
+    const float4 a0 = a[0], a1 = a[1];
+    o[0] = a0.x; o[plane] = a0.y; o[2 * plane] = a0.z; o[3 * plane] = a0.w;
+    o[4 * plane] = a1.x; o[5 * plane] = a1.y; o[6 * plane] = a1.z; o[7 * plane] = a1.w;
+}
+
+// out [L][8][ld]: the compact list of the plan (valid_rows, nvalid) holds the valid pairs in atom-row order and, per
+// atom, in slot order, so entry i of the list is pair i of the batch's CSR neighbour lists whenever those lists carry
+// no padding marker.  One thread per list entry and layer.
+__global__ void attn_to_csr_kernel(const float* __restrict__ attn, long long rows, const int32_t* __restrict__ valid_rows,
+                                   const int32_t* __restrict__ nvalid, int ld, float* __restrict__ out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= ld || i >= *nvalid) return;
+    const int l = blockIdx.y;
+    const float4* a = reinterpret_cast<const float4*>(attn + ((size_t)l * rows + valid_rows[i]) * 8);
+    const float4 a0 = a[0], a1 = a[1];
+    float* o = out + (size_t)l * 8 * ld + i;
+    o[0] = a0.x; o[(size_t)ld] = a0.y; o[2 * (size_t)ld] = a0.z; o[3 * (size_t)ld] = a0.w;
+    o[4 * (size_t)ld] = a1.x; o[5 * (size_t)ld] = a1.y; o[6 * (size_t)ld] = a1.z; o[7 * (size_t)ld] = a1.w;
+}
+
+static int attn_args_ok(const char* who, const float* attn, int L, long long rows, const float* out) {
+    if (L <= 0 || L > 65535) { scann_set_error("%s: bad layer count L=%d", who, L); return 0; }
+    if (rows <= 0 || rows > 0x7fffffffLL) { scann_set_error("%s: bad plan row count %lld", who, rows); return 0; }
+    if (!attn || !out) { scann_set_error("%s: attn / out is NULL", who); return 0; }
+    if ((uintptr_t)attn & 15) { scann_set_error("%s: attn must be 16-byte aligned", who); return 0; }
+    return 1;
+}
+
+extern "C" int scann_attn_to_padded(const float* attn, int L, long long rows, const int32_t* cnt, const int32_t* rowptr,
+                                    const uint8_t* neighbor_mask, int B, int M, int N, float* out, void* stream) {
+    if (!attn_args_ok("attn_to_padded", attn, L, rows, out)) return 1;
+    if (!pack_shape_ok("attn_to_padded", B, M, N)) return 1;
+    if ((long long)B * 8 * M * N > 0x7fffffffLL) {
+        scann_set_error("attn_to_padded: B*8*M*N = %lld scores per layer exceed int32", (long long)B * 8 * M * N);
+        return 1;
+    }
+    if (!cnt || !rowptr || !neighbor_mask) { scann_set_error("attn_to_padded: cnt / rowptr / neighbor_mask is NULL"); return 1; }
+    const int T = B * M * N;
+    attn_to_padded_kernel<<<dim3((T + 255) / 256, L), 256, 0, (cudaStream_t)stream>>>(attn, rows, cnt, rowptr,
+                                                                                      neighbor_mask, B, M, N, out);
+    return scann_check_launch("scann_attn_to_padded");
+}
+
+extern "C" int scann_attn_to_csr(const float* attn, int L, long long rows, const int32_t* valid_rows,
+                                 const int32_t* nvalid, int ld, float* out, void* stream) {
+    if (!attn_args_ok("attn_to_csr", attn, L, rows, out)) return 1;
+    if (ld <= 0) { scann_set_error("attn_to_csr: bad ld=%d", ld); return 1; }
+    if (!valid_rows || !nvalid) { scann_set_error("attn_to_csr: valid_rows / nvalid is NULL"); return 1; }
+    attn_to_csr_kernel<<<dim3((ld + 255) / 256, L), 256, 0, (cudaStream_t)stream>>>(attn, rows, valid_rows, nvalid, ld, out);
+    return scann_check_launch("scann_attn_to_csr");
+}

@@ -562,6 +562,10 @@ class Engine:
         # on the buffer being zero when it is first used (scann_plan_build)
         b.scratch = torch.zeros(6 * ngroups + 16, **i32)
         b.inv_ptr = None            # inverse neighbour CSR (deterministic mode, scann_plan_inverse)
+        # local-attention scores (predict_step(local_attention=...)), allocated when first requested: [L, rows, 8] in
+        # plan order as the kernels store them, and per layout the unpacked copy
+        b.attn = None
+        b.scores = {}
         b.graphs = {}
         return b
 
@@ -845,9 +849,10 @@ class Engine:
               "embed_forward")
         self.launches += 1
 
-    def forward(self, b: Batch, training: bool = False, attn_out: Optional[list] = None, replan: bool = False,
+    def forward(self, b: Batch, training: bool = False, attn: Optional[torch.Tensor] = None, replan: bool = False,
                 side_work=None):
-        """Runs the whole graph; returns (y[B], ga[B*M]) device tensors (views of the workspace).
+        """Runs the whole graph; returns (y[B], ga[B*M]) device tensors (views of the workspace).  ``attn``
+        ([L, rows, 8] fp32, or None): the local-attention kernels store every layer's softmax there, in pair-plan order.
 
         Two branches meet in front of the first per-atom projection: the pair plan (``replan``) and the geometry
         initialisation need the neighbour lists only, the weight operand images and the embedding need the atoms
@@ -897,7 +902,7 @@ class Engine:
         if embed_ev is not None:
             main.wait_event(embed_ev)         # x_0 and the weight images are ready
         if self.use_chain and (not training or self.tc_la_bwd):
-            return self._forward_chained(b, ws, training, attn_out)    # (first launch without PDL, then switched on)
+            return self._forward_chained(b, ws, training, attn)    # (first launch without PDL, then switched on)
         self._pdl(not fork)
         for l in range(L):
             la = layer_name("local_attention", l)
@@ -909,10 +914,7 @@ class Engine:
             fg = f"{la}/filter_geo/kernel"
             ctxpre = ws["ctxpre"][l] if training else None
             out = h if sp.use_attn_norm else x_out
-            attn = None
-            if attn_out is not None:
-                attn = torch.zeros(b.rows, 8, dtype=torch.float32, device=self.device)
-                attn_out.append(attn)
+            attn_l = _p(attn, l * b.rows * 8)
             if not sp.g_update:
                 # SCANN without geometry update (attention.py:155): only the query block of proj is needed
                 self._dense([_p(x_in)], D, [self.w(f"{la}/query/kernel")], [self.w(f"{la}/query/bias")], 1, 1, R,
@@ -923,7 +925,7 @@ class Engine:
                     self.la_grid, b.stride, b.mma_rows, _p(b.ntiles), _p(b.tile_a0), _p(b.tile_a1), _p(b.cnt), _p(b.rowptr), _p(b.pair_c),
                     _p(b.pair_j), _p(x_in), _p(proj), _p(b.pair_d), _p(b.pair_w), _p(self.centers_d), self.w(fg),
                     self.w(f"{la}/filter_geo/bias"), self.w(f"{la}/key/kernel"), self.w(f"{la}/key/bias"),
-                    self.w(f"{la}/layer_norm/gamma"), self.w(f"{la}/layer_norm/beta"), 0, _p(out), _p(attn), 0, 0, *self._adrop(training, l), st),
+                    self.w(f"{la}/layer_norm/gamma"), self.w(f"{la}/layer_norm/beta"), 0, _p(out), attn_l, 0, 0, *self._adrop(training, l), st),
                     "la_forward_noupdate_tc")
                 self.launches += 2
                 if sp.use_attn_norm:
@@ -946,7 +948,7 @@ class Engine:
                        self.w(fg, D * D), self.w(f"{la}/key/kernel"), self.w(f"{la}/key/bias"),
                        self.w(f"{la}/layer_norm_g/gamma"), self.w(f"{la}/layer_norm_g/beta"),
                        self.w(f"{la}/layer_norm/gamma"), self.w(f"{la}/layer_norm/beta"),
-                       _p(g_out), _p(ctxpre), _p(out), _p(attn))
+                       _p(g_out), _p(ctxpre), _p(out), attn_l)
             if "la_fwd" in self._skip:
                 pass
             elif self.tc_la_fwd:
@@ -998,7 +1000,7 @@ class Engine:
                                             gg, bg, gam, bet, g_out, ctxpre, out, attn, pre_out, k_out, *adrop,
                                             _p(self.status), st), "la_forward_pipe")
 
-    def _forward_chained(self, b: Batch, ws: dict, training: bool, attn_out: Optional[list]):
+    def _forward_chained(self, b: Batch, ws: dict, training: bool, attn: Optional[torch.Tensor]):
         """Layers of the forward pass with the per-atom Dense layers fused (scann_dense_chain):
         [projections of layer 0] -> LA_0 -> [ResidualNorm_0 + projections of layer 1] -> LA_1 -> ... ->
         [ResidualNorm_{L-1} + after_Lc + GlobalAttention q/k] -> GA + head."""
@@ -1039,10 +1041,7 @@ class Engine:
             fg = f"{la}/filter_geo/kernel"
             li, x_in, x_out, proj, h, h1, out = bufs(l)
             ctxpre = ws["ctxpre"][l] if training else None
-            attn = None
-            if attn_out is not None:
-                attn = torch.zeros(b.rows, 8, dtype=torch.float32, device=self.device)
-                attn_out.append(attn)
+            attn_l = _p(attn, l * b.rows * 8)
             self._ev("la_forward", True)
             if "la_fwd" in self._skip:
                 pass
@@ -1055,7 +1054,7 @@ class Engine:
                     _p(b.pair_c), _p(b.pair_j), _p(x_in), _p(proj), _p(g_in), self.w(fg, D * D),
                     self.w(f"{la}/key/kernel"), self.w(f"{la}/key/bias"), self.w(f"{la}/layer_norm_g/gamma"),
                     self.w(f"{la}/layer_norm_g/beta"), self.w(f"{la}/layer_norm/gamma"),
-                    self.w(f"{la}/layer_norm/beta"), _p(g_out), _p(ctxpre), _p(out), _p(attn)),
+                    self.w(f"{la}/layer_norm/beta"), _p(g_out), _p(ctxpre), _p(out), attn_l),
                     _p(ws["pre"][l]) if save else 0, _p(ws["kk"][l]) if save else 0, self._adrop(training, l), st)
                 self.launches += 2
             elif self.noup_pipe and b.stride == 32 and "gsave" in ws:
@@ -1067,7 +1066,7 @@ class Engine:
                 check(lib.scann_la_forward_pipe(
                     self.la_grid, b.rows, 2, _p(b.ntiles), _p(b.pair_c), _p(b.pair_j), _p(x_in), _p(proj), 0, 0,
                     self.w(f"{la}/key/kernel"), self.w(f"{la}/key/bias"), 0, 0, self.w(f"{la}/layer_norm/gamma"),
-                    self.w(f"{la}/layer_norm/beta"), _p(gbuf), _p(ctxpre), _p(out), _p(attn), 0,
+                    self.w(f"{la}/layer_norm/beta"), _p(gbuf), _p(ctxpre), _p(out), attn_l, 0,
                     _p(ws["kk"][l]) if training else 0, *self._adrop(training, l), _p(self.status), st),
                     "la_forward_pipe")
                 self.launches += 2
@@ -1076,7 +1075,7 @@ class Engine:
                     self.la_grid, b.stride, b.mma_rows, _p(b.ntiles), _p(b.tile_a0), _p(b.tile_a1), _p(b.cnt), _p(b.rowptr),
                     _p(b.pair_c), _p(b.pair_j), _p(x_in), _p(proj), _p(b.pair_d), _p(b.pair_w), _p(self.centers_d),
                     self.w(fg), self.w(f"{la}/filter_geo/bias"), self.w(f"{la}/key/kernel"), self.w(f"{la}/key/bias"),
-                    self.w(f"{la}/layer_norm/gamma"), self.w(f"{la}/layer_norm/beta"), _p(ctxpre), _p(out), _p(attn),
+                    self.w(f"{la}/layer_norm/gamma"), self.w(f"{la}/layer_norm/beta"), _p(ctxpre), _p(out), attn_l,
                     _p(ws["gsave"][l]) if training else 0, _p(ws["kk"][l]) if training else 0, *self._adrop(training, l), st),
                     "la_forward_noupdate_tc")
                 self.launches += 1
@@ -1680,27 +1679,79 @@ class Engine:
                                       int(apply), self._stream()), "adam_step")
         self.launches += 1
 
-    def predict_step(self, b: Batch, replan: bool = False):
-        """Inference forward (plan + graph of kernels) -> (y[B], ga[B*M]) device tensors."""
-        key = ("infer", replan)
+    def predict_step(self, b: Batch, replan: bool = False, local_attention=False):
+        """Inference forward (plan + graph of kernels) -> (y[B], ga[B*M]) device tensors.
+
+        ``local_attention``: also return every layer's local-attention scores, ``(y, ga, scores)``.  The kernels store
+        them in plan order and one more launch unpacks them (``_unpack_scores``); the graph that does so is captured
+        under its own key, ``("infer", replan, layout)``, so the graph without scores stays as it is.  True or
+        ``"padded"``: scores [L, B, 8, M, N], the reference's layout.  ``"csr"``: scores [L, 8, rows] whose first P
+        columns are the batch's P pairs in the order of its CSR neighbour lists (lists without the padding marker
+        1000, as ``voronoi.NeighborSelection.csr`` writes them).  The tensors belong to the shape class: the next step
+        of the class overwrites them."""
+        layout = score_layout(local_attention)
+        key = ("infer", replan) if layout is None else ("infer", replan, layout)
         self._flush_host(b)
         if self._wimg_dirty:
             self._weight_images()        # outside the captured graph: only needed after the parameters changed
+        if layout is not None:
+            self._score_buffers(b, layout)
         if not self.use_graphs or self.prof is not None:
-            return self.forward(b, training=False, replan=replan)
-        g = b.graphs.get(key)
-        if g is None:
-            self.forward(b, training=False, replan=replan)
-            torch.cuda.synchronize()
-            g = torch.cuda.CUDAGraph()
-            n0 = self.launches
-            with torch.cuda.graph(g):
-                self.forward(b, training=False, replan=replan)
-            g.n_launches = self.launches - n0
-            b.graphs[key] = g
-            self.graph_captures += 1
+            self._infer_body(b, replan, layout)
         else:
-            self.launches += g.n_launches
-        g.replay()
+            g = b.graphs.get(key)
+            if g is None:
+                self._infer_body(b, replan, layout)
+                torch.cuda.synchronize()
+                g = torch.cuda.CUDAGraph()
+                n0 = self.launches
+                with torch.cuda.graph(g):
+                    self._infer_body(b, replan, layout)
+                g.n_launches = self.launches - n0
+                b.graphs[key] = g
+                self.graph_captures += 1
+            else:
+                self.launches += g.n_launches
+            g.replay()
         ws = self._workspace(b, False)
-        return ws["y"], ws["ga"]
+        if layout is None:
+            return ws["y"], ws["ga"]
+        return ws["y"], ws["ga"], b.scores[layout]
+
+    def _infer_body(self, b: Batch, replan: bool, layout: Optional[str]) -> None:
+        self.forward(b, training=False, attn=b.attn if layout is not None else None, replan=replan)
+        if layout is not None:
+            self._unpack_scores(b, layout)
+
+    def _score_buffers(self, b: Batch, layout: str) -> None:
+        """The shape class's buffers of the local-attention scores (allocated when first requested)."""
+        L, dev = self.spec.n_attention, self.device
+        if b.attn is None:
+            b.attn = torch.empty(L, b.rows, 8, dtype=torch.float32, device=dev)
+        if layout not in b.scores:
+            shape = (L, b.B, 8, b.M, b.N) if layout == "padded" else (L, 8, b.rows)
+            b.scores[layout] = torch.empty(shape, dtype=torch.float32, device=dev)
+
+    def _unpack_scores(self, b: Batch, layout: str) -> None:
+        """Plan-ordered scores (b.attn) -> b.scores[layout], one launch for all layers."""
+        L, st = self.spec.n_attention, self._stream()
+        self._ev("attn_unpack", True)
+        if layout == "padded":
+            check(lib.scann_attn_to_padded(_p(b.attn), L, b.rows, _p(b.cnt), _p(b.rowptr), _p(b.nmask), b.B, b.M, b.N,
+                                           _p(b.scores[layout]), st), "attn_to_padded")
+        else:
+            check(lib.scann_attn_to_csr(_p(b.attn), L, b.rows, _p(b.valid_rows), _p(b.nvalid), b.rows,
+                                        _p(b.scores[layout]), st), "attn_to_csr")
+        self._ev("attn_unpack", False)
+        self.launches += 1
+
+
+def score_layout(local_attention) -> Optional[str]:
+    """``local_attention`` argument of ``Engine.predict_step`` -> None, "padded" or "csr"."""
+    if isinstance(local_attention, str):
+        if local_attention not in ("padded", "csr"):
+            raise ValueError(f"local_attention must be a bool, 'padded' or 'csr', not {local_attention!r}")
+        return local_attention
+    if not isinstance(local_attention, (bool, np.bool_)):
+        raise TypeError(f"local_attention must be a bool, 'padded' or 'csr', not {type(local_attention).__name__}")
+    return "padded" if local_attention else None

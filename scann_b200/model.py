@@ -11,7 +11,7 @@ from __future__ import annotations
 import functools
 import math
 import os
-from typing import Dict, Iterable, Optional
+from typing import Dict, Iterable, NamedTuple, Optional
 
 import numpy as np
 import torch
@@ -67,6 +67,43 @@ def _structure_chunks(n_atoms, batch_size: int):
     if c0 < len(n_atoms):
         out.append((c0, len(n_atoms)))
     return out
+
+
+class LocalAttentionScores(NamedTuple):
+    """Local-attention scores of one structure (``predict_structures(..., local_attention=True)``).  Pairs
+    ``site_offsets[i]:site_offsets[i + 1]`` are the kept neighbours of site i in the order of
+    ``compute_voronoi_neighbor``'s list for that site: site ``neighbors[p]`` at ``distances[p]`` (so periodic images of
+    one site stay apart).  ``scores[l, h, p]`` is the weight of pair p in head h of local-attention layer l."""
+    site_offsets: np.ndarray        # int32 [n + 1]
+    neighbors: np.ndarray           # int32 [P_s]
+    distances: np.ndarray           # float32 [P_s]
+    scores: np.ndarray              # float32 [n_attention, num_head, P_s]
+
+
+def split_pair_scores(struct_atom_off, atom_nbr_off, nbr_idx, nbr_d, scores):
+    """The [L, 8, P] scores of one CSR batch (``Engine.predict_step(..., local_attention="csr")``, trimmed to its P
+    pairs) and the batch's CSR arrays -> one ``LocalAttentionScores`` per structure."""
+    sa = np.asarray(struct_atom_off, np.int64)
+    an = np.asarray(atom_nbr_off, np.int64)
+    scores = np.asarray(scores, np.float32)
+    if sa.ndim != 1 or len(sa) < 1 or an.ndim != 1 or len(an) != sa[-1] - sa[0] + 1:
+        raise ValueError("struct_atom_off [B+1] and atom_nbr_off [A+1] do not describe one CSR batch")
+    P = int(an[-1] - an[0])
+    if scores.ndim != 3 or scores.shape[2] != P or len(nbr_idx) < P or len(nbr_d) < P:
+        raise ValueError(f"scores {scores.shape}, {len(nbr_idx)} neighbours and {len(nbr_d)} distances for {P} pairs")
+    idx, d = np.asarray(nbr_idx, np.int32), np.asarray(nbr_d, np.float32)
+    a = (sa - sa[0]).tolist()
+    p = (an[sa - sa[0]] - an[0]).tolist()
+    off = (an - an[0]).astype(np.int32)
+    # views into the batch's arrays (one allocation per structure: its site offsets)
+    return [LocalAttentionScores(off[a[s]:a[s + 1] + 1] - off[a[s]], idx[p[s]:p[s + 1]], d[p[s]:p[s + 1]],
+                                 scores[:, :, p[s]:p[s + 1]]) for s in range(len(a) - 1)]
+
+
+def _check_flag(name: str, value) -> bool:
+    if not isinstance(value, (bool, np.bool_)):
+        raise TypeError(f"{name} must be a bool, not {type(value).__name__}")
+    return bool(value)
 
 
 def _batch_errors(y, y_true) -> Dict[str, float]:
@@ -191,27 +228,40 @@ class ScannKerasModel:
         self.dropout = True
 
     # ---- inference -------------------------------------------------------------------------
-    def predict(self, inputs: Dict[str, object], batch_size: Optional[int] = None, verbose: int = 0):
+    def predict(self, inputs: Dict[str, object], batch_size: Optional[int] = None, verbose: int = 0,
+                local_attention: bool = False):
         """Keras ``Model.predict``: numpy in, numpy out.  Keras would split the batch into
-        sub-batches of 32; structures are independent so one pass gives identical results."""
+        sub-batches of 32; structures are independent so one pass gives identical results.
+
+        ``local_attention=True`` appends the local-attention scores of every layer, one float32 array
+        [n_attention, B, num_head, M, N]: ``[y, ga, la]`` in infer mode, ``[y, la]`` otherwise.  Element l is what the
+        reference's layer ``local_attention[_l]`` returns as ``output[0]`` (the softmax over each atom's neighbour
+        slots, scann/layers/attention.py:186-189): masked slots are 0 and an atom without valid neighbours has 1/N in
+        every slot.  The other outputs are those of the plain call."""
+        scores = _check_flag("local_attention", local_attention)
         eng = self.engine
         # a ragged CSR batch (DataIterator.csr_item) is expanded to the padded layout on the device
         b = eng.load_batch_csr(inputs, plan=False) if "struct_atom_off" in inputs else eng.load_batch(inputs, plan=False)
-        y, ga = eng.predict_step(b, replan=True)
+        y, ga, *la = eng.predict_step(b, replan=True, local_attention=scores)
         y_h = y.cpu().numpy().reshape(b.B, 1)          # synchronises the stream
         eng.check_status()
         self.last_e2e_bytes = (b.h2d_bytes, y.numel() * 4)
+        out = [y_h]
         if self.infer:
             ga_h = ga.cpu().numpy().reshape(b.B, b.M, 1)
             self.last_e2e_bytes = (self.last_e2e_bytes[0], self.last_e2e_bytes[1] + ga.numel() * 4)
-            return [y_h, ga_h]
-        return y_h
+            out.append(ga_h)
+        if scores:
+            out.append(la[0].cpu().numpy())
+            self.last_e2e_bytes = (self.last_e2e_bytes[0], self.last_e2e_bytes[1] + la[0].numel() * 4)
+        return out if len(out) > 1 else y_h
 
     def __call__(self, inputs, training: bool = False):
         return self.predict(inputs)
 
     def predict_structures(self, structs, d_t: float = 4.0, w_t: float = 0.4, angle: Optional[bool] = None,
-                           batch_size: int = 128, cutoff: float = 13.0, allow_pathological: bool = False):
+                           batch_size: int = 128, cutoff: float = 13.0, allow_pathological: bool = False,
+                           local_attention: bool = False):
         """Structures in, ``[target [S, 1], ga_score]`` out: the README flow (``compute_voronoi_neighbor`` ->
         ``prepare_input_pmt`` -> ``predict``) for many structures, with the neighbour lists selected and batched on
         the device (``voronoi.select_neighbors``).  ``ga_score`` is a list of S float32 arrays, one value per atom,
@@ -228,8 +278,14 @@ class ScannKerasModel:
 
         Refused: ring-feature models (the ring / aromatic flags come from openbabel, not from the geometry) and
         ``feature='cgcnn'`` models -- use ``predict`` on ``DataIterator`` batches for those -- and structures with
-        more than 1000 atoms (1000 is the reference's neighbour padding marker)."""
+        more than 1000 atoms (1000 is the reference's neighbour padding marker).
+
+        ``local_attention=True`` returns ``[target, ga_score, la]``: ``la`` holds one ``LocalAttentionScores`` per
+        structure, in input order -- every kept (site, neighbour) pair with its score in each head of each
+        local-attention layer.  The scores of the padding are not copied back.  ``target`` and ``ga_score`` are those
+        of the plain call."""
         from . import voronoi as V
+        scores = _check_flag("local_attention", local_attention)
         spec = self.spec
         if spec.use_ring:
             raise NotImplementedError("predict_structures: use_ring models need the ring / aromatic flags of openbabel, "
@@ -252,7 +308,7 @@ class ScannKerasModel:
         column = bool(spec.g_update) if angle is None else bool(angle)
         eng = self.engine
         y_out = np.zeros((len(structs), 1), np.float32)
-        ga_out = []
+        ga_out, la_out = [], []
         for c0, c1 in _structure_chunks([len(X) for X in checked[1]], batch_size):
             sel = V.select_neighbors(structs[c0:c1], d_t, w_t, column, cutoff, allow_pathological, first_index=c0,
                                      _checked=(checked[0][c0:c1], checked[1][c0:c1]))
@@ -261,12 +317,16 @@ class ScannKerasModel:
                 csr = sel.csr(s0, s1)
                 M, N = shape_class(csr["M"], csr["N"])
                 b = eng.load_batch_device_csr(csr, M=M, N=N, plan=False)
-                y, ga = eng.predict_step(b, replan=True)
+                y, ga, *la = eng.predict_step(b, replan=True, local_attention="csr" if scores else False)
                 y_out[c0 + s0:c0 + s1, 0] = y.cpu().numpy()           # synchronises the stream
                 ga_h = ga.cpu().numpy().reshape(b.B, b.M)
                 ga_out.extend(ga_h[i, :n].copy() for i, n in enumerate(csr["n_atoms"]))
+                if scores:
+                    # the batch's pairs only, and its lists from the CSR blob on the device
+                    la_out.extend(split_pair_scores(*(csr[k].cpu().numpy() for k in (
+                        "struct_atom_off", "atom_nbr_off", "nbr_idx", "nbr_d")), la[0][:, :, :csr["P"]].cpu().numpy()))
         eng.check_status()
-        return [y_out, ga_out]
+        return [y_out, ga_out, la_out] if scores else [y_out, ga_out]
 
     # ---- training --------------------------------------------------------------------------
     def compile(self, loss=None, optimizer=None, metrics=None, learning_rate=None):
@@ -550,17 +610,19 @@ class SCANN:
         return out * self.std + self.mean
 
     def _predict_structures(self, structs, d_t: float = 4.0, w_t: float = 0.4, angle: Optional[bool] = None,
-                            batch_size: int = 128, cutoff: float = 13.0, allow_pathological: bool = False):
+                            batch_size: int = 128, cutoff: float = 13.0, allow_pathological: bool = False,
+                            local_attention: bool = False):
         """``ScannKerasModel.predict_structures`` with the target scaled back like ``predict_data``."""
-        y, ga = self.model.predict_structures(structs, d_t=d_t, w_t=w_t, angle=angle, batch_size=batch_size,
-                                              cutoff=cutoff, allow_pathological=allow_pathological)
-        return y * self.std + self.mean, ga
+        y, *rest = self.model.predict_structures(structs, d_t=d_t, w_t=w_t, angle=angle, batch_size=batch_size,
+                                                 cutoff=cutoff, allow_pathological=allow_pathological,
+                                                 local_attention=local_attention)
+        return (y * self.std + self.mean, *rest)
 
     @property
     def predict_structures(self):
         """``predict_structures(structs, d_t=4.0, w_t=0.4, angle=None, batch_size=128, cutoff=13.0,
-        allow_pathological=False)``: ``ScannKerasModel.predict_structures`` with the target scaled back like
-        ``predict_data``.  (A property, not a plain method: the record of SCANN's plain public methods in
+        allow_pathological=False, local_attention=False)``: ``ScannKerasModel.predict_structures`` with the target
+        scaled back like ``predict_data``.  (A property, not a plain method: the record of SCANN's plain public methods in
         tests/golden/reference/graph_public_surface.npz stays the surface that was compared with the reference's SCANN,
         which has no such method.)"""
         return functools.partial(SCANN._predict_structures, self)
