@@ -344,7 +344,9 @@ int scann_la_wpart_reduce(const float* wpart, const int32_t* ntiles, int grid, i
  * over that many rows; rows < 0: per-pair problem over the tile-padded pair rows (ntiles * tile_stride rows, rows
  * with pair_c < 0 skipped; or, when the plan's compact list valid_rows / nvalid is given, exactly the valid rows),
  * with X rows multiplied by xg[pair_j[row]] when xg != NULL.  db (nullable) += column
- * sums of Y (bias gradient).  `problems` is a DEVICE array; results are accumulated with atomics. */
+ * sums of Y (bias gradient).  `problems` is a DEVICE array; results are accumulated with atomics.
+ * scann_wgrad_batch_max_problems(): the most problems one launch takes (1 <= nprob <= it); a longer list is cut into
+ * several launches. */
 typedef struct ScannWgradProblem {
     const float* X;
     const float* Y;
@@ -358,6 +360,7 @@ typedef struct ScannWgradProblem {
 int scann_wgrad_batch_tc(int grid, const ScannWgradProblem* problems, int nprob, const int32_t* ntiles, int tile_stride,
                          const int32_t* pair_c, const int32_t* pair_j, const int32_t* valid_rows, const int32_t* valid_j,
                          const int32_t* nvalid, void* stream);
+int scann_wgrad_batch_max_problems(void);
 
 /* ---- global attention + property head ---------------------------------------------------------
  * GlobalAttention.call (scann/layers/attention.py:267-318) + bf_property / predict_property / mrelu

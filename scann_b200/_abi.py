@@ -59,6 +59,7 @@ PROTOTYPES = {
     "scann_la_backward_pipe": (ci, [ci, C.c_longlong, ci] + [vp] * 14 + [ci] + [vp] * 8 + [vp, ci, vp, vp]),
     "scann_la_wgrad_tc": (ci, [ci, ci] + [vp] * 9 + [vp]),
     "scann_wgrad_batch_tc": (ci, [ci, vp, ci, vp, ci, vp, vp, vp, vp, vp, vp]),
+    "scann_wgrad_batch_max_problems": (ci, []),
     "scann_la_wpart_reduce": (ci, [vp, vp, ci, ci, vp, vp, vp]),
     "scann_ga_head_forward": (ci, [vp, vp, ci, ci, ci, vp, vp, vp, vp, ci, vp, vp, vp, vp, vp]),
     "scann_ga_head_backward": (ci, [vp, vp, ci, ci, ci, vp, vp, vp, vp, vp, vp, vp, vp, vp]),

@@ -400,7 +400,7 @@ static int wgrad_batch_launch(int grid, const void* problems_dev, int nprob, con
                               const int32_t* pair_c, const int32_t* pair_j, const int32_t* valid_rows,
                               const int32_t* valid_j, const int32_t* nvalid, float* slots, float* bslots, void* stream) {
     if (nprob < 1 || nprob > WG_MAX_PROBLEMS) { scann_set_error("wgrad_batch_tc: nprob must be in 1..%d", WG_MAX_PROBLEMS); return 1; }
-    if (tile_stride != 32 && tile_stride != 64 && tile_stride != 128) { scann_set_error("wgrad_batch_tc: tile_stride must be 64 or 128"); return 1; }
+    if (tile_stride != 32 && tile_stride != 64 && tile_stride != 128) { scann_set_error("wgrad_batch_tc: tile_stride must be 32, 64 or 128"); return 1; }
     static bool configured = false;
     if (!configured) {
         cudaError_t e = cudaFuncSetAttribute(wgrad_batch_tc_kernel<DET>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WG_SMEM);
@@ -434,6 +434,10 @@ extern "C" int scann_wgrad_batch_tc_det(int grid, const void* problems_dev, int 
     return wgrad_batch_launch<true>(grid, problems_dev, nprob, ntiles, tile_stride, pair_c, pair_j, valid_rows, valid_j,
                                     nvalid, slots, bslots, stream);
 }
+
+// Longest problem table one scann_wgrad_batch_tc / _det / reduce launch takes (the table is staged in shared memory);
+// a longer one is cut into several launches.
+extern "C" int scann_wgrad_batch_max_problems(void) { return WG_MAX_PROBLEMS; }
 
 extern "C" int scann_wgrad_batch_reduce(int grid, const void* problems_dev, int nprob, const int32_t* ntiles, int tile_stride,
                                         const int32_t* valid_rows, const int32_t* nvalid, const float* slots,

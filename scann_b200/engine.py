@@ -1463,29 +1463,32 @@ class Engine:
                   [self.gw(fg, 0), self.gw(fg, 2 * D * D), self.gw(f"{la}/query/kernel")],
                   [self.gw(f"{la}/filter_geo/bias"), 0, self.gw(f"{la}/query/bias")])
         if batched and "wgrad" not in self._skip:
-            table, count = self._wgrad_table(b, ws)
             self._pdl(False)
             self._ev("wgrad_batch", True)
-            if self.deterministic:
-                check(lib.scann_wgrad_batch_tc_det(self.la_grid, _p(table), count, _p(b.ntiles), b.stride, _p(b.pair_c),
-                                                   _p(b.pair_j), _p(b.valid_rows), _p(b.valid_j), _p(b.nvalid),
-                                                   _p(ws["wg_slots"]), _p(ws["wg_bslots"]), st), "wgrad_batch_tc_det")
-                check(lib.scann_wgrad_batch_reduce(self.la_grid, _p(table), count, _p(b.ntiles), b.stride,
-                                                   _p(b.valid_rows), _p(b.nvalid), _p(ws["wg_slots"]),
-                                                   _p(ws["wg_bslots"]), st), "wgrad_batch_reduce")
+            # deterministic mode: each launch's reduce has read the slots before the next launch (same stream) rewrites them
+            for table, count in self._wgrad_table(b, ws):
+                if self.deterministic:
+                    check(lib.scann_wgrad_batch_tc_det(self.la_grid, table, count, _p(b.ntiles), b.stride, _p(b.pair_c),
+                                                       _p(b.pair_j), _p(b.valid_rows), _p(b.valid_j), _p(b.nvalid),
+                                                       _p(ws["wg_slots"]), _p(ws["wg_bslots"]), st), "wgrad_batch_tc_det")
+                    check(lib.scann_wgrad_batch_reduce(self.la_grid, table, count, _p(b.ntiles), b.stride,
+                                                       _p(b.valid_rows), _p(b.nvalid), _p(ws["wg_slots"]),
+                                                       _p(ws["wg_bslots"]), st), "wgrad_batch_reduce")
+                    self.launches += 1
+                else:
+                    check(lib.scann_wgrad_batch_tc(self.la_grid, table, count, _p(b.ntiles), b.stride, _p(b.pair_c),
+                                                   _p(b.pair_j), _p(b.valid_rows), _p(b.valid_j), _p(b.nvalid), st),
+                          "wgrad_batch_tc")
                 self.launches += 1
-            else:
-                check(lib.scann_wgrad_batch_tc(self.la_grid, _p(table), count, _p(b.ntiles), b.stride, _p(b.pair_c),
-                                               _p(b.pair_j), _p(b.valid_rows), _p(b.valid_j), _p(b.nvalid), st),
-                      "wgrad_batch_tc")
             self._ev("wgrad_batch", False)
-            self.launches += 1
         self._backward_tail(b, ws, dg_up, side, main)
 
     def _wgrad_table(self, b: Batch, ws: dict):
-        """Device table of all dW += X^T Y problems of a train step (pointers into this workspace)."""
-        if "wg_table" in ws:
-            return ws["wg_table"], ws["wg_count"]
+        """Device table of all dW += X^T Y problems of a train step (pointers into this workspace), as the
+        (device address, problem count) of each launch: 4 + 7 L problems for SCANN+ with attention normalisation, at most
+        scann_wgrad_batch_max_problems() per launch (one launch up to 13 layers)."""
+        if "wg_launches" in ws:
+            return ws["wg_launches"]
         sp = self.spec
         L, R = sp.n_attention, b.R
         probs = []
@@ -1523,8 +1526,9 @@ class Engine:
         arr = (WgradProblem * len(probs))(*probs)
         host = torch.frombuffer(bytearray(bytes(arr)), dtype=torch.uint8)
         ws["wg_table"] = host.to(self.device)
-        ws["wg_count"] = len(probs)
-        return ws["wg_table"], ws["wg_count"]
+        step, size = lib.scann_wgrad_batch_max_problems(), ctypes.sizeof(WgradProblem)
+        ws["wg_launches"] = [(_p(ws["wg_table"], i * size), min(step, len(probs) - i)) for i in range(0, len(probs), step)]
+        return ws["wg_launches"]
 
     def _backward_prep(self, ws: dict, stream: int) -> None:
         """Work the backward needs that does not depend on the forward: transposed weight blocks and

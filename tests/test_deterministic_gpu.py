@@ -32,6 +32,9 @@ REPRO = {
     # 16 384 atom rows: more than one wave of the warp-specialised chained kernel, so the round-1 chained kernel runs
     "ptgp_b64_l2_round1_chain": ("ptgp", "ptgp", 64, 2, NOUP, False, "atomic"),
     "cgcnn_ring_b16_l2": ("qm9", "qm9", 16, 2, {"use_ring": True}, False, "cgcnn"),
+    # deeper than one weight-gradient launch holds (4 + 7 L problems): two launches, each with its own reduce
+    "qm9_b4_l14": ("qm9", "qm9", 4, 14, {}, False, "atomic"),
+    "qm9_b4_l20": ("qm9", "qm9", 4, 20, {}, False, "atomic"),
 }
 
 
@@ -201,14 +204,16 @@ def test_golden_cases_keep_their_accuracy(name):
 
 
 # the full-configuration cases of test_gpu_parity.py that the deterministic mode trains
-FULL = {"qm9_b128_l7": ("qm9", "qm9", 128, {}), "ptgp_b16_l11": ("ptgp", "ptgp", 16, NOUP)}
+FULL = {"qm9_b128_l7": ("qm9", "qm9", 128, {}), "ptgp_b16_l11": ("ptgp", "ptgp", 16, NOUP),
+        "qm9_b352_l2": ("qm9", "qm9", 352, {"n_attention": 2}), "ptgp_b64_l2": ("ptgp", "ptgp", 64, dict(NOUP, n_attention=2))}
 
 
 @pytest.mark.parametrize("name", list(FULL))
 def test_full_configuration_keeps_its_accuracy(name):
     """Full depth: outputs, ga_score, loss and every per-tensor gradient against the fp64 oracle, with the bounds
     test_full_configuration_parity_against_oracle applies to the default engine."""
-    from tests.test_gpu_parity import TOL_GRAD as PTOL, TOL_OUT, rel
+    from scann_b200._abi import lib
+    from tests.test_gpu_parity import ROUND1_CHAIN, TOL_GRAD as PTOL, TOL_OUT, rel
     cfg_name, shape, B, over = FULL[name]
     cfg = get_config(cfg_name)
     cfg["model"].update(over)
@@ -217,6 +222,8 @@ def test_full_configuration_keeps_its_accuracy(name):
     arena = lay.randomize_arena(21)
     ring = bool(spec.use_ring)
     inputs, target = make_batch(shape, 13, B=B, use_ring=ring)
+    if name in ROUND1_CHAIN:
+        assert B * inputs["atomic"].shape[1] > lib.scann_dense_chain2_max_rows()
     w = lay.to_dict(arena)
     l2n = [e.name for e in lay if e.l2]
     kw = _oracle_kwargs(spec)

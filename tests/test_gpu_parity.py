@@ -255,7 +255,13 @@ FULL_CASES = {
     # 16 of the 64 structures of the bench batch (256 atoms each, all 11 layers) keep the fp64 oracle's autograd
     # tape within a few GB
     "ptgp_b16_l11": ("ptgp", "ptgp", 16, {"g_update": False, "gaussian_d": 4.0}),
+    # more atom rows than one wave of the warp-specialised chained kernel covers (scann_dense_chain2_max_rows: 9 472 on a
+    # 148-SM B200), so every chained Dense launch runs on the round-1 kernel: SCANN+ at 352 x 29 = 10 208 rows, and
+    # bench.py's PtGP batch (64 x 256 = 16 384 rows) at two layers
+    "qm9_b352_l2": ("qm9", "qm9", 352, {"n_attention": 2}),
+    "ptgp_b64_l2": ("ptgp", "ptgp", 64, {"g_update": False, "gaussian_d": 4.0, "n_attention": 2}),
 }
+ROUND1_CHAIN = ("qm9_b352_l2", "ptgp_b64_l2")
 
 
 @pytest.mark.parametrize("name", list(FULL_CASES))
@@ -274,6 +280,8 @@ def test_full_configuration_parity_against_oracle(name):
     l2n = [e.name for e in lay if e.l2]
     loss, y_ref, ga_ref, grads = O.loss_and_grads(w, inputs, target, l2n, **kw)
     eng, b, y, ga = run_forward(spec, arena, inputs)
+    if name in ROUND1_CHAIN:
+        assert b.R > eng.chain2_max_rows
     # At full depth and batch the reference's OWN fp32 arithmetic (the fp32 oracle: same graph, same op order) is not
     # within 1e-5 of fp64 on the worst of the B*M ga scores: the synthetic QM9 batch holds structures whose global
     # attention scores nearly cancel (ga error of the fp32 oracle 8.0e-6, fullerene without ga normalisation 1.7e-4).
@@ -959,15 +967,28 @@ def test_weight_images_are_bit_exact():
         assert np.array_equal(got[b].view(np.uint32), _weight_image_reference(W).view(np.uint32))
 
 
-@pytest.mark.parametrize("R", [100, 3712, 5000, 10000])
+# row counts of the chained kernels, resolved on the device (chain_rows): one row, a ragged 32-row tile, one wave of
+# 32-row tiles and one row more (64-row tiles), one wave of 64-row tiles (scann_dense_chain2_max_rows) and one row more
+# (where the engine switches to the round-1 chained kernel), two waves and a ragged tile
+CHAIN_ROWS = ["1", "31", "33", "32sms", "32sms+1", "max", "max+1", "2max+5"]
+
+
+def chain_rows(name):
+    from scann_b200 import _abi
+    _abi.require_gpu()
+    sms, mx = _abi.lib.scann_device_sm_count(), _abi.lib.scann_dense_chain2_max_rows()
+    named = {"32sms": 32 * sms, "32sms+1": 32 * sms + 1, "max": mx, "max+1": mx + 1, "2max+5": 2 * mx + 5}
+    return named[name] if name in named else int(name)
+
+
+@pytest.mark.parametrize("R", [100, 3712, 5000, 10000] + CHAIN_ROWS)
 def test_chain2_matches_round1_chain_and_reference(R):
     """scann_dense_chain2 (warp-specialised, weight images) against scann_dense_chain and an fp64 restatement on a
     ResidualNorm-like step list (attention.py:25-40 + the next layer's projections): 32-row tiles (R <= 32 x SMs), 64-row
     tiles, several waves, a ragged last tile."""
     import ctypes
-    from scann_b200 import _abi
     from scann_b200._abi import ChainStep, chain_step, check, lib
-    _abi.require_gpu()
+    R = chain_rows(R)
     rng = np.random.default_rng(R)
     D = 128
     Ws = [(rng.standard_normal((D, D)) / np.sqrt(D)).astype(np.float32) for _ in range(4)]
