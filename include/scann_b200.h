@@ -132,6 +132,15 @@ int scann_cgcnn_embed_backward(const float* atomic92, const float* emb_rows, con
                                const float* Wr, const float* br, const float* We, const float* t0, const float* dx0,
                                float* d_cat_ws, float* dWemb, float* dbemb, float* dWr, float* dbr, float* dWe, float* dbe,
                                const void* drop_ctl, void* stream);
+/* feature == "cgcnn" on batches that carry atomic numbers (scann_model.py:364-365): embed_atom's output for an atom
+ * is row Z of emb_table = table @ W + b ([Z_rows, E]: scann_cgcnn_embed_forward with R = Z_rows over the per-element
+ * table [Z_rows, 92], then scann_embed_forward with emb = emb_table, n_atoms = Z_rows, emb_rows = NULL), so no
+ * per-atom feature vector is built.  Backward: scann_embed_backward(_det) with emb = emb_table, n_atoms = Z_rows and
+ * d_emb = a ZEROED [Z_rows, E] buffer leaves the per-element gradient there; this call ACCUMULATES
+ * dW[f, k] += sum_z table[z, f] d_emb[z, k] and db[k] += sum_z d_emb[z, k] (one thread per output, z ascending:
+ * deterministic).  Refused: F != 92, E outside 1..128, Z_rows < 1. */
+int scann_cgcnn_table_backward(const float* table, const float* d_emb, int Z_rows, int F, int E, float* dW, float* db,
+                               void* stream);
 /* Gradients are ACCUMULATED into d_emb, dWr, dbr, dWe, dbe.  G_ws: (n_atoms+3)*128 floats. */
 int scann_embed_backward(const int32_t* atomic, const float* ring, int R, int E, int n_atoms, const float* emb,
                          const float* Wr, const float* br, const float* We, const float* t0, const float* dx0,

@@ -33,6 +33,7 @@ PROTOTYPES = {
     "scann_embed_forward": (ci, [vp, vp, ci, ci, ci] + [vp] * 7 + [vp, vp, vp, vp]),
     "scann_cgcnn_embed_forward": (ci, [vp, vp, vp, ci, ci, ci, vp, vp]),
     "scann_cgcnn_embed_backward": (ci, [vp, vp, vp, ci, ci, ci] + [vp] * 12 + [vp, vp]),
+    "scann_cgcnn_table_backward": (ci, [vp, vp, ci, ci, ci, vp, vp, vp]),
     "scann_embed_backward": (ci, [vp, vp, ci, ci, ci] + [vp] * 12 + [vp, vp]),
     "scann_geom_init_forward": (ci, [vp, ci, ci] + [vp] * 10 + [vp]),
     "scann_geom_init_backward": (ci, [vp, ci, ci] + [vp] * 14 + [vp]),

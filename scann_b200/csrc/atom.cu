@@ -305,6 +305,23 @@ __global__ void __launch_bounds__(128) embed_bwd_cols_kernel(const float* __rest
         if (c < 2) dWr[c * 10 + k] += acc; else dbr[k] += acc;
     }
 }
+// Batches that carry atomic numbers: embed_atom's output for an atom is row Z of emb_table = table @ W + b, so its
+// gradients are dW[f, k] += sum_z table[z, f] d_emb[z, k] and db[k] += sum_z d_emb[z, k], with d_emb the per-element
+// sums of embed_bwd_final_kernel.  grid = F + 1 CTAs (the last one: db), thread k; z ascending (deterministic).
+__global__ void __launch_bounds__(128) cgcnn_table_bwd_kernel(const float* __restrict__ table,
+                                                              const float* __restrict__ d_emb, int Z, int F, int E,
+                                                              float* __restrict__ dW, float* __restrict__ db) {
+    const int k = threadIdx.x, f = blockIdx.x;
+    if (k >= E) return;
+    float acc = 0.f;
+    if (f < F) {
+        for (int z = 0; z < Z; ++z) acc = fmaf(table[(size_t)z * F + f], d_emb[(size_t)z * E + k], acc);
+        dW[(size_t)f * E + k] += acc;
+    } else {
+        for (int z = 0; z < Z; ++z) acc += d_emb[(size_t)z * E + k];
+        db[k] += acc;
+    }
+}
 
 // ---------------------------------------------------------------------------------------------
 // Geometry initialisation (g_update): g0 = swish(rbf_d Wd + bd) * swish(rbf_w Ww + bw)
@@ -980,6 +997,19 @@ extern "C" int scann_cgcnn_embed_backward_det(const float* atomic92, const float
                                                              (float*)nullptr, (const ScannDropCtl*)drop_ctl);
     embed_bwd_cols_kernel<<<F + 1 + (ring ? 3 : 0), 128, 0, st>>>(atomic92, ring, R, F, E, d_cat_ws, dWemb, dbemb, dWr, dbr);
     return scann_check_launch("scann_cgcnn_embed_backward_det");
+}
+
+// embed_atom's gradients from the per-element gradient d_emb [Z_rows, E] of emb_table = table @ W + b, ACCUMULATED
+// into dW [F, E] and db [E].  One thread per output element, z ascending: the same bits in both training modes.
+extern "C" int scann_cgcnn_table_backward(const float* table, const float* d_emb, int Z_rows, int F, int E, float* dW,
+                                          float* db, void* stream) {
+    if (F != 92 || E < 1 || E > 128 || Z_rows < 1) {
+        scann_set_error("cgcnn_table_backward: bad sizes Z_rows=%d F=%d E=%d (F must be 92, E in 1..128, Z_rows >= 1)",
+                        Z_rows, F, E);
+        return 1;
+    }
+    cgcnn_table_bwd_kernel<<<F + 1, 128, 0, (cudaStream_t)stream>>>(table, d_emb, Z_rows, F, E, dW, db);
+    return scann_check_launch("scann_cgcnn_table_backward");
 }
 
 extern "C" int scann_geom_init_forward(const int32_t* ntiles, int grid, int tile_stride, const int32_t* pair_c, const float* pair_d,

@@ -31,18 +31,54 @@ def set_atomic_features(table) -> np.ndarray:
     number, keys are strings, key "0" is the padding atom).  ``table``: such a dict, or an array ``[Z + 1, 92]``.
     The table itself is data of the CGCNN project and is not shipped with this package."""
     global ATOMIC_FEATURES
+    arr = _table_array(table)
+    if arr.ndim != 2:
+        raise ValueError("atomic feature table must be [Z + 1, features]")
+    ATOMIC_FEATURES = arr
+    return arr
+
+
+def _table_array(table) -> np.ndarray:
+    """A feature table given as CGCNN's ``atom_init.json`` dict (string keys) or as an array -> float32 array."""
     if isinstance(table, dict):
         zmax = max(int(k) for k in table)
         width = len(next(iter(table.values())))
         arr = np.zeros((zmax + 1, width), np.float32)
         for k, v in table.items():
             arr[int(k)] = np.asarray(v, np.float32)
+        return arr
+    return np.ascontiguousarray(table, np.float32)
+
+
+def check_atomic_features(table) -> np.ndarray:
+    """The per-element feature table of a ``feature='cgcnn'`` model as the device routes read it: a 2-D float32 array
+    (or an ``atom_init.json`` dict) with exactly 92 columns, finite, and at least row 0 (padded atoms read row 0, as
+    ``DataIterator`` gives them ``ATOMIC_FEATURES[0]``).  Returns it as a C-contiguous float32 array."""
+    if isinstance(table, dict):
+        arr = _table_array(table)
     else:
-        arr = np.ascontiguousarray(table, np.float32)
-    if arr.ndim != 2:
-        raise ValueError("atomic feature table must be [Z + 1, features]")
-    ATOMIC_FEATURES = arr
+        arr = np.asarray(table)
+        if arr.dtype != np.float32:
+            raise ValueError(f"atomic_features must be float32, not {arr.dtype}")
+        arr = np.ascontiguousarray(arr)
+    if arr.ndim != 2 or arr.shape[1] != 92 or arr.shape[0] < 1:
+        raise ValueError(f"atomic_features must be [Z + 1, 92] (row 0: the padding atom), not {list(arr.shape)}")
+    if not np.isfinite(arr).all():
+        r = int(np.flatnonzero(~np.isfinite(arr).all(1))[0])
+        raise ValueError(f"atomic_features: row {r} holds a value that is not finite")
     return arr
+
+
+def check_table_rows(z, atom_off, rows: int) -> None:
+    """Every atomic number of a data set (``z`` flat, structure s = atoms ``atom_off[s]:atom_off[s + 1]``) has a row in
+    a feature table of ``rows`` rows; else ValueError naming the first structure that does not."""
+    z = np.asarray(z)
+    bad = (z < 0) | (z >= rows)
+    if bad.any():
+        a = int(np.argmax(bad))
+        s = int(np.searchsorted(np.asarray(atom_off), a, side="right")) - 1
+        raise ValueError(f"structure {s}: atomic number {int(z[a])} has no row in the atomic feature table "
+                         f"({rows} rows, atomic numbers 0..{rows - 1})")
 
 
 def load_atomic_features(path: str) -> np.ndarray:
@@ -63,6 +99,8 @@ class DataIterator:
             raise NotImplementedError("feature='cgcnn' needs the per-element feature table: pass atomic_features= or call "
                                       "scann_b200.datagenerator.load_atomic_features(<atom_init.json>)")
         self.batch_size, self.shuffle, self.use_ring, self.feature = batch_size, shuffle, use_ring, feature
+        # the table the cgcnn batches of this iterator are built with (DeviceDataIterator.from_data_iterator takes it)
+        self.atomic_features = ATOMIC_FEATURES if feature == "cgcnn" else None
         self.weight_index = 2 if g_update else 3                       # datagenerator.py:48-50
         self.converter = 1000 if converter else 1.0                    # :54-57
         S = len(data_energy)
@@ -124,10 +162,11 @@ _INT32_MAX = 0x7fffffff
 _DEVICE_ARRAYS = ("struct_atom_off", "atom_nbr_off", "z", "nbr_idx", "nbr_w", "nbr_d", "ring", "target")
 
 
-def _refuse_structures_route(who: str, use_ring: bool, feature: str) -> None:
-    if feature == "cgcnn":
-        raise NotImplementedError(f"{who}: feature='cgcnn' batches carry per-atom feature vectors; train from "
-                                  "DataIterator(..., feature='cgcnn') (padded batches)")
+def _refuse_structures_route(who: str, use_ring: bool, feature: str, atomic_features=None) -> None:
+    if feature == "cgcnn" and atomic_features is None:
+        raise NotImplementedError(f"{who}: feature='cgcnn' needs the per-element feature table the model embeds atoms "
+                                  "with: pass atomic_features=<[Z + 1, 92] float32 array> (for from_data_iterator: "
+                                  "build the DataIterator with atomic_features=)")
     if use_ring:
         raise NotImplementedError(f"{who}: use_ring models need the ring / aromatic flags of openbabel, which the "
                                   "geometry does not give; build a DataIterator(..., use_ring=True) from the "
@@ -157,18 +196,28 @@ class DeviceDataIterator:
     ``DataIterator`` (copied back from the device) for any other consumer.
 
     Build it with ``from_data_iterator`` (the reference's ``.npy`` flow) or ``from_structures`` (Voronoi neighbour
-    lists selected on the device; nothing per site reaches the host).  ``feature='cgcnn'`` is not supported."""
+    lists selected on the device; nothing per site reaches the host).
+
+    ``feature='cgcnn'``: the iterator carries the per-element feature table ``atomic_features`` ([Z + 1, 92] float32)
+    on the host; the device arrays keep the atomic numbers, and the model embeds them through that table
+    (``Engine.set_atomic_features``), so no per-atom feature vector is built.  ``__getitem__`` returns the feature
+    vectors ``atomic_features[Z]`` as ``DataIterator.__getitem__`` does."""
 
     def __init__(self, arrays: Dict[str, object], energy: np.ndarray, atom_off: np.ndarray, pair_off: np.ndarray,
                  nmax: np.ndarray, npairs: np.ndarray, batch_size: int = 32, shuffle: bool = False,
-                 use_ring: bool = False, weight_index: int = 3, converter: float = 1.0, indexes=None):
+                 use_ring: bool = False, weight_index: int = 3, converter: float = 1.0, indexes=None,
+                 feature: str = "atomic", atomic_features=None):
         """Low-level constructor.  ``arrays``: device tensors ``struct_atom_off`` [S+1] / ``atom_nbr_off`` [A+1] (int32,
         from 0), ``z`` [A], ``nbr_idx`` / ``nbr_w`` / ``nbr_d`` [P], ``ring`` [A, 2] int32 or None, ``target`` [S]
         float32.  Host: ``energy`` [S] float32 (the targets), ``atom_off`` / ``pair_off`` [S+1] int64 (first atom /
         pair of each structure), ``nmax`` [S] (longest neighbour list, 1000 entries included) and ``npairs`` [S]
         (entries other than 1000).  ``indexes``: the current epoch order (default: a first ``on_epoch_end``, as
-        ``DataIterator`` does)."""
-        self.batch_size, self.shuffle, self.use_ring, self.feature = batch_size, shuffle, use_ring, "atomic"
+        ``DataIterator`` does).  ``feature='cgcnn'`` needs ``atomic_features`` (``check_atomic_features``)."""
+        if feature not in ("atomic", "cgcnn"):
+            raise ValueError(f"feature must be 'atomic' or 'cgcnn', got {feature!r}")
+        _refuse_structures_route("DeviceDataIterator", False, feature, atomic_features)
+        self.batch_size, self.shuffle, self.use_ring, self.feature = batch_size, shuffle, use_ring, feature
+        self.atomic_features = check_atomic_features(atomic_features) if feature == "cgcnn" else None
         self.weight_index, self.converter = weight_index, converter
         for k in _DEVICE_ARRAYS:
             setattr(self, k, arrays.get(k))
@@ -185,11 +234,17 @@ class DeviceDataIterator:
     # ------------------------------------------------------------------ constructors
     @classmethod
     def from_data_iterator(cls, it: "DataIterator", device=None) -> "DeviceDataIterator":
-        """Upload a host ``DataIterator``'s flat arrays once and take over its settings and its current order."""
-        _refuse_structures_route("DeviceDataIterator", False, getattr(it, "feature", "atomic"))
+        """Upload a host ``DataIterator``'s flat arrays once and take over its settings and its current order (and, for
+        ``feature='cgcnn'``, the feature table it was built with)."""
+        feature = getattr(it, "feature", "atomic")
+        table = getattr(it, "atomic_features", None) if feature == "cgcnn" else None
+        _refuse_structures_route("DeviceDataIterator.from_data_iterator", False, feature, table)
         atom_off = np.asarray(it.atom_off, np.int64)
         nbr_off = np.asarray(it.nbr_off, np.int64)
         _check_int32_offsets(atom_off, nbr_off[atom_off])
+        if table is not None:
+            table = check_atomic_features(table)
+            check_table_rows(it.z, atom_off, len(table))
         pair_off, nmax, npairs = cls.host_sizes(atom_off, nbr_off, it.nbr_idx)
         from . import _abi
         import torch
@@ -203,7 +258,8 @@ class DeviceDataIterator:
                   "nbr_d": up(it.nbr_d, np.float32), "target": up(it.energy, np.float32),
                   "ring": up(it.ring, np.int32) if it.use_ring else None}
         return cls(arrays, it.energy, atom_off, pair_off, nmax, npairs, batch_size=it.batch_size, shuffle=it.shuffle,
-                   use_ring=it.use_ring, weight_index=it.weight_index, converter=it.converter, indexes=it.indexes)
+                   use_ring=it.use_ring, weight_index=it.weight_index, converter=it.converter, indexes=it.indexes,
+                   feature=feature, atomic_features=table)
 
     @staticmethod
     def host_sizes(atom_off, nbr_off, nbr_idx):
@@ -223,19 +279,23 @@ class DeviceDataIterator:
     def from_structures(cls, structs, targets, batch_size: int = 32, shuffle: bool = False, g_update: bool = True,
                         d_t: float = 4.0, w_t: float = 0.4, angle=None, cutoff: float = 13.0,
                         allow_pathological: bool = False, converter: bool = False, use_ring: bool = False,
-                        feature: str = "atomic", device=None) -> "DeviceDataIterator":
+                        feature: str = "atomic", atomic_features=None, device=None) -> "DeviceDataIterator":
         """The iterator ``DataIterator(data_energy, compute_voronoi_neighbors(structs, d_t, w_t), ...)`` would be, with
         the neighbour lists selected and flattened on the device (``voronoi.select_neighbors``, in the chunks of
         ``predict_structures``): no facet record and no neighbour list reaches the host.  ``targets``: one value per
         structure.  ``angle``: the weight column (True = solid angle, False = normalised); None picks the one
         ``DataIterator`` trains a model with this ``g_update`` on.  ``d_t`` / ``w_t`` / ``cutoff`` /
-        ``allow_pathological``: as in ``compute_voronoi_neighbors``.
+        ``allow_pathological``: as in ``compute_voronoi_neighbors``.  ``feature='cgcnn'`` needs ``atomic_features``, the
+        model's per-element feature table ([Z + 1, 92] float32).
 
-        Refused: ``use_ring`` and ``feature='cgcnn'`` (``NotImplementedError``); structures without sites or with more
-        than 1000 (1000 is the reference's neighbour padding marker) (``ValueError``, naming the structure)."""
+        Refused: ``use_ring``, and ``feature='cgcnn'`` without ``atomic_features`` (``NotImplementedError``); structures
+        without sites, with more than 1000 (1000 is the reference's neighbour padding marker) or, for ``feature='cgcnn'``,
+        with an atomic number that has no row in the table (``ValueError``, naming the structure)."""
         from . import voronoi as V
         from .model import MAX_STRUCTURE_ATOMS, _structure_chunks
-        _refuse_structures_route("DeviceDataIterator.from_structures", use_ring, feature)
+        _refuse_structures_route("DeviceDataIterator.from_structures", use_ring, feature, atomic_features)
+        if feature == "cgcnn":
+            atomic_features = check_atomic_features(atomic_features)
         structs = list(structs)
         targets = list(np.asarray(targets, dtype=object).reshape(-1))
         if len(targets) != len(structs):
@@ -254,6 +314,9 @@ class DeviceDataIterator:
         atom_off = np.zeros(len(structs) + 1, np.int64)
         np.cumsum(n_atoms, out=atom_off[1:])
         _check_int32_offsets(atom_off)
+        if feature == "cgcnn":
+            check_table_rows(np.concatenate([np.asarray(s.atomic_numbers).reshape(-1) for s in structs]), atom_off,
+                             len(atomic_features))
         conv = 1000 if converter else 1.0
         energy = np.array([float(t) * conv for t in targets], "float32")
         column = bool(g_update) if angle is None else bool(angle)
@@ -291,7 +354,8 @@ class DeviceDataIterator:
                   "nbr_idx": cat(0, torch.int32), "nbr_w": cat(1, torch.float32), "nbr_d": cat(2, torch.float32),
                   "target": torch.from_numpy(energy).to(dev), "ring": None}
         return cls(arrays, energy, atom_off, pair_off, np.concatenate(nmax), npairs, batch_size=batch_size,
-                   shuffle=shuffle, use_ring=False, weight_index=2 if column else 3, converter=conv)
+                   shuffle=shuffle, use_ring=False, weight_index=2 if column else 3, converter=conv, feature=feature,
+                   atomic_features=atomic_features)
 
     # ------------------------------------------------------------------ Sequence protocol
     def on_epoch_end(self):
@@ -352,7 +416,15 @@ class DeviceDataIterator:
         return csr, self.energy[sel]
 
     def __getitem__(self, idx: int):
-        """``DataIterator.__getitem__``: the padded batch, gathered by ``scann_gather_batch`` and copied back."""
+        """``DataIterator.__getitem__``: the padded batch, gathered by ``scann_gather_batch`` and copied back (for
+        ``feature='cgcnn'`` with the atomic numbers replaced by their feature vectors, as ``DataIterator`` does)."""
+        inputs, target = self._gathered_item(idx)
+        if self.feature == "cgcnn":
+            inputs["atomic"] = self.atomic_features[inputs["atomic"]]
+        return inputs, target
+
+    def _gathered_item(self, idx: int):
+        """The padded batch with atomic numbers, gathered on the device and copied back."""
         import torch
         from ._abi import check, lib
         start, B, M, N, _ = self.batch_shape(idx)

@@ -23,6 +23,7 @@ from .params import ParamLayout, layer_name
 
 TILE = 128
 PLAN_GSZ = 128
+TABLE_ROUTE = "atomic_features"     # last item of the graph keys of cgcnn batches embedded through the table
 D = 128
 L2_COEF = 1e-4
 
@@ -56,6 +57,9 @@ class Batch:
         self.tile_cap = 0
         self.P_host = None          # number of valid pairs when known on the host
         self.A_host = None
+        # feature='cgcnn' only: TABLE_ROUTE when the batch carries atomic numbers (CSR / gathered batches, embedded
+        # through the engine's per-element table), None when it carries the padded feature vectors (load_batch)
+        self.route = None
 
 
 class Engine:
@@ -182,6 +186,47 @@ class Engine:
         # every weight-gradient GEMM of the step in one persistent launch at the end of the backward pass
         self.use_wgrad_batch = os.environ.get("SCANN_WGRAD_BATCH", "1") == "1" and self.use_chain and self.tc_la_bwd
         self._nccl_warned = False
+        # feature='cgcnn': per-element feature table [Z_rows, 92] on the device (set_atomic_features), its host copy and
+        # the buffers of the table route: emb_table / d_emb [Z_rows, E], G [Z_rows + 3, 128]
+        self.atomic_features: Optional[torch.Tensor] = None
+        self._afeat_host: Optional[np.ndarray] = None
+        self._tab: Dict[str, torch.Tensor] = {}
+
+    # ------------------------------------------------------------------ feature='cgcnn' on atomic numbers
+    def set_atomic_features(self, table) -> None:
+        """The per-element feature table ([Z_rows, 92] float32, row 0 = padding atom) a ``feature='cgcnn'`` model embeds
+        batches that carry atomic numbers with (``load_batch_csr``, ``load_batch_device_csr``, ``load_batch_gather``):
+        embed_atom's output for an atom is row Z of ``table @ W + b``, computed once per forward.  A table of the same
+        shape is copied into the same device buffer in stream order (captured graphs stay valid); one with another row
+        count replaces the buffer and drops the captured graphs of that route."""
+        from .datagenerator import check_atomic_features
+        if self.spec.feature != "cgcnn":
+            raise ValueError("set_atomic_features: only feature='cgcnn' models read a per-element feature table")
+        t = check_atomic_features(table)
+        old = self._afeat_host
+        if old is not None and old.shape == t.shape:
+            if not np.array_equal(old.view(np.uint32), t.view(np.uint32)):
+                self.atomic_features.copy_(torch.from_numpy(t))
+                self._afeat_host = t.copy()
+            return
+        Z, E, dev = t.shape[0], self.spec.embedding_dim, self.device
+        self.atomic_features = torch.from_numpy(t).to(dev)
+        self._afeat_host = t.copy()
+        f = dict(dtype=torch.float32, device=dev)
+        self._tab = {"emb": torch.empty(Z, E, **f), "d_emb": torch.empty(Z, E, **f), "G": torch.empty(Z + 3, D, **f)}
+        for b in self._batches.values():
+            for k in [k for k in b.graphs if k[-1] == TABLE_ROUTE]:
+                del b.graphs[k]
+
+    def _table_route(self) -> Optional[str]:
+        """Route of a batch that arrives as atomic numbers: TABLE_ROUTE for a cgcnn model (which then needs the table)."""
+        if self.spec.feature != "cgcnn":
+            return None
+        if self.atomic_features is None:
+            raise ValueError("this feature='cgcnn' model got a batch of atomic numbers (CSR or device-gathered) before "
+                             "its per-element feature table: call Engine.set_atomic_features(table) or pass "
+                             "atomic_features= to the call that built the batches")
+        return TABLE_ROUTE
 
     # ------------------------------------------------------------------ deterministic mode
     def _check_deterministic_support(self) -> None:
@@ -294,6 +339,7 @@ class Engine:
         b = self._get_batch(B, M, N, P_host)
         b.P_host = P_host
         b.h2d_bytes = 0
+        b.route = None
         dev = self.device
         key = (B, M, N, b.tile_cap, b.tile_rows, b.stride)
 
@@ -407,12 +453,14 @@ class Engine:
         """Stage one RAGGED batch (``DataIterator.csr_item`` of scann_b200/datagenerator.py): the CSR arrays travel
         in one host->device copy (valid atoms / pairs only) and ``scann_pack_batch`` expands them into the padded
         device buffers -- the device form of the reference's DataIterator.__getitem__."""
+        route = self._table_route()
         sa, an = csr["struct_atom_off"], csr["atom_nbr_off"]
         B, M, N = len(sa) - 1, int(csr["M"]), int(csr["N"])
         idx = np.asarray(csr["nbr_idx"], np.int32)
         P_host = int(np.count_nonzero(idx != 1000))
         b = self._get_batch(B, M, N, P_host)
         b.P_host = P_host
+        b.route = route
         segs = [("sa", np.asarray(sa, np.int32)), ("an", np.asarray(an, np.int32)), ("z", np.asarray(csr["z"], np.int32)),
                 ("idx", idx), ("w", np.asarray(csr["nbr_w"], np.float32)), ("d", np.asarray(csr["nbr_d"], np.float32))]
         if self.spec.use_ring:
@@ -463,6 +511,7 @@ class Engine:
         blob ``csr["blob"]`` with the byte offsets ``csr["offsets"]`` (keys sa, an, z, idx, w, d) and the host sizes
         ``B`` / ``M`` / ``N`` / ``P``.  ``M`` / ``N`` may be raised above the batch's own (shape classes); the padding
         is masked.  Nothing crosses to or from the host."""
+        route = self._table_route()
         B, P = int(csr["B"]), int(csr["P"])
         M = int(csr["M"]) if M is None else int(M)
         N = int(csr["N"]) if N is None else int(N)
@@ -471,6 +520,7 @@ class Engine:
         b = self._get_batch(B, M, N, P)
         b.P_host = P
         b.h2d_bytes = 0
+        b.route = route
         self._pack_csr(b, csr["blob"], csr["offsets"])
         if plan:
             self._plan(b)
@@ -482,6 +532,7 @@ class Engine:
         ``(B, M, N, P)`` -- the exact sizes of the batch, so that it shares the class and the captured graphs of the
         same structures loaded by ``load_batch_csr``.  The targets go to ``b.target``.  Nothing crosses to or from the
         host."""
+        route = self._table_route()
         B, M, N, P = int(B), int(M), int(N), int(P)
         if B <= 0 or M <= 0 or N <= 0:
             raise ValueError(f"gather_batch: bad shape B={B} M={M} N={N}")
@@ -491,6 +542,7 @@ class Engine:
         b = self._get_batch(B, M, N, P)
         b.P_host = P
         b.h2d_bytes = 0
+        b.route = route
         b.host_dirty = False            # the pinned mirror is stale: it must not be copied over what is gathered here
         use_ring = self.spec.use_ring
         if use_ring and data.ring is None:
@@ -757,16 +809,22 @@ class Engine:
             add(gs, 2 * gi, N_RBF * D, gslot, self.gw("neighbor_w/kernel"), N_RBF * D)
             add(gs, 2 * gi, D, gslot, self.gw("neighbor_d/bias"), 2 * N_RBF * D)
             add(gs, 2 * gi, D, gslot, self.gw("neighbor_w/bias"), 2 * N_RBF * D + D)
+        i_cg = len(ents)
         if sp.feature == "cgcnn":
             cs = ws["cg_slots"]
             add(cs, cs.shape[0], kin * D, (kin + 1) * D, self.gw("dense_embed/kernel"))
             add(cs, cs.shape[0], D, (kin + 1) * D, self.gw("dense_embed/bias"), kin * D)
         add(ws["head_slots"], b.B, D, D, self.gw("predict_property/kernel"))
         add(ws["head_bslots"], b.B, 1, 1, self.gw("predict_property/bias"))
-        arr = (_abi.SlotSum * len(ents))(*ents)
-        ws["slot_table"] = torch.frombuffer(bytearray(bytes(arr)), dtype=torch.uint8).to(dev)
-        ws["slot_count"] = len(ents)
+
+        def table(es):
+            arr = (_abi.SlotSum * len(es))(*es)
+            return torch.frombuffer(bytearray(bytes(arr)), dtype=torch.uint8).to(dev), len(es)
+        ws["slot_table"], ws["slot_count"] = table(ents)
         ws["slot_max"] = max(e.count for e in ents)
+        if sp.feature == "cgcnn":
+            # table route: dense_embed's gradients come out of the embedding backward itself, cg_slots are not written
+            ws["slot_table_" + TABLE_ROUTE], ws["slot_count_" + TABLE_ROUTE] = table(ents[:i_cg] + ents[i_cg + 2:])
 
     def _ln_grads(self, ws: dict, l: int, which: int, name: str) -> dict:
         """dgamma / dbeta of a LayerNorm-backward chain step: the gradient arena, or the slot arrays of the deterministic
@@ -833,6 +891,20 @@ class Engine:
         R, E = b.R, sp.embedding_dim
         ring = sp.use_ring
         cg = sp.feature == "cgcnn"
+        if b.route == TABLE_ROUTE:
+            # embed_atom over the per-element table once (emb_table = table @ W + b), then the lookup of row Z: the
+            # arithmetic of each row is that of the padded route's per-atom rows, bit for bit
+            Z, emb = self.atomic_features.shape[0], self._tab["emb"]
+            check(lib.scann_cgcnn_embed_forward(_p(self.atomic_features), self.w("embed_atom/kernel"),
+                                                self.w("embed_atom/bias"), Z, 92, E, _p(emb), st), "cgcnn_embed_forward")
+            self.launches += 1
+            check(lib.scann_embed_forward(_p(b.atomic), _p(b.ring) if ring else 0, R, E, Z, _p(emb),
+                                          self.w("extra_embed/kernel") if ring else 0, self.w("extra_embed/bias") if ring else 0,
+                                          self.w("dense_embed/kernel"), self.w("dense_embed/bias"),
+                                          _p(ws["t0"]) if training else 0, _p(ws["x"][0]), _p(self.status),
+                                          _p(self.adam_scalars, 8) if training else 0, 0, st), "embed_forward")
+            self.launches += 1
+            return
         if cg:
             if "emb_rows" not in ws:
                 ws["emb_rows"] = torch.empty(R, E, dtype=torch.float32, device=self.device)
@@ -1287,7 +1359,7 @@ class Engine:
                                                    self.gw("neighbor_w/bias"), gst), "geom_init_backward")
         E = sp.embedding_dim
         ring = sp.use_ring
-        if sp.feature == "cgcnn":
+        if sp.feature == "cgcnn" and b.route != TABLE_ROUTE:
             # deterministic mode: dense_embed's gradients go to per-CTA slots (scann_slot_reduce)
             dense = (_p(ws["cg_slots"]),) if self.deterministic else \
                 (self.gw("dense_embed/kernel"), self.gw("dense_embed/bias"))
@@ -1303,15 +1375,34 @@ class Engine:
                 ev.record(side)
                 main.wait_event(ev)
             return
-        Gslots = (_p(ws["emb_slots"]),) if self.deterministic else ()
+        if b.route == TABLE_ROUTE:
+            # the per-element gradient of emb_table lands in the zeroed d_emb, then goes through the table into
+            # embed_atom's kernel / bias (scann_cgcnn_table_backward)
+            tab = self._tab
+            n_emb, emb, G, d_emb = self.atomic_features.shape[0], _p(tab["emb"]), tab["G"], _p(tab["d_emb"])
+            tab["d_emb"].zero_()
+            if self.deterministic:
+                ns = lib.scann_embed_backward_det_slots(R)
+                if ws.get("emb_slots_table") is None or ws["emb_slots_table"].shape[:2] != (ns, n_emb + 3):
+                    ws["emb_slots_table"] = torch.empty(ns, n_emb + 3, D, dtype=torch.float32, device=self.device)
+                Gslots = (_p(ws["emb_slots_table"]),)
+            else:
+                Gslots = ()
+        else:
+            n_emb, emb, G, d_emb = sp.n_atoms, self.w("embed_atom/embeddings"), ws["G"], self.gw("embed_atom/embeddings")
+            Gslots = (_p(ws["emb_slots"]),) if self.deterministic else ()
         check((lib.scann_embed_backward_det if self.deterministic else lib.scann_embed_backward)(
-            _p(b.atomic), _p(b.ring) if ring else 0, R, E, sp.n_atoms, self.w("embed_atom/embeddings"),
+            _p(b.atomic), _p(b.ring) if ring else 0, R, E, n_emb, emb,
             self.w("extra_embed/kernel") if ring else 0, self.w("extra_embed/bias") if ring else 0,
-            self.w("dense_embed/kernel"), _p(ws["t0"]), _p(dx), _p(ws["G"]), *Gslots,
-            self.gw("embed_atom/embeddings"), self.gw("extra_embed/kernel") if ring else 0,
+            self.w("dense_embed/kernel"), _p(ws["t0"]), _p(dx), _p(G), *Gslots,
+            d_emb, self.gw("extra_embed/kernel") if ring else 0,
             self.gw("extra_embed/bias") if ring else 0, self.gw("dense_embed/kernel"), self.gw("dense_embed/bias"),
             _p(self.adam_scalars, 8), st), "embed_backward")
         self.launches += 4
+        if b.route == TABLE_ROUTE:
+            check(lib.scann_cgcnn_table_backward(_p(self.atomic_features), d_emb, n_emb, 92, E, self.gw("embed_atom/kernel"),
+                                                 self.gw("embed_atom/bias"), st), "cgcnn_table_backward")
+            self.launches += 1
         if side is not main:             # join: the optimiser needs every weight gradient
             ev = torch.cuda.Event()
             ev.record(side)
@@ -1596,6 +1687,8 @@ class Engine:
         self._set_adam(lr, batch_global or b.B)
         self._flush_host(b)
         key = ("train", replan, apply, want_grads, allreduce is not None)
+        if b.route:
+            key += (b.route,)
         if not self.use_graphs or self.prof is not None:
             self._train_body(b, allreduce, apply, want_grads, replan)
         else:
@@ -1651,8 +1744,9 @@ class Engine:
         n = self.layout.total
         if self.deterministic:
             self._pdl(False)
-            check(lib.scann_slot_reduce(_p(ws["slot_table"]), ws["slot_count"], ws["slot_max"], self._stream()),
-                  "slot_reduce")
+            sfx = "_" + b.route if b.route else ""
+            check(lib.scann_slot_reduce(_p(ws["slot_table" + sfx]), ws["slot_count" + sfx], ws["slot_max"],
+                                        self._stream()), "slot_reduce")
             self.launches += 1
         if p2p is not None:
             if self.deterministic:
@@ -1695,6 +1789,8 @@ class Engine:
         of the class overwrites them."""
         layout = score_layout(local_attention)
         key = ("infer", replan) if layout is None else ("infer", replan, layout)
+        if b.route:
+            key += (b.route,)
         self._flush_host(b)
         if self._wimg_dirty:
             self._weight_images()        # outside the captured graph: only needed after the parameters changed

@@ -261,7 +261,7 @@ class ScannKerasModel:
 
     def predict_structures(self, structs, d_t: float = 4.0, w_t: float = 0.4, angle: Optional[bool] = None,
                            batch_size: int = 128, cutoff: float = 13.0, allow_pathological: bool = False,
-                           local_attention: bool = False):
+                           local_attention: bool = False, atomic_features=None):
         """Structures in, ``[target [S, 1], ga_score]`` out: the README flow (``compute_voronoi_neighbor`` ->
         ``prepare_input_pmt`` -> ``predict``) for many structures, with the neighbour lists selected and batched on
         the device (``voronoi.select_neighbors``).  ``ga_score`` is a list of S float32 arrays, one value per atom,
@@ -276,9 +276,15 @@ class ScannKerasModel:
         multiple of 4 up to 32, then of 8), so that structures of different sizes replay a handful of CUDA graphs
         instead of capturing one per batch.  The padding is masked and trimmed from the outputs.
 
-        Refused: ring-feature models (the ring / aromatic flags come from openbabel, not from the geometry) and
-        ``feature='cgcnn'`` models -- use ``predict`` on ``DataIterator`` batches for those -- and structures with
-        more than 1000 atoms (1000 is the reference's neighbour padding marker).
+        ``feature='cgcnn'`` models need ``atomic_features``, the per-element feature table they were trained with
+        ([Z + 1, 92] float32, CGCNN's ``atom_init.json`` as an array or dict): the model embeds the atomic numbers
+        through it on the device (``Engine.set_atomic_features``), with the outputs of ``predict`` on the padded
+        ``DataIterator(..., feature='cgcnn', atomic_features=...)`` batches of the same structures.
+
+        Refused: ring-feature models (the ring / aromatic flags come from openbabel, not from the geometry) -- use
+        ``predict`` on ``DataIterator`` batches for those --, ``feature='cgcnn'`` models without ``atomic_features``
+        (``NotImplementedError``), and structures with more than 1000 atoms (1000 is the reference's neighbour padding
+        marker) or, for ``feature='cgcnn'``, with an atomic number the table has no row for (``ValueError``).
 
         ``local_attention=True`` returns ``[target, ga_score, la]``: ``la`` holds one ``LocalAttentionScores`` per
         structure, in input order -- every kept (site, neighbour) pair with its score in each head of each
@@ -291,9 +297,13 @@ class ScannKerasModel:
             raise NotImplementedError("predict_structures: use_ring models need the ring / aromatic flags of openbabel, "
                                       "which the geometry does not give; build the batches with DataIterator(..., "
                                       "use_ring=True) and call predict")
-        if spec.feature == "cgcnn":
-            raise NotImplementedError("predict_structures: feature='cgcnn' batches carry per-atom feature vectors; build "
-                                      "them with DataIterator(..., feature='cgcnn') and call predict")
+        if spec.feature == "cgcnn" and atomic_features is None:
+            raise NotImplementedError("predict_structures: a feature='cgcnn' model embeds atoms through the per-element "
+                                      "feature table it was trained with: pass atomic_features=<[Z + 1, 92] float32 "
+                                      "array>")
+        if spec.feature != "cgcnn" and atomic_features is not None:
+            raise ValueError("predict_structures: atomic_features is the table of feature='cgcnn' models; this model "
+                             "embeds atomic numbers")
         structs = list(structs)
         checked = V._arrays(structs)
         for k, X in enumerate(checked[1]):
@@ -307,6 +317,13 @@ class ScannKerasModel:
             raise ValueError("batch_size must be >= 1")
         column = bool(spec.g_update) if angle is None else bool(angle)
         eng = self.engine
+        if atomic_features is not None:
+            from .datagenerator import check_atomic_features, check_table_rows
+            table = check_atomic_features(atomic_features)
+            n_at = np.array([len(X) for X in checked[1]], np.int64)
+            check_table_rows(np.concatenate([np.asarray(s.atomic_numbers).reshape(-1) for s in structs]),
+                             np.concatenate([[0], np.cumsum(n_at)]), len(table))
+            eng.set_atomic_features(table)
         y_out = np.zeros((len(structs), 1), np.float32)
         ga_out, la_out = [], []
         for c0, c1 in _structure_chunks([len(X) for X in checked[1]], batch_size):
@@ -381,10 +398,16 @@ class ScannKerasModel:
         y = self.predict(inputs)
         return _batch_errors(y[0] if isinstance(y, list) else y, y_true)
 
+    def _use_table_of(self, data) -> None:
+        """A feature='cgcnn' model on a ``DeviceDataIterator``: embed through the iterator's feature table."""
+        if self.spec.feature == "cgcnn" and getattr(data, "atomic_features", None) is not None:
+            self.engine.set_atomic_features(data.atomic_features)
+
     def predict_device_batch(self, data, idx: int):
         """Predictions of batch ``idx`` of a ``DeviceDataIterator``, gathered on the device: ``(y [B, 1], targets
         [B])`` as host float32 arrays -- the same values ``predict(data[idx][0])`` gives."""
         eng = self.engine
+        self._use_table_of(data)
         b = eng.load_batch_gather(data, *data.batch_shape(idx), plan=False)
         y, _ = eng.predict_step(b, replan=True)
         y_h = y.cpu().numpy().reshape(b.B, 1)          # synchronises the stream
@@ -420,6 +443,8 @@ class ScannKerasModel:
                     maes.append(float(pin[2]))
 
             eng = self.engine
+            if on_device:
+                self._use_table_of(x)
             eng.overlap_h2d = True
             try:
                 for i in range(len(x)):
@@ -611,17 +636,17 @@ class SCANN:
 
     def _predict_structures(self, structs, d_t: float = 4.0, w_t: float = 0.4, angle: Optional[bool] = None,
                             batch_size: int = 128, cutoff: float = 13.0, allow_pathological: bool = False,
-                            local_attention: bool = False):
+                            local_attention: bool = False, atomic_features=None):
         """``ScannKerasModel.predict_structures`` with the target scaled back like ``predict_data``."""
         y, *rest = self.model.predict_structures(structs, d_t=d_t, w_t=w_t, angle=angle, batch_size=batch_size,
                                                  cutoff=cutoff, allow_pathological=allow_pathological,
-                                                 local_attention=local_attention)
+                                                 local_attention=local_attention, atomic_features=atomic_features)
         return (y * self.std + self.mean, *rest)
 
     @property
     def predict_structures(self):
         """``predict_structures(structs, d_t=4.0, w_t=0.4, angle=None, batch_size=128, cutoff=13.0,
-        allow_pathological=False, local_attention=False)``: ``ScannKerasModel.predict_structures`` with the target
+        allow_pathological=False, local_attention=False, atomic_features=None)``: ``ScannKerasModel.predict_structures`` with the target
         scaled back like ``predict_data``.  (A property, not a plain method: the record of SCANN's plain public methods in
         tests/golden/reference/graph_public_surface.npz stays the surface that was compared with the reference's SCANN,
         which has no such method.)"""
@@ -680,11 +705,11 @@ class SCANN:
                                                          for ix in (train, valid, test)]
         return train, valid, test
 
-    def _prepare_structures(self, structs, targets, split: bool = True, **voronoi_args):
+    def _prepare_structures(self, structs, targets, split: bool = True, atomic_features=None, **voronoi_args):
         """``SCANN.prepare_structures``: see the property."""
         from .datagenerator import DeviceDataIterator, _refuse_structures_route
         hy, cm = self.config["hyper"], self.config["model"]
-        _refuse_structures_route("SCANN.prepare_structures", cm["use_ring"], cm["feature"])
+        _refuse_structures_route("SCANN.prepare_structures", cm["use_ring"], cm["feature"], atomic_features)
         structs = list(structs)
         targets = list(np.asarray(targets, dtype=object).reshape(-1))
         if len(targets) != len(structs):
@@ -698,19 +723,22 @@ class SCANN:
             return DeviceDataIterator.from_structures([structs[k] for k in ix], rows[list(ix), 1],
                                                       batch_size=hy["batch_size"], shuffle=shuffle,
                                                       g_update=cm["g_update"], use_ring=cm["use_ring"],
-                                                      feature=cm["feature"], **voronoi_args)
+                                                      feature=cm["feature"],
+                                                      atomic_features=atomic_features if cm["feature"] == "cgcnn" else None,
+                                                      **voronoi_args)
 
         return self._attach_iterators(len(structs), iterator, split)
 
     @property
     def prepare_structures(self):
-        """``prepare_structures(structs, targets, split=True, **voronoi_args)``: ``prepare_dataset`` for structures
-        and their targets instead of the reference's data files.  The same target scaling (``hyper.scaler``), config
-        entries and split of the global numpy generator; ``trainIter`` / ``validIter`` / ``testIter`` (or ``dataIter``)
-        are ``DeviceDataIterator.from_structures`` (``voronoi_args``: ``d_t``, ``w_t``, ``angle``, ``cutoff``,
-        ``allow_pathological``, ``converter``), so training and evaluation gather their batches on the device.
-        Refused for ``use_ring`` and ``feature='cgcnn'`` models.  (A property for the same reason as
-        ``predict_structures``.)"""
+        """``prepare_structures(structs, targets, split=True, atomic_features=None, **voronoi_args)``: ``prepare_dataset``
+        for structures and their targets instead of the reference's data files.  The same target scaling
+        (``hyper.scaler``), config entries and split of the global numpy generator; ``trainIter`` / ``validIter`` /
+        ``testIter`` (or ``dataIter``) are ``DeviceDataIterator.from_structures`` (``voronoi_args``: ``d_t``, ``w_t``,
+        ``angle``, ``cutoff``, ``allow_pathological``, ``converter``), so training and evaluation gather their batches on
+        the device.  ``feature='cgcnn'`` models need ``atomic_features``, their per-element feature table ([Z + 1, 92]
+        float32).  Refused for ``use_ring`` models and for ``feature='cgcnn'`` without ``atomic_features``.  (A property
+        for the same reason as ``predict_structures``.)"""
         return functools.partial(SCANN._prepare_structures, self)
 
     def create_callbacks(self):
