@@ -81,6 +81,37 @@ def check_table_rows(z, atom_off, rows: int) -> None:
                          f"({rows} rows, atomic numbers 0..{rows - 1})")
 
 
+def check_ring_aromatic(ring_aromatic, n_atoms) -> np.ndarray:
+    """The ring / aromatic flags of a ``use_ring`` model's structures as the device routes read them: one ``[n_k, 2]``
+    array of integers per structure, in order (the third item of a reference ``data_energy`` row, or openbabel's ring
+    and aromaticity perception run by the caller), ``n_atoms[k]`` = n_k sites.  The values must fit in int32, the type
+    ``DataIterator`` keeps them in.  Returns them concatenated as one C-contiguous int32 array ``[sum(n_k), 2]``;
+    else ValueError naming the first structure (its index in ``n_atoms``) whose flags do not fit."""
+    n_atoms = [int(n) for n in n_atoms]
+    try:
+        flags = list(ring_aromatic)
+    except TypeError:
+        raise ValueError("ring_aromatic must be a sequence of [n_sites, 2] integer arrays, one per structure") from None
+    if len(flags) != len(n_atoms):
+        raise ValueError(f"{len(n_atoms)} structures but {len(flags)} ring_aromatic arrays")
+    out = np.zeros((sum(n_atoms), 2), np.int32)
+    a0 = 0
+    for k, (f, n) in enumerate(zip(flags, n_atoms)):
+        arr = np.asarray(f)
+        if arr.shape != (n, 2):
+            raise ValueError(f"structure {k}: ring_aromatic must be [{n}, 2] (one row per site), not {list(arr.shape)}")
+        if arr.dtype.kind == "f":
+            if not (np.isfinite(arr).all() and (arr == np.round(arr)).all()):
+                raise ValueError(f"structure {k}: ring_aromatic holds a value that is not an integer")
+        elif arr.dtype.kind not in "biu":
+            raise ValueError(f"structure {k}: ring_aromatic must hold integers, not {arr.dtype}")
+        if arr.size and (arr.min() < -_INT32_MAX - 1 or arr.max() > _INT32_MAX):
+            raise ValueError(f"structure {k}: ring_aromatic holds a value outside int32")
+        out[a0:a0 + n] = arr
+        a0 += n
+    return out
+
+
 def load_atomic_features(path: str) -> np.ndarray:
     """``set_atomic_features`` from a JSON file in CGCNN's ``atom_init.json`` format ({"1": [...], "2": [...], ...})."""
     import json
@@ -162,15 +193,23 @@ _INT32_MAX = 0x7fffffff
 _DEVICE_ARRAYS = ("struct_atom_off", "atom_nbr_off", "z", "nbr_idx", "nbr_w", "nbr_d", "ring", "target")
 
 
-def _refuse_structures_route(who: str, use_ring: bool, feature: str, atomic_features=None) -> None:
+def _refuse_structures_route(who: str, use_ring: bool, feature: str, atomic_features=None,
+                             ring_aromatic=None) -> None:
     if feature == "cgcnn" and atomic_features is None:
         raise NotImplementedError(f"{who}: feature='cgcnn' needs the per-element feature table the model embeds atoms "
                                   "with: pass atomic_features=<[Z + 1, 92] float32 array> (for from_data_iterator: "
                                   "build the DataIterator with atomic_features=)")
-    if use_ring:
-        raise NotImplementedError(f"{who}: use_ring models need the ring / aromatic flags of openbabel, which the "
-                                  "geometry does not give; build a DataIterator(..., use_ring=True) from the "
-                                  "reference's data files and convert it with DeviceDataIterator.from_data_iterator")
+    _refuse_ring_route(who, use_ring, ring_aromatic)
+
+
+def _refuse_ring_route(who: str, use_ring: bool, ring_aromatic) -> None:
+    if use_ring and ring_aromatic is None:
+        raise NotImplementedError(f"{who}: use_ring models read the ring / aromatic flags of openbabel, which the "
+                                  "geometry does not give: pass ring_aromatic=<one [n_sites, 2] integer array per "
+                                  "structure> (the third item of the reference's data_energy rows, or openbabel's ring "
+                                  "and aromaticity perception run on the structures)")
+    if not use_ring and ring_aromatic is not None:
+        raise ValueError(f"{who}: ring_aromatic is read by use_ring models only; this one has use_ring=False")
 
 
 def _check_int32_offsets(atom_off: np.ndarray, pair_off: Optional[np.ndarray] = None) -> None:
@@ -279,21 +318,26 @@ class DeviceDataIterator:
     def from_structures(cls, structs, targets, batch_size: int = 32, shuffle: bool = False, g_update: bool = True,
                         d_t: float = 4.0, w_t: float = 0.4, angle=None, cutoff: float = 13.0,
                         allow_pathological: bool = False, converter: bool = False, use_ring: bool = False,
-                        feature: str = "atomic", atomic_features=None, device=None) -> "DeviceDataIterator":
+                        feature: str = "atomic", atomic_features=None, ring_aromatic=None,
+                        device=None) -> "DeviceDataIterator":
         """The iterator ``DataIterator(data_energy, compute_voronoi_neighbors(structs, d_t, w_t), ...)`` would be, with
         the neighbour lists selected and flattened on the device (``voronoi.select_neighbors``, in the chunks of
         ``predict_structures``): no facet record and no neighbour list reaches the host.  ``targets``: one value per
         structure.  ``angle``: the weight column (True = solid angle, False = normalised); None picks the one
         ``DataIterator`` trains a model with this ``g_update`` on.  ``d_t`` / ``w_t`` / ``cutoff`` /
         ``allow_pathological``: as in ``compute_voronoi_neighbors``.  ``feature='cgcnn'`` needs ``atomic_features``, the
-        model's per-element feature table ([Z + 1, 92] float32).
+        model's per-element feature table ([Z + 1, 92] float32).  ``use_ring=True`` needs ``ring_aromatic``: one
+        ``[n_sites, 2]`` integer array per structure (the third item of a ``data_energy`` row; ``check_ring_aromatic``),
+        uploaded once as the iterator's ``ring`` array.
 
-        Refused: ``use_ring``, and ``feature='cgcnn'`` without ``atomic_features`` (``NotImplementedError``); structures
-        without sites, with more than 1000 (1000 is the reference's neighbour padding marker) or, for ``feature='cgcnn'``,
-        with an atomic number that has no row in the table (``ValueError``, naming the structure)."""
+        Refused: ``use_ring`` without ``ring_aromatic``, and ``feature='cgcnn'`` without ``atomic_features``
+        (``NotImplementedError``); ``ring_aromatic`` without ``use_ring``, flags of the wrong count, shape or values,
+        structures without sites, with more than 1000 (1000 is the reference's neighbour padding marker) or, for
+        ``feature='cgcnn'``, with an atomic number that has no row in the table (``ValueError``, naming the
+        structure)."""
         from . import voronoi as V
         from .model import MAX_STRUCTURE_ATOMS, _structure_chunks
-        _refuse_structures_route("DeviceDataIterator.from_structures", use_ring, feature, atomic_features)
+        _refuse_structures_route("DeviceDataIterator.from_structures", use_ring, feature, atomic_features, ring_aromatic)
         if feature == "cgcnn":
             atomic_features = check_atomic_features(atomic_features)
         structs = list(structs)
@@ -317,6 +361,7 @@ class DeviceDataIterator:
         if feature == "cgcnn":
             check_table_rows(np.concatenate([np.asarray(s.atomic_numbers).reshape(-1) for s in structs]), atom_off,
                              len(atomic_features))
+        ring = check_ring_aromatic(ring_aromatic, n_atoms) if use_ring else None
         conv = 1000 if converter else 1.0
         energy = np.array([float(t) * conv for t in targets], "float32")
         column = bool(g_update) if angle is None else bool(angle)
@@ -352,10 +397,11 @@ class DeviceDataIterator:
             return torch.cat([p[k] for p in parts]) if parts else torch.empty(0, dtype=dt, device=dev)
         arrays = {"struct_atom_off": torch.from_numpy(atom_off.astype(np.int32)).to(dev), "atom_nbr_off": an, "z": z,
                   "nbr_idx": cat(0, torch.int32), "nbr_w": cat(1, torch.float32), "nbr_d": cat(2, torch.float32),
-                  "target": torch.from_numpy(energy).to(dev), "ring": None}
+                  "target": torch.from_numpy(energy).to(dev),
+                  "ring": torch.from_numpy(ring).to(dev) if use_ring else None}
         return cls(arrays, energy, atom_off, pair_off, np.concatenate(nmax), npairs, batch_size=batch_size,
-                   shuffle=shuffle, use_ring=False, weight_index=2 if column else 3, converter=conv, feature=feature,
-                   atomic_features=atomic_features)
+                   shuffle=shuffle, use_ring=bool(use_ring), weight_index=2 if column else 3, converter=conv,
+                   feature=feature, atomic_features=atomic_features)
 
     # ------------------------------------------------------------------ Sequence protocol
     def on_epoch_end(self):

@@ -261,7 +261,7 @@ class ScannKerasModel:
 
     def predict_structures(self, structs, d_t: float = 4.0, w_t: float = 0.4, angle: Optional[bool] = None,
                            batch_size: int = 128, cutoff: float = 13.0, allow_pathological: bool = False,
-                           local_attention: bool = False, atomic_features=None):
+                           local_attention: bool = False, atomic_features=None, ring_aromatic=None):
         """Structures in, ``[target [S, 1], ga_score]`` out: the README flow (``compute_voronoi_neighbor`` ->
         ``prepare_input_pmt`` -> ``predict``) for many structures, with the neighbour lists selected and batched on
         the device (``voronoi.select_neighbors``).  ``ga_score`` is a list of S float32 arrays, one value per atom,
@@ -281,9 +281,15 @@ class ScannKerasModel:
         through it on the device (``Engine.set_atomic_features``), with the outputs of ``predict`` on the padded
         ``DataIterator(..., feature='cgcnn', atomic_features=...)`` batches of the same structures.
 
-        Refused: ring-feature models (the ring / aromatic flags come from openbabel, not from the geometry) -- use
-        ``predict`` on ``DataIterator`` batches for those --, ``feature='cgcnn'`` models without ``atomic_features``
-        (``NotImplementedError``), and structures with more than 1000 atoms (1000 is the reference's neighbour padding
+        ``use_ring`` models need ``ring_aromatic``: one ``[n_sites, 2]`` integer array per structure, in input order.
+        These flags come from openbabel's ring and aromaticity perception, not from the geometry: pass the third item of
+        the reference's ``data_energy`` rows, or run openbabel on the structures.  Each chunk's flags are uploaded once
+        and copied into its batches on the device; the outputs are those of ``predict`` on the padded
+        ``DataIterator(..., use_ring=True)`` batches of the same structures.
+
+        Refused: ``use_ring`` models without ``ring_aromatic`` and ``feature='cgcnn'`` models without
+        ``atomic_features`` (``NotImplementedError``); ``ring_aromatic`` for a model without ``use_ring``, flags of the
+        wrong count, shape or values, structures with more than 1000 atoms (1000 is the reference's neighbour padding
         marker) or, for ``feature='cgcnn'``, with an atomic number the table has no row for (``ValueError``).
 
         ``local_attention=True`` returns ``[target, ga_score, la]``: ``la`` holds one ``LocalAttentionScores`` per
@@ -291,12 +297,10 @@ class ScannKerasModel:
         local-attention layer.  The scores of the padding are not copied back.  ``target`` and ``ga_score`` are those
         of the plain call."""
         from . import voronoi as V
+        from .datagenerator import _refuse_ring_route, check_ring_aromatic
         scores = _check_flag("local_attention", local_attention)
         spec = self.spec
-        if spec.use_ring:
-            raise NotImplementedError("predict_structures: use_ring models need the ring / aromatic flags of openbabel, "
-                                      "which the geometry does not give; build the batches with DataIterator(..., "
-                                      "use_ring=True) and call predict")
+        _refuse_ring_route("predict_structures", spec.use_ring, ring_aromatic)
         if spec.feature == "cgcnn" and atomic_features is None:
             raise NotImplementedError("predict_structures: a feature='cgcnn' model embeds atoms through the per-element "
                                       "feature table it was trained with: pass atomic_features=<[Z + 1, 92] float32 "
@@ -316,22 +320,27 @@ class ScannKerasModel:
         if batch_size < 1:
             raise ValueError("batch_size must be >= 1")
         column = bool(spec.g_update) if angle is None else bool(angle)
+        n_at = np.array([len(X) for X in checked[1]], np.int64)
+        atom_off = np.concatenate([[0], np.cumsum(n_at)])
+        ring = check_ring_aromatic(ring_aromatic, n_at) if spec.use_ring else None
         eng = self.engine
         if atomic_features is not None:
             from .datagenerator import check_atomic_features, check_table_rows
             table = check_atomic_features(atomic_features)
-            n_at = np.array([len(X) for X in checked[1]], np.int64)
             check_table_rows(np.concatenate([np.asarray(s.atomic_numbers).reshape(-1) for s in structs]),
-                             np.concatenate([[0], np.cumsum(n_at)]), len(table))
+                             atom_off, len(table))
             eng.set_atomic_features(table)
         y_out = np.zeros((len(structs), 1), np.float32)
         ga_out, la_out = [], []
         for c0, c1 in _structure_chunks([len(X) for X in checked[1]], batch_size):
             sel = V.select_neighbors(structs[c0:c1], d_t, w_t, column, cutoff, allow_pathological, first_index=c0,
                                      _checked=(checked[0][c0:c1], checked[1][c0:c1]))
+            # the chunk's flags, uploaded once; each batch copies its contiguous atom rows on the device
+            d_ring = (torch.from_numpy(ring[atom_off[c0]:atom_off[c1]]).to(sel.sel_count.device)
+                      if ring is not None else None)
             for s0 in range(0, c1 - c0, batch_size):
                 s1 = min(s0 + batch_size, c1 - c0)
-                csr = sel.csr(s0, s1)
+                csr = sel.csr(s0, s1, ring=d_ring)
                 M, N = shape_class(csr["M"], csr["N"])
                 b = eng.load_batch_device_csr(csr, M=M, N=N, plan=False)
                 y, ga, *la = eng.predict_step(b, replan=True, local_attention="csr" if scores else False)
@@ -636,20 +645,21 @@ class SCANN:
 
     def _predict_structures(self, structs, d_t: float = 4.0, w_t: float = 0.4, angle: Optional[bool] = None,
                             batch_size: int = 128, cutoff: float = 13.0, allow_pathological: bool = False,
-                            local_attention: bool = False, atomic_features=None):
+                            local_attention: bool = False, atomic_features=None, ring_aromatic=None):
         """``ScannKerasModel.predict_structures`` with the target scaled back like ``predict_data``."""
         y, *rest = self.model.predict_structures(structs, d_t=d_t, w_t=w_t, angle=angle, batch_size=batch_size,
                                                  cutoff=cutoff, allow_pathological=allow_pathological,
-                                                 local_attention=local_attention, atomic_features=atomic_features)
+                                                 local_attention=local_attention, atomic_features=atomic_features,
+                                                 ring_aromatic=ring_aromatic)
         return (y * self.std + self.mean, *rest)
 
     @property
     def predict_structures(self):
         """``predict_structures(structs, d_t=4.0, w_t=0.4, angle=None, batch_size=128, cutoff=13.0,
-        allow_pathological=False, local_attention=False, atomic_features=None)``: ``ScannKerasModel.predict_structures`` with the target
-        scaled back like ``predict_data``.  (A property, not a plain method: the record of SCANN's plain public methods in
-        tests/golden/reference/graph_public_surface.npz stays the surface that was compared with the reference's SCANN,
-        which has no such method.)"""
+        allow_pathological=False, local_attention=False, atomic_features=None, ring_aromatic=None)``:
+        ``ScannKerasModel.predict_structures`` with the target scaled back like ``predict_data``.  (A property, not a
+        plain method: the record of SCANN's plain public methods in tests/golden/reference/graph_public_surface.npz stays
+        the surface that was compared with the reference's SCANN, which has no such method.)"""
         return functools.partial(SCANN._predict_structures, self)
 
     # ---- training shell (scann_model.py:163-313) ------------------------------------------------------------
@@ -705,15 +715,23 @@ class SCANN:
                                                          for ix in (train, valid, test)]
         return train, valid, test
 
-    def _prepare_structures(self, structs, targets, split: bool = True, atomic_features=None, **voronoi_args):
+    def _prepare_structures(self, structs, targets, split: bool = True, atomic_features=None, ring_aromatic=None,
+                            **voronoi_args):
         """``SCANN.prepare_structures``: see the property."""
-        from .datagenerator import DeviceDataIterator, _refuse_structures_route
+        from .datagenerator import DeviceDataIterator, _refuse_structures_route, check_ring_aromatic
         hy, cm = self.config["hyper"], self.config["model"]
-        _refuse_structures_route("SCANN.prepare_structures", cm["use_ring"], cm["feature"], atomic_features)
+        _refuse_structures_route("SCANN.prepare_structures", cm["use_ring"], cm["feature"], atomic_features,
+                                 ring_aromatic)
         structs = list(structs)
         targets = list(np.asarray(targets, dtype=object).reshape(-1))
         if len(targets) != len(structs):
             raise ValueError(f"{len(structs)} structures but {len(targets)} targets")
+        ring = None
+        if cm["use_ring"]:              # checked in the caller's order, so that an error names the caller's index
+            n_at = [len(np.asarray(s.cart_coords).reshape(-1, 3)) for s in structs]
+            atom_off = np.concatenate([[0], np.cumsum(n_at, dtype=np.int64)])
+            flat = check_ring_aromatic(ring_aromatic, n_at)
+            ring = [flat[atom_off[k]:atom_off[k + 1]] for k in range(len(structs))]
         rows = np.empty((len(structs), 2), dtype=object)          # the rows of load_dataset: [atoms, target]
         rows[:, 1] = [float(t) for t in targets]
         self._scale_targets(rows)
@@ -725,20 +743,25 @@ class SCANN:
                                                       g_update=cm["g_update"], use_ring=cm["use_ring"],
                                                       feature=cm["feature"],
                                                       atomic_features=atomic_features if cm["feature"] == "cgcnn" else None,
+                                                      ring_aromatic=[ring[k] for k in ix] if ring is not None else None,
                                                       **voronoi_args)
 
         return self._attach_iterators(len(structs), iterator, split)
 
     @property
     def prepare_structures(self):
-        """``prepare_structures(structs, targets, split=True, atomic_features=None, **voronoi_args)``: ``prepare_dataset``
-        for structures and their targets instead of the reference's data files.  The same target scaling
-        (``hyper.scaler``), config entries and split of the global numpy generator; ``trainIter`` / ``validIter`` /
-        ``testIter`` (or ``dataIter``) are ``DeviceDataIterator.from_structures`` (``voronoi_args``: ``d_t``, ``w_t``,
-        ``angle``, ``cutoff``, ``allow_pathological``, ``converter``), so training and evaluation gather their batches on
-        the device.  ``feature='cgcnn'`` models need ``atomic_features``, their per-element feature table ([Z + 1, 92]
-        float32).  Refused for ``use_ring`` models and for ``feature='cgcnn'`` without ``atomic_features``.  (A property
-        for the same reason as ``predict_structures``.)"""
+        """``prepare_structures(structs, targets, split=True, atomic_features=None, ring_aromatic=None,
+        **voronoi_args)``: ``prepare_dataset`` for structures and their targets instead of the reference's data files.
+        The same target scaling (``hyper.scaler``), config entries and split of the global numpy generator;
+        ``trainIter`` / ``validIter`` / ``testIter`` (or ``dataIter``) are ``DeviceDataIterator.from_structures``
+        (``voronoi_args``: ``d_t``, ``w_t``, ``angle``, ``cutoff``, ``allow_pathological``, ``converter``), so training
+        and evaluation gather their batches on the device.  ``feature='cgcnn'`` models need ``atomic_features``, their
+        per-element feature table ([Z + 1, 92] float32).  ``use_ring`` models (``model.use_ring`` of the config) need
+        ``ring_aromatic``, one ``[n_sites, 2]`` integer array per structure (the third item of the reference's
+        ``data_energy`` rows, or openbabel's perception run on the structures); the flags follow their structures
+        through the split, as ``prepare_dataset``'s rows do.  Refused for ``use_ring`` models without ``ring_aromatic``
+        and for ``feature='cgcnn'`` without ``atomic_features``.  (A property for the same reason as
+        ``predict_structures``.)"""
         return functools.partial(SCANN._prepare_structures, self)
 
     def create_callbacks(self):

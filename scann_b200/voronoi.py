@@ -206,18 +206,26 @@ class NeighborSelection:
     def __len__(self):
         return len(self.struct_atom_off) - 1
 
-    def csr(self, s0: int = 0, s1: int = None) -> dict:
+    def csr(self, s0: int = 0, s1: int = None, ring: torch.Tensor = None) -> dict:
         """Structures ``s0 .. s1 - 1`` as the CSR batch of ``DataIterator.csr_item`` in ONE device blob (``"blob"``,
         byte offsets ``"offsets"``; device views ``struct_atom_off``, ``atom_nbr_off``, ``z``, ``nbr_idx``, ``nbr_w``,
         ``nbr_d``).  Host side: ``B``, ``M`` (most atoms), ``N`` (most kept neighbours), ``P`` (kept pairs) and per
-        structure ``n_atoms``, ``nmax``, ``npairs``."""
+        structure ``n_atoms``, ``nmax``, ``npairs``.
+
+        ``ring``: the ring / aromatic flags of every atom row of the selection, a device int32 tensor ``[A, 2]``.  The
+        rows of the batch's atoms (contiguous) are copied into a ``"ring"`` segment of the blob (view ``ring`` [nA, 2]),
+        which ``Engine.load_batch_device_csr`` packs like ``DataIterator.csr_item``'s ``ring``."""
         s1 = len(self) if s1 is None else s1
         B = s1 - s0
         sa = self.struct_atom_off
         a0, nA = int(sa[s0]), int(sa[s1] - sa[s0])
         dev = self.sel_count.device
+        if ring is not None and (ring.dtype != torch.int32 or ring.device != dev or
+                                 tuple(ring.shape) != (int(sa[-1]), 2) or not ring.is_contiguous()):
+            raise ValueError(f"ring must be a contiguous int32 tensor [{int(sa[-1])}, 2] on {dev}, not "
+                             f"{ring.dtype} {list(ring.shape)} on {ring.device}")
         sizes_b = [("sa", 4 * (B + 1)), ("an", 4 * (nA + 1)), ("z", 4 * nA), ("idx", 4 * nA * _SEL), ("w", 4 * nA * _SEL),
-                   ("d", 4 * nA * _SEL)]
+                   ("d", 4 * nA * _SEL)] + ([("ring", 8 * nA)] if ring is not None else [])
         offs, off = {}, 0
         for name, nb in sizes_b:
             offs[name] = off
@@ -230,6 +238,8 @@ class NeighborSelection:
             self.sel_idx.data_ptr(), self.sel_w.data_ptr(), self.sel_d.data_ptr(), blob.data_ptr(), offs["sa"],
             offs["an"], offs["z"], offs["idx"], offs["w"], offs["d"], sizes.data_ptr(),
             ctypes.c_void_p(stream.cuda_stream)), "scann_voronoi_batch_csr"))
+        if ring is not None:            # one device-to-device copy on the same stream
+            blob[offs["ring"]:offs["ring"] + 8 * nA].view(torch.int32).copy_(ring[a0:a0 + nA].reshape(-1))
         host = torch.empty(2 * B, dtype=torch.int32, pin_memory=True)
         host.copy_(sizes, non_blocking=True)
         stream.synchronize()
@@ -240,11 +250,14 @@ class NeighborSelection:
 
         def view(name, dt, n):
             return blob[offs[name]:offs[name] + 4 * n].view(dt)
-        return {"blob": blob, "offsets": offs, "B": B, "M": int(n_atoms.max()), "N": int(nmax.max()), "P": P,
-                "n_atoms": n_atoms, "nmax": nmax, "npairs": npairs,
-                "struct_atom_off": view("sa", torch.int32, B + 1), "atom_nbr_off": view("an", torch.int32, nA + 1),
-                "z": view("z", torch.int32, nA), "nbr_idx": view("idx", torch.int32, P),
-                "nbr_w": view("w", torch.float32, P), "nbr_d": view("d", torch.float32, P)}
+        out = {"blob": blob, "offsets": offs, "B": B, "M": int(n_atoms.max()), "N": int(nmax.max()), "P": P,
+               "n_atoms": n_atoms, "nmax": nmax, "npairs": npairs,
+               "struct_atom_off": view("sa", torch.int32, B + 1), "atom_nbr_off": view("an", torch.int32, nA + 1),
+               "z": view("z", torch.int32, nA), "nbr_idx": view("idx", torch.int32, P),
+               "nbr_w": view("w", torch.float32, P), "nbr_d": view("d", torch.float32, P)}
+        if ring is not None:
+            out["ring"] = view("ring", torch.int32, 2 * nA).view(nA, 2)
+        return out
 
 
 def _select_pass(d_lat, d_x, d_sa, sa_off, atoms, cut, allow_pathological, d_t, w_t, column, sel):
