@@ -399,15 +399,19 @@ int scann_loss_value(const float* params, const float* l2mask, int n, const floa
  * Centres: centre_atom [C] (global atom row), centre_struct [C], cutoff [C] (Angstrom; the point set is every image
  * within it).  allow_pathological: emit the finite facets of a cell that also has unbounded ones (otherwise such a
  * centre emits nothing and carries flag 1: pymatgen's caller widens its cutoff and runs it again).
- * slots: C * cap records of scratch (cap <= 64), slot_count [C] int32.  The result goes to `blob` (device):
+ * slots: C * cap records of scratch (cap 1..256), slot_count [C] int32.  cap <= 64 runs the narrow cell search (64
+ * facet slots, 32 vertices per facet, 4 centres per CTA); a larger cap runs the wide one (256 slots, 64 vertices per
+ * facet, one centre per CTA in ~33 KB of shared memory), for the centres whose cell overflows the narrow one.
+ * A cell that fits in the narrow form gets the same records, bit for bit, from either.  The result goes to `blob`:
  *   int32 off[C+1] (CSR), int32 flags[C] (1 = unbounded facet, plus the SCANN_ERR_VORONOI_* bits of that centre),
  *   zero padding to a multiple of 32 bytes, then ScannVoronoiFacet records (centre c: off[c] .. off[c+1]);
  *   blob bytes >= round_up(4 * (2C + 1), 32) + 32 * C * cap.
  * Records of a centre: its finite facets with solid angle > 0, in no particular order.  host_blob (nullable, host,
  * pinned for an asynchronous copy) receives the whole blob with one cudaMemcpyAsync on `stream`.
  * status [0] |= SCANN_ERR_VORONOI_*: two points of a cell closer than 1e-8 Angstrom, a capacity of the kernel
- * exceeded (64 facets, 32 vertices per facet, 128 points of one distance shell, |image| <= 511), a centre without a
- * finite facet, a cut whose facet boundary is not one cycle (numerically inconsistent input). */
+ * exceeded (the form's facet slots -- the box takes 6 -- and vertices per facet, 128 points of one distance shell,
+ * |image| <= 511; the slots bound the cell while it is built, which can hold more facets than the final one), a centre
+ * without a finite facet, a cut whose facet boundary is not one cycle (numerically inconsistent input). */
 #define SCANN_ERR_VORONOI_COINCIDENT 32
 #define SCANN_ERR_VORONOI_CAPACITY 64
 #define SCANN_ERR_VORONOI_NO_FACET 128
@@ -432,9 +436,11 @@ int scann_voronoi_neighbors(const double* lattice, const double* coords, const i
  * its records by (distance, site, n0, n1, n2) -- fp64 distance, image components decoded -- keeps those with
  * distance <= d_thresh and normalized >= w_thresh (fp64) and writes them to row r = centre_row[c] of the staging arrays:
  * sel_count[r], and at r * 64 + i: sel_idx = site, sel_w = (float)solid_angle (weight_column 0) or (float)normalized
- * (weight_column 1), sel_d = (float)distance, all rounded to nearest.  One warp per centre, rank by counting; a centre
- * whose cell was dropped (flag 1 without allow_pathological) has no record and writes count 0.
- * status |= SCANN_ERR_VORONOI_CAPACITY if a centre has more than 64 records.
+ * (weight_column 1), sel_d = (float)distance, all rounded to nearest.  One warp per centre, rank by counting (up to 64
+ * records two per lane, 65..256 ranked against the records in global memory); a centre whose cell was dropped (flag 1
+ * without allow_pathological) has no record and writes count 0.  Staging rows hold 64 neighbours: a centre that keeps
+ * more writes its true count to sel_count, only its first 64 to the row, and sets SCANN_ERR_VORONOI_CAPACITY in
+ * status, as does a centre of more than 256 records.
  * scann_voronoi_batch_csr writes structures s0 .. s0 + n_structs - 1 (struct_atom_off [S+1] and z [A] over the same
  * atom rows as the staging arrays; atom0 = struct_atom_off[s0] and n_atoms, known to the caller) as the CSR batch of
  * scann_pack_batch into the device blob `csr` at the byte offsets off_*: struct_atom_off [n_structs+1] (from 0),

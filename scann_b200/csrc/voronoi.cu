@@ -27,6 +27,8 @@
 // themselves never enter a result: a finite cell has none left, and a facet that touches the box is infinite.
 // Precision: vertices come from 3x3 solves on planes of magnitude |x_j - x_i|, not from interpolation along edges,
 // so the box size does not limit the accuracy of the finite cell.
+#include <type_traits>
+
 #include "common.cuh"
 
 #define SCANN_ERR_VORONOI_COINCIDENT 32
@@ -35,10 +37,14 @@
 #define SCANN_ERR_VORONOI_TOPOLOGY 256
 #define VOR_INFINITE 1          // per-centre flag: the cell has an unbounded facet in S (host retries / drops it)
 
-#define VOR_FMAX 64             // facet slots per cell, slots 0..5 = the box
-#define VOR_VMAX 32             // vertices per facet
+// The cell search comes in two forms, the same code at two capacities (vor_cells_kernel<F, V, WARPS>):
+#define VOR_FMAX 64             // narrow form: facet slots per cell, slots 0..5 = the box
+#define VOR_VMAX 32             //   vertices per facet
+#define VOR_WARPS 4             //   centres per CTA
+#define VOR_FMAX_WIDE 256       // wide form, for the centres whose cell overflows the narrow one (labels stay uint8_t)
+#define VOR_VMAX_WIDE 64        //   vertices per facet (64-bit vertex masks)
+#define VOR_WARPS_WIDE 1        //   centres per CTA: ~33 KB of shared memory per warp
 #define VOR_CB 128              // candidates per distance band
-#define VOR_WARPS 4             // centres per CTA
 #define VOR_IMG_MAX 511         // |n_k| of a packed image (10 bits per component)
 
 struct VorFacet {               // one finite facet of a centre's cell (32 bytes; ScannVoronoiFacet in the header)
@@ -46,20 +52,29 @@ struct VorFacet {               // one finite facet of a centre's cell (32 bytes
     int32_t site, image;        // image = (n0 + 512) | (n1 + 512) << 10 | (n2 + 512) << 20
 };
 
+// a set of vertices of one facet: one bit per vertex
+template <int V> using VorMask = typename std::conditional<(V > 32), uint64_t, uint32_t>::type;
+__device__ __forceinline__ int vor_popc(uint32_t m) { return __popc(m); }
+__device__ __forceinline__ int vor_popc(uint64_t m) { return __popcll(m); }
+__device__ __forceinline__ int vor_hibit(uint32_t m) { return 31 - __clz(m); }
+__device__ __forceinline__ int vor_hibit(uint64_t m) { return 63 - __clzll(m); }
+
+// One centre's cell: F facet slots of up to V vertices.
+template <int F, int V>
 struct VorWarp {
-    double4 pl[VOR_FMAX];       // facet plane: n.x <= w with x relative to the centre
+    double4 pl[F];              // facet plane: n.x <= w with x relative to the centre
     double cd2[VOR_CB];         // candidates of the current band
     int cj[VOR_CB], cimg[VOR_CB];
-    int fsite[VOR_FMAX], fimg[VOR_FMAX];
-    uint32_t omask[VOR_FMAX];   // vertices outside the plane being inserted
+    int fsite[F], fimg[F];
+    VorMask<V> omask[F];        // vertices outside the plane being inserted
     double edge[32];
     int hist[32];
     int ncol;
     uint8_t order[VOR_CB];
-    uint8_t lab[VOR_FMAX][VOR_VMAX];
-    uint8_t tmp[32][VOR_VMAX];
-    uint8_t nv[VOR_FMAX];
-    uint8_t succ[VOR_FMAX];
+    uint8_t lab[F][V];
+    uint8_t tmp[32][V];
+    uint8_t nv[F];
+    uint8_t succ[F];
 };
 
 __device__ __forceinline__ double3 d3sub(double3 a, double3 b) { return make_double3(a.x - b.x, a.y - b.y, a.z - b.z); }
@@ -125,16 +140,23 @@ __device__ __forceinline__ void vor_for_each_image(const double* X, const double
     }
 }
 
-__global__ void __launch_bounds__(32 * VOR_WARPS) vor_cells_kernel(
+// One warp per centre; lane l owns facet slots l, l + 32, ... (F / 32 of them).  The free slot a cut takes is the lowest
+// free one, so a cell that fits in the narrow form gets the same slots, hence the same bits, from either form.
+template <int F, int V, int WARPS>
+__global__ void __launch_bounds__(32 * WARPS) vor_cells_kernel(
         const double* __restrict__ lattice, const double* __restrict__ coords, const int32_t* __restrict__ sa_off,
         const int32_t* __restrict__ centre_atom, const int32_t* __restrict__ centre_struct,
         const double* __restrict__ cutoff, int n_centres, int allow_pathological, int cap, VorFacet* __restrict__ slots,
         int32_t* __restrict__ slot_count, int32_t* __restrict__ centre_flags, int32_t* __restrict__ status) {
-    __shared__ VorWarp sm[VOR_WARPS];
+    static_assert(F % 32 == 0 && F <= 256 && V <= 64, "slot labels are uint8_t, vertex masks at most 64 bits");
+    static_assert(sizeof(VorWarp<F, V>) * WARPS <= 48 * 1024, "static shared memory of a CTA");
+    constexpr int P = F / 32;           // facet slots per lane
+    using M = VorMask<V>;
+    __shared__ VorWarp<F, V> sm[WARPS];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int c = blockIdx.x * VOR_WARPS + w;
+    const int c = blockIdx.x * WARPS + w;
     if (c >= n_centres) return;
-    VorWarp& W = sm[w];
+    VorWarp<F, V>& W = sm[w];
     const int i = centre_atom[c], s = centre_struct[c];
     const int a0 = sa_off[s], a1 = sa_off[s + 1];
     double L[9], B[9];
@@ -156,7 +178,7 @@ __global__ void __launch_bounds__(32 * VOR_WARPS) vor_cells_kernel(
 
     // ---- the box: slot 2a (+axis a) / 2a+1 (-axis a); polygons counter-clockwise seen from outside
     const double H = 1e5 * fmax(cut, 1.0);
-    for (int t = lane; t < VOR_FMAX; t += 32) W.nv[t] = 0;
+    for (int t = lane; t < F; t += 32) W.nv[t] = 0;
     __syncwarp();
     if (lane < 6) {
         int a = lane >> 1, pos = (lane & 1) == 0, b = (a + 1) % 3, cc = (a + 2) % 3;
@@ -263,15 +285,15 @@ __global__ void __launch_bounds__(32 * VOR_WARPS) vor_cells_kernel(
             // classify every vertex against the new plane; largest vertex distance of the current cell
             double r2 = 0.0;
             int nonfinite = 0;
-            for (int h = 0; h < 2; ++h) {
+            for (int h = 0; h < P; ++h) {
                 const int f = lane + 32 * h, n = W.nv[f];
-                uint32_t m = 0;
+                M m = 0;
                 for (int k = 0; k < n; ++k) {
                     double3 v = vor_vertex(W.pl, f, W.lab[f][k == 0 ? n - 1 : k - 1], W.lab[f][k]);
                     r2 = fmax(r2, x3dot(v, v));
                     const double scale = __dmul_rn(tol, __dadd_rn(sqrt(d2), fabs(v.x) + fabs(v.y) + fabs(v.z)));
                     if (!(fabs(v.x) + fabs(v.y) + fabs(v.z) < INFINITY)) nonfinite = 1;     // planes without one point
-                    if (__dadd_rn(x3dot(v, e), -off) > scale) m |= 1u << k;
+                    if (__dadd_rn(x3dot(v, e), -off) > scale) m |= M(1) << k;
                 }
                 W.omask[f] = m;
             }
@@ -280,29 +302,39 @@ __global__ void __launch_bounds__(32 * VOR_WARPS) vor_cells_kernel(
             if (__any_sync(0xffffffffu, nonfinite)) { err |= SCANN_ERR_VORONOI_TOPOLOGY; break; }
             if (d2 > 4.0 * r2) { done = true; break; }      // security radius reached: S adds nothing more
             bool any = false;
-            for (int h = 0; h < 2; ++h) any |= W.omask[lane + 32 * h] != 0;
+            for (int h = 0; h < P; ++h) any |= W.omask[lane + 32 * h] != 0;
             if (!__any_sync(0xffffffffu, any)) continue;
-            // a free slot for the new facet (free before this cut)
-            bool fr0 = lane >= 6 && W.nv[lane] == 0, fr1 = W.nv[lane + 32] == 0;
-            unsigned b0 = __ballot_sync(0xffffffffu, fr0), b1 = __ballot_sync(0xffffffffu, fr1);
-            if (!b0 && !b1) { err |= SCANN_ERR_VORONOI_CAPACITY; break; }
-            const int p = b0 ? __ffs(b0) - 1 : 32 + __ffs(b1) - 1;
+            // a free slot for the new facet (free before this cut): the lowest one
+            int p;
+            if constexpr (P == 2) {                           // the narrow form as it always was: the same SASS
+                bool fr0 = lane >= 6 && W.nv[lane] == 0, fr1 = W.nv[lane + 32] == 0;
+                unsigned b0 = __ballot_sync(0xffffffffu, fr0), b1 = __ballot_sync(0xffffffffu, fr1);
+                if (!b0 && !b1) { err |= SCANN_ERR_VORONOI_CAPACITY; break; }
+                p = b0 ? __ffs(b0) - 1 : 32 + __ffs(b1) - 1;
+            } else {
+                p = -1;
+                for (int h = P - 1; h >= 0; --h) {
+                    const unsigned b = __ballot_sync(0xffffffffu, (h > 0 || lane >= 6) && W.nv[lane + 32 * h] == 0);
+                    if (b) p = 32 * h + __ffs(b) - 1;
+                }
+                if (p < 0) { err |= SCANN_ERR_VORONOI_CAPACITY; break; }
+            }
             // cut every facet: the inside run plus the entry and exit vertices
             int bad = 0, npart = 0, first = -1;
-            for (int h = 0; h < 2; ++h) {
+            for (int h = 0; h < P; ++h) {
                 const int f = lane + 32 * h, n = W.nv[f];
-                const uint32_t m = W.omask[f];
+                const M m = W.omask[f];
                 if (m == 0 || n == 0) continue;
-                const uint32_t full = n == 32 ? 0xffffffffu : (1u << n) - 1u;
+                const M full = n == V ? ~M(0) : (M(1) << n) - M(1);
                 if (m == full) { W.nv[f] = 0; continue; }
                 int runs = 0, kx = 0;
                 for (int k = 0; k < n; ++k) {
                     int k1 = k + 1 == n ? 0 : k + 1;
                     if (!((m >> k) & 1) && ((m >> k1) & 1)) { ++runs; kx = k; }
                 }
-                const int nin = n - __popc(m);
+                const int nin = n - vor_popc(m);
                 if (runs != 1) { bad |= SCANN_ERR_VORONOI_TOPOLOGY; continue; }
-                if (nin + 2 > VOR_VMAX) { bad |= SCANN_ERR_VORONOI_CAPACITY; continue; }
+                if (nin + 2 > V) { bad |= SCANN_ERR_VORONOI_CAPACITY; continue; }
                 int kin = kx - nin + 1;                       // first inside vertex of the run ending at kx
                 if (kin < 0) kin += n;
                 int o = 0;
@@ -323,8 +355,8 @@ __global__ void __launch_bounds__(32 * VOR_WARPS) vor_cells_kernel(
             if (bad) { err |= bad; break; }
             if (lane == 0) {                                  // the new facet's boundary: f -> succ(f)
                 int f = first, k = 0;
-                do { if (k < VOR_VMAX) W.lab[p][k] = (uint8_t)f; ++k; f = W.succ[f]; } while (f != first && k <= VOR_FMAX);
-                if (k > VOR_VMAX) err |= SCANN_ERR_VORONOI_CAPACITY;
+                do { if (k < V) W.lab[p][k] = (uint8_t)f; ++k; f = W.succ[f]; } while (f != first && k <= F);
+                if (k > V) err |= SCANN_ERR_VORONOI_CAPACITY;
                 else if (f != first || k != npart) err |= SCANN_ERR_VORONOI_TOPOLOGY;
                 W.nv[p] = err ? 0 : (uint8_t)k;
                 W.pl[p] = make_double4(e.x, e.y, e.z, off);
@@ -339,11 +371,11 @@ __global__ void __launch_bounds__(32 * VOR_WARPS) vor_cells_kernel(
 
     // ---- finite facets: solid angle (pymatgen's fan formula), distance, site, image
     int flags = 0, nkeep = 0;
-    double sa[2] = {0.0, 0.0};
-    bool keep[2] = {false, false};
+    double sa[P] = {};
+    bool keep[P] = {};
     if (!err) {
         bool inf = false;
-        for (int h = 0; h < 2; ++h) {
+        for (int h = 0; h < P; ++h) {
             const int f = lane + 32 * h, n = W.nv[f];
             if (f < 6 || n == 0) continue;
             bool touches = false;
@@ -351,20 +383,20 @@ __global__ void __launch_bounds__(32 * VOR_WARPS) vor_cells_kernel(
             if (touches) { inf = true; continue; }
             // drop coincident consecutive vertices (a cluster of degree-3 vertices is one point of the cell)
             const double tol2 = 1e-18 * W.pl[f].w * 2.0;      // (1e-9 * |x_j - x_i|)^2
-            uint32_t kept = 0;
+            M kept = 0;
             double3 v0 = vor_vertex(W.pl, f, W.lab[f][n - 1], W.lab[f][0]), prev = v0;
             kept = 1;
             int nk = 1, lastk = 0;
             for (int k = 1; k < n; ++k) {
                 double3 v = vor_vertex(W.pl, f, W.lab[f][k - 1], W.lab[f][k]), dv = d3sub(v, prev);
-                if (d3dot(dv, dv) > tol2) { kept |= 1u << k; prev = v; ++nk; lastk = k; }
+                if (d3dot(dv, dv) > tol2) { kept |= M(1) << k; prev = v; ++nk; lastk = k; }
             }
             while (nk > 1) {                                  // trailing vertices that coincide with the first
                 double3 v = vor_vertex(W.pl, f, W.lab[f][lastk - 1], W.lab[f][lastk]), dv = d3sub(v, v0);
                 if (d3dot(dv, dv) > tol2) break;
-                kept &= ~(1u << lastk);
+                kept &= ~(M(1) << lastk);
                 --nk;
-                lastk = 31 - __clz(kept);
+                lastk = vor_hibit(kept);
             }
             if (nk < 3) continue;
             double3 r0 = v0, rk = v0;
@@ -387,13 +419,14 @@ __global__ void __launch_bounds__(32 * VOR_WARPS) vor_cells_kernel(
             keep[h] = ang > 0.0;
         }
         if (__any_sync(0xffffffffu, inf)) flags |= VOR_INFINITE;
-        double mx = fmax(sa[0], sa[1]);
+        double mx = sa[0];
+        for (int h = 1; h < P; ++h) mx = fmax(mx, sa[h]);
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
         const bool emit = allow_pathological || !(flags & VOR_INFINITE);
         if (emit) {
             int base = 0;
-            for (int h = 0; h < 2; ++h) {
+            for (int h = 0; h < P; ++h) {
                 unsigned bal = __ballot_sync(0xffffffffu, keep[h]);
                 if (keep[h]) {
                     const int k = base + __popc(bal & ((1u << lane) - 1u));
@@ -472,8 +505,8 @@ extern "C" int scann_voronoi_neighbors(const double* lattice, const double* coor
                                        const int32_t* centre_atom, const int32_t* centre_struct, const double* cutoff,
                                        int n_centres, int allow_pathological, int cap, void* slots, int32_t* slot_count,
                                        void* blob, void* host_blob, int32_t* status, void* stream) {
-    if (n_centres < 0 || cap <= 0 || cap > VOR_FMAX) {
-        scann_set_error("scann_voronoi_neighbors: n_centres %d, cap %d (1..%d)", n_centres, cap, VOR_FMAX);
+    if (n_centres < 0 || cap <= 0 || cap > VOR_FMAX_WIDE) {
+        scann_set_error("scann_voronoi_neighbors: n_centres %d, cap %d (1..%d)", n_centres, cap, VOR_FMAX_WIDE);
         return 1;
     }
     if (n_centres == 0) return 0;
@@ -481,9 +514,15 @@ extern "C" int scann_voronoi_neighbors(const double* lattice, const double* coor
     int32_t* off = (int32_t*)blob;
     int32_t* flags = off + n_centres + 1;
     VorFacet* rec = (VorFacet*)((char*)blob + vor_header_bytes(n_centres));
-    vor_cells_kernel<<<(n_centres + VOR_WARPS - 1) / VOR_WARPS, 32 * VOR_WARPS, 0, st>>>(
-        lattice, coords, struct_atom_off, centre_atom, centre_struct, cutoff, n_centres, allow_pathological, cap,
-        (VorFacet*)slots, slot_count, flags, status);
+    if (cap <= VOR_FMAX)        // the narrow form
+        vor_cells_kernel<VOR_FMAX, VOR_VMAX, VOR_WARPS><<<(n_centres + VOR_WARPS - 1) / VOR_WARPS, 32 * VOR_WARPS, 0, st>>>(
+            lattice, coords, struct_atom_off, centre_atom, centre_struct, cutoff, n_centres, allow_pathological, cap,
+            (VorFacet*)slots, slot_count, flags, status);
+    else                        // the wide form
+        vor_cells_kernel<VOR_FMAX_WIDE, VOR_VMAX_WIDE, VOR_WARPS_WIDE>
+            <<<(n_centres + VOR_WARPS_WIDE - 1) / VOR_WARPS_WIDE, 32 * VOR_WARPS_WIDE, 0, st>>>(
+            lattice, coords, struct_atom_off, centre_atom, centre_struct, cutoff, n_centres, allow_pathological, cap,
+            (VorFacet*)slots, slot_count, flags, status);
     vor_scan_kernel<<<1, 1024, 0, st>>>(slot_count, n_centres, off);
     vor_compact_kernel<<<(n_centres + 7) / 8, 256, 0, st>>>((const VorFacet*)slots, slot_count, off, n_centres, cap, rec);
     if (int rc = scann_check_launch("scann_voronoi_neighbors")) return rc;
@@ -503,6 +542,8 @@ extern "C" int scann_voronoi_neighbors(const double* lattice, const double* coor
 // compute_voronoi_neighbors, DataIterator): order the facets by (distance, site, n0, n1, n2), keep distance <= d_thresh
 // and normalised solid angle >= w_thresh (fp64), and write (site, (float)weight, (float)distance).
 #define VOR_SEL_WARPS 8
+#define VOR_SEL 64              // staging slots per atom row: the most neighbours an atom keeps
+#define VOR_SEL_MAX VOR_FMAX_WIDE   // records per centre (the wide cell search's capacity)
 
 // Facet a before facet b in the host's np.lexsort order.  The image components compare as stored: (x & 1023) and
 // (x & 1023) - 512 order alike, but the packed word itself would compare n2 first.
@@ -517,22 +558,65 @@ __device__ __forceinline__ bool vor_before(double da, int sa, int ia, double db,
     return false;
 }
 
-// One warp per centre: up to 64 records, two per lane; the rank of a kept record is the number of kept records before
-// it in the host's order (ties, which would be one facet listed twice, by record position: a stable sort).
-__global__ void __launch_bounds__(32 * VOR_SEL_WARPS) vor_select_kernel(
+// The select of a centre with more records than two per lane: each lane ranks its records against all of the centre's
+// records in global memory (rare: only centres of the wide cell search).  Out of line, so that it leaves the register
+// allocation of the two-per-lane code alone.
+__device__ __noinline__ void vor_select_wide(const VorFacet* __restrict__ rec, int k, double d_thresh, double w_thresh,
+                                             int column, int lane, int r, int32_t* __restrict__ sel_count,
+                                             int32_t* __restrict__ sel_idx, float* __restrict__ sel_w,
+                                             float* __restrict__ sel_d, int32_t* __restrict__ status) {
+    const size_t row = (size_t)r * VOR_SEL;
+    int kept = 0;
+    for (int i = lane; i < k; i += 32) {
+        const VorFacet ri = rec[i];
+        if (!(ri.distance <= d_thresh && ri.normalized >= w_thresh)) continue;
+        int rank = 0;
+        for (int j = 0; j < k; ++j) {
+            const double dj = rec[j].distance;
+            if (j == i || !(dj <= d_thresh && rec[j].normalized >= w_thresh)) continue;
+            const int sj = rec[j].site, ij = rec[j].image;
+            rank += vor_before(dj, sj, ij, ri.distance, ri.site, ri.image) ||
+                    (j < i && !vor_before(ri.distance, ri.site, ri.image, dj, sj, ij));
+        }
+        if (rank < VOR_SEL) {
+            sel_idx[row + rank] = ri.site;
+            sel_w[row + rank] = __double2float_rn(column ? ri.normalized : ri.solid_angle);
+            sel_d[row + rank] = __double2float_rn(ri.distance);
+        }
+        ++kept;
+    }
+    kept = __reduce_add_sync(0xffffffffu, kept);
+    if (lane == 0) {
+        sel_count[r] = kept;                    // the true count: more than VOR_SEL is an error the host reports
+        if (kept > VOR_SEL) atomicOr(status, SCANN_ERR_VORONOI_CAPACITY);
+    }
+}
+
+// One warp per centre; the rank of a kept record is the number of kept records before it in the host's order (ties,
+// which would be one facet listed twice, by record position: a stable sort).  Up to 64 records: two per lane, ranked
+// in shared memory.  65..256 records (a centre of the wide cell search): a loop over the lane's records, ranked against
+// the records in global memory; more than 64 kept ones write their true count and set the capacity bit.
+// Min. blocks 1: with the out-of-line call and no min. blocks, ptxas (CUDA 12.9, sm_100a) gives the kernel 32 registers
+// and spills 8 bytes; with it, 40 registers and no spill.
+__global__ void __launch_bounds__(32 * VOR_SEL_WARPS, 1) vor_select_kernel(
         const int32_t* __restrict__ off, const VorFacet* __restrict__ rec, const int32_t* __restrict__ centre_row, int n,
         double d_thresh, double w_thresh, int column, int32_t* __restrict__ sel_count, int32_t* __restrict__ sel_idx,
         float* __restrict__ sel_w, float* __restrict__ sel_d, int32_t* __restrict__ status) {
-    __shared__ double s_d[VOR_SEL_WARPS][VOR_FMAX];
-    __shared__ int s_site[VOR_SEL_WARPS][VOR_FMAX], s_img[VOR_SEL_WARPS][VOR_FMAX];
+    __shared__ double s_d[VOR_SEL_WARPS][VOR_SEL];
+    __shared__ int s_site[VOR_SEL_WARPS][VOR_SEL], s_img[VOR_SEL_WARPS][VOR_SEL];
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int c = blockIdx.x * VOR_SEL_WARPS + w;
     if (c >= n) return;                         // whole warps only: the kernel has no block-level barrier
     const int o = off[c];
     int k = off[c + 1] - o;
-    if (k > VOR_FMAX) {
+    if (k > VOR_SEL_MAX) {
         if (lane == 0) atomicOr(status, SCANN_ERR_VORONOI_CAPACITY);
-        k = VOR_FMAX;
+        k = VOR_SEL_MAX;
+    }
+    if (k > VOR_SEL) {                          // warp-uniform
+        vor_select_wide(rec + o, k, d_thresh, w_thresh, column, lane, centre_row[c], sel_count, sel_idx, sel_w, sel_d,
+                        status);
+        return;
     }
     VorFacet r[2];
     bool keep[2];
@@ -550,7 +634,7 @@ __global__ void __launch_bounds__(32 * VOR_SEL_WARPS) vor_select_kernel(
         }
     }
     __syncwarp();
-    const size_t row = (size_t)centre_row[c] * VOR_FMAX;
+    const size_t row = (size_t)centre_row[c] * VOR_SEL;
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
         const int i = lane + 32 * h;
@@ -602,10 +686,10 @@ __global__ void vor_batch_fill_kernel(const int32_t* __restrict__ sa, const int3
     const int a = t >> 5, lane = t & 31;
     if (a >= A) return;
     const int row = a0 + a, k = sel_count[row], p = an[a];
-    for (int i = lane; i < k; i += 32) {
-        idx_out[p + i] = sel_idx[(size_t)row * VOR_FMAX + i];
-        w_out[p + i] = sel_w[(size_t)row * VOR_FMAX + i];
-        d_out[p + i] = sel_d[(size_t)row * VOR_FMAX + i];
+    for (int i = lane; i < min(k, VOR_SEL); i += 32) {    // k > VOR_SEL: select has flagged the centre
+        idx_out[p + i] = sel_idx[(size_t)row * VOR_SEL + i];
+        w_out[p + i] = sel_w[(size_t)row * VOR_SEL + i];
+        d_out[p + i] = sel_d[(size_t)row * VOR_SEL + i];
     }
     if (lane == 0) {
         z_out[a] = z[row];

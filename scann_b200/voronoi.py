@@ -6,6 +6,8 @@ tessellation of every periodic image within ``cutoff``) and keeps the facets wit
 normalised by the site's largest, is at least ``w_thresh``.  Here every site of every structure is one warp of
 ``scann_voronoi_neighbors`` (csrc/voronoi.cu, fp64); pymatgen's retry loop -- a site whose cell still has an unbounded
 facet is run again with ``cutoff = min(2 cutoff, longest cell diagonal + 0.011)`` -- re-launches only those sites.
+The cell search holds 64 facets; a site whose cell overflows it (a surface atom that sees a slab's periodic images
+across the vacuum) runs again, at the same cutoff, in the wide form of 256 facets, and stays wide through later retries.
 
 A structure is anything with ``.cart_coords`` ``[n, 3]`` and ``.lattice.matrix`` ``[3, 3]`` (rows = lattice vectors),
 e.g. a pymatgen ``Structure``.  A molecule must be boxed first (pymatgen: ``Molecule.get_boxed_structure``).
@@ -22,15 +24,36 @@ from scann_b200 import _abi
 
 ERR_COINCIDENT, ERR_CAPACITY, ERR_NO_FACET, ERR_TOPOLOGY = 32, 64, 128, 256
 _INFINITE = 1
-_CAP = 64                       # facet records per centre (the kernel's facet capacity)
-_CHUNK = 1 << 16                # centres per launch
+_CAP = 64                       # facet records per centre of the narrow cell search (its facet capacity)
+_CAP_WIDE = 256                 # ... of the wide one, for the centres whose cell overflows the narrow one
+_CHUNK = 1 << 16                # centres per narrow launch
+_CHUNK_WIDE = _CHUNK * _CAP // _CAP_WIDE    # centres per wide launch: the same bytes of facet slots
 FACET = np.dtype([("solid_angle", "<f8"), ("normalized", "<f8"), ("distance", "<f8"), ("site", "<i4"),
                   ("image", "<i4")])
 _MESSAGES = {ERR_COINCIDENT: "two points of its Voronoi point set are closer than 1e-8 Angstrom",
-             ERR_CAPACITY: "its Voronoi cell exceeds the kernel's capacity (64 facets, 32 vertices per facet, 128 "
+             ERR_CAPACITY: "its Voronoi cell exceeds the kernel's capacity (256 facets, 64 vertices per facet, 128 "
                            "points in one distance shell, images up to 511 cells away)",
              ERR_NO_FACET: "its Voronoi cell has no finite facet",
              ERR_TOPOLOGY: "a cut of its Voronoi cell was numerically inconsistent"}
+# a capacity error together with another error bit in the narrow pass (not retried wide)
+_CAPACITY_NARROW = ("its Voronoi cell exceeds the kernel's capacity (64 facets, 32 vertices per facet, 128 points in "
+                    "one distance shell, images up to 511 cells away)")
+
+
+def _why(err, wide):
+    return "; ".join(_CAPACITY_NARROW if b == ERR_CAPACITY and not wide else m
+                     for b, m in _MESSAGES.items() if err & b)
+
+
+def _passes(todo, wide):
+    """The launches of one round of the retry loop: (centres, cap, wide) for the narrow centres of ``todo``, in
+    chunks of ``_CHUNK``, then for its wide ones, in chunks of ``_CHUNK_WIDE``.  A list, split before the first launch:
+    a centre that overflows the narrow form in this round is marked wide for the next round, not added to this one."""
+    out = []
+    for w, cap, chunk in ((False, _CAP, _CHUNK), (True, _CAP_WIDE, _CHUNK_WIDE)):
+        part = todo[wide[todo] == w]
+        out += [(part[c0:c0 + chunk], cap, w) for c0 in range(0, len(part), chunk)]
+    return out
 
 
 def max_cutoff(lattice) -> float:
@@ -57,8 +80,9 @@ def _arrays(structs):
     return lats, xs
 
 
-def _run(lat, X, sa_off, atoms, cut, allow_pathological):
-    """One launch over the listed centres -> (off [C+1], flags [C], records)."""
+def _run(lat, X, sa_off, atoms, cut, allow_pathological, cap=_CAP):
+    """One launch over the listed centres with ``cap`` facet slots each (<= 64: the narrow cell search, up to 256: the
+    wide one) -> (off [C+1], flags [C], records)."""
     _abi.require_gpu()
     dev = torch.device("cuda", torch.cuda.current_device())
     C = len(atoms)
@@ -70,8 +94,8 @@ def _run(lat, X, sa_off, atoms, cut, allow_pathological):
     d_cs = torch.from_numpy(cs.astype(np.int32)).to(dev)
     d_cut = torch.from_numpy(np.ascontiguousarray(cut, np.float64)).to(dev)
     head = (4 * (2 * C + 1) + 31) // 32 * 32
-    nbytes = head + FACET.itemsize * C * _CAP
-    slots = torch.empty(FACET.itemsize * C * _CAP, dtype=torch.uint8, device=dev)
+    nbytes = head + FACET.itemsize * C * cap
+    slots = torch.empty(FACET.itemsize * C * cap, dtype=torch.uint8, device=dev)
     count = torch.empty(C, dtype=torch.int32, device=dev)
     blob = torch.empty(nbytes, dtype=torch.uint8, device=dev)
     host = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
@@ -79,7 +103,7 @@ def _run(lat, X, sa_off, atoms, cut, allow_pathological):
     stream = torch.cuda.current_stream(dev)
     _abi.check(_abi.lib.scann_voronoi_neighbors(
         d_lat.data_ptr(), d_x.data_ptr(), d_sa.data_ptr(), d_at.data_ptr(), d_cs.data_ptr(), d_cut.data_ptr(), C,
-        1 if allow_pathological else 0, _CAP, slots.data_ptr(), count.data_ptr(), blob.data_ptr(),
+        1 if allow_pathological else 0, cap, slots.data_ptr(), count.data_ptr(), blob.data_ptr(),
         ctypes.c_void_p(host.data_ptr()), status.data_ptr(), ctypes.c_void_p(stream.cuda_stream)),
         "scann_voronoi_neighbors")
     stream.synchronize()
@@ -107,18 +131,21 @@ def voronoi_polyhedra(structs: Sequence, cutoff: float = 13.0, allow_pathologica
     tops = np.array([max_cutoff(L) for L in lats])
     cut = np.full(A, float(cutoff))
     result = [None] * A
+    wide = np.zeros(A, bool)
     todo = np.arange(A)
     while len(todo):
         again = []
-        for c0 in range(0, len(todo), _CHUNK):
-            atoms = todo[c0:c0 + _CHUNK]
-            off, flags, rec = _run(lat, X, sa_off, atoms, cut[atoms], allow_pathological)
+        for atoms, cap, is_wide in _passes(todo, wide):
+            off, flags, rec = _run(lat, X, sa_off, atoms, cut[atoms], allow_pathological, cap)
             for k, a in enumerate(atoms):
                 err = int(flags[k]) & ~_INFINITE
                 s, site = int(sid[a]), int(a - sa_off[sid[a]])
+                if err == ERR_CAPACITY and not is_wide:   # the cell overflows the narrow form: again, wide
+                    wide[a] = True
+                    again.append(a)
+                    continue
                 if err:
-                    why = "; ".join(m for b, m in _MESSAGES.items() if err & b)
-                    raise ValueError(f"structure {s}, site {site}: {why}")
+                    raise ValueError(f"structure {s}, site {site}: {_why(err, is_wide)}")
                 if flags[k] & _INFINITE and not allow_pathological:
                     if cut[a] >= tops[s]:
                         raise ValueError(f"structure {s}, site {site}: infinite Voronoi facet at the largest cutoff "
@@ -175,7 +202,7 @@ def compute_voronoi_neighbor(struct, d_thresh: float = 4.0, w_thresh: float = 0.
 # scann_voronoi_select orders and thresholds each centre's records into per-atom staging rows, and
 # scann_voronoi_batch_csr writes any run of structures as the CSR batch that Engine.load_batch_device_csr packs.
 # Only the per-centre flags (retry / error) and a few sizes per batch come back to the host.
-_SEL = _CAP                     # staging slots per atom row (the kernel's facet capacity)
+_SEL = 64                       # staging slots per atom row: the most neighbours an atom keeps
 _ALIGN = 16
 
 # optional CUDA-event log (tools/structure_predict_bench.py): name -> list of (start, end) event pairs
@@ -260,8 +287,10 @@ class NeighborSelection:
         return out
 
 
-def _select_pass(d_lat, d_x, d_sa, sa_off, atoms, cut, allow_pathological, d_t, w_t, column, sel):
-    """One cell search over the listed centres, its records thresholded into the staging rows -> flags [C] (host)."""
+def _select_pass(d_lat, d_x, d_sa, sa_off, atoms, cut, allow_pathological, d_t, w_t, column, sel, cap=_CAP):
+    """One cell search over the listed centres (``cap`` as in ``_run``), its records thresholded into the staging rows
+    -> (flags [C], kept [C] or None) on the host.  ``kept``: the true kept count of every centre, returned only when a
+    centre keeps more neighbours than a staging row holds."""
     dev = d_x.device
     C = len(atoms)
     cs = np.searchsorted(sa_off, atoms, side="right") - 1
@@ -273,28 +302,32 @@ def _select_pass(d_lat, d_x, d_sa, sa_off, atoms, cut, allow_pathological, d_t, 
     d_at, d_cs = d_up[:4 * C].view(torch.int32), d_up[4 * C:8 * C].view(torch.int32)
     d_cut = d_up[8 * C:].view(torch.float64)
     hb = (4 * (2 * C + 1) + 31) // 32 * 32
-    slots = torch.empty(FACET.itemsize * C * _CAP, dtype=torch.uint8, device=dev)
+    slots = torch.empty(FACET.itemsize * C * cap, dtype=torch.uint8, device=dev)
     count = torch.empty(C, dtype=torch.int32, device=dev)
-    blob = torch.empty(hb + FACET.itemsize * C * _CAP, dtype=torch.uint8, device=dev)
-    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    blob = torch.empty(hb + FACET.itemsize * C * cap, dtype=torch.uint8, device=dev)
+    status = torch.zeros(2, dtype=torch.int32, device=dev)       # [0]: the cell search, [1]: the select
     stream = torch.cuda.current_stream(dev)
     st = ctypes.c_void_p(stream.cuda_stream)
-    _timed("voronoi_neighbors", stream, lambda: _abi.check(_abi.lib.scann_voronoi_neighbors(
+    wide = "_wide" if cap > _CAP else ""
+    _timed("voronoi_neighbors" + wide, stream, lambda: _abi.check(_abi.lib.scann_voronoi_neighbors(
         d_lat.data_ptr(), d_x.data_ptr(), d_sa.data_ptr(), d_at.data_ptr(), d_cs.data_ptr(), d_cut.data_ptr(), C,
-        1 if allow_pathological else 0, _CAP, slots.data_ptr(), count.data_ptr(), blob.data_ptr(), None,
+        1 if allow_pathological else 0, cap, slots.data_ptr(), count.data_ptr(), blob.data_ptr(), None,
         status.data_ptr(), st), "scann_voronoi_neighbors"))
     count_, idx, w, d = sel
-    _timed("voronoi_select", stream, lambda: _abi.check(_abi.lib.scann_voronoi_select(
+    _timed("voronoi_select" + wide, stream, lambda: _abi.check(_abi.lib.scann_voronoi_select(
         blob.data_ptr(), d_at.data_ptr(), C, float(d_t), float(w_t), 0 if column else 1, count_.data_ptr(),
-        idx.data_ptr(), w.data_ptr(), d.data_ptr(), status.data_ptr(), st), "scann_voronoi_select"))
-    host = torch.empty(C + 1, dtype=torch.int32, pin_memory=True)
+        idx.data_ptr(), w.data_ptr(), d.data_ptr(), status.data_ptr() + 4, st), "scann_voronoi_select"))
+    host = torch.empty(C + 2, dtype=torch.int32, pin_memory=True)
     host[:C].copy_(blob[4 * (C + 1):4 * (2 * C + 1)].view(torch.int32), non_blocking=True)
     host[C:].copy_(status, non_blocking=True)
     stream.synchronize()
     h = host.numpy()
-    if h[C] & ERR_CAPACITY and not (h[:C] & ERR_CAPACITY).any():
-        raise _abi.ScannAbiError("scann_voronoi_select: a centre has more records than the staging rows hold")
-    return h[:C].copy()
+    kept = None
+    if h[C + 1] & ERR_CAPACITY:         # more kept neighbours than a staging row holds (or a malformed blob)
+        kept = count_[torch.from_numpy(np.asarray(atoms, np.int64)).to(dev)].cpu().numpy()
+        if not (kept > _SEL).any():
+            raise _abi.ScannAbiError("scann_voronoi_select: a centre has more records than the select accepts")
+    return h[:C].copy(), kept
 
 
 def select_neighbors(structs: Sequence, d_thresh: float = 4.0, w_thresh: float = 0.4, angle: bool = True,
@@ -327,26 +360,38 @@ def select_neighbors(structs: Sequence, d_thresh: float = 4.0, w_thresh: float =
     sid = np.repeat(np.arange(len(xs)), nat)
     tops = np.array([max_cutoff(L) for L in lats])
     cut = np.full(A, float(cutoff))
+    wide = np.zeros(A, bool)
     todo = np.arange(A)
     while len(todo):
         again = []
-        for c0 in range(0, len(todo), _CHUNK):
-            atoms = todo[c0:c0 + _CHUNK]
-            flags = _select_pass(d_lat, d_x, d_sa, sa_off, atoms, cut[atoms], allow_pathological, d_thresh, w_thresh,
-                                 angle, sel)
+        for atoms, cap, is_wide in _passes(todo, wide):
+            flags, kept = _select_pass(d_lat, d_x, d_sa, sa_off, atoms, cut[atoms], allow_pathological, d_thresh,
+                                       w_thresh, angle, sel, cap)
             for k in np.flatnonzero(flags):         # the checks of voronoi_polyhedra, in the same order
                 a = int(atoms[k])
                 err = int(flags[k]) & ~_INFINITE
                 s, site = int(sid[a]), int(a - sa_off[sid[a]])
+                if err == ERR_CAPACITY and not is_wide:
+                    wide[a] = True
+                    again.append(a)
+                    continue
                 if err:
-                    why = "; ".join(m for b, m in _MESSAGES.items() if err & b)
-                    raise ValueError(f"structure {first_index + s}, site {site}: {why}")
+                    raise ValueError(f"structure {first_index + s}, site {site}: {_why(err, is_wide)}")
                 if not allow_pathological:
                     if cut[a] >= tops[s]:
                         raise ValueError(f"structure {first_index + s}, site {site}: infinite Voronoi facet at the "
                                          f"largest cutoff {cut[a]:.3f} Angstrom")
                     cut[a] = min(2 * cut[a], tops[s] + 0.001)
                     again.append(a)
+            if kept is not None:                    # a centre whose cell is final keeps more than a row holds
+                for k in np.flatnonzero(kept > _SEL):
+                    a = int(atoms[k])
+                    if a in again:
+                        continue
+                    s, site = int(sid[a]), int(a - sa_off[sid[a]])
+                    raise ValueError(f"structure {first_index + s}, site {site}: {int(kept[k])} neighbours kept "
+                                     f"(distance <= {d_thresh}, normalised solid angle >= {w_thresh}), more than the "
+                                     f"{_SEL} a neighbour list holds")
         todo = np.array(again, np.int64)
     return out
 
